@@ -41,6 +41,7 @@ sys.path.insert(0, ROOT)
 METRIC = "vcycle_dofs_per_s"
 UNIT = "DOFs/s"
 ESS = np.ones(6, dtype=np.int32)
+DUMP_MAX_BYTES = 64 * 10 ** 6          # --dump-outputs: all files of one run together
 
 
 def peaks():
@@ -160,6 +161,20 @@ class ClockSampler:
         return out
 
 
+def dump_outputs(dirname, arrays, budget=DUMP_MAX_BYTES):
+    """--dump-outputs: each array as dirname/<name>.npy in float64.  An array larger than its share of the budget is
+    stored at a fixed, seeded sample of its indices (ascending), so two builds run with the same arguments store the same
+    entries and can be compared file by file."""
+    os.makedirs(dirname, exist_ok=True)
+    share = budget // max(len(arrays), 1)
+    for name, a in arrays.items():
+        a = np.ascontiguousarray(a, dtype=np.float64).ravel()
+        cap = (share - 128) // a.itemsize                  # 128 bytes: the .npy header of a 1-D array
+        if a.size > cap:
+            a = a[np.sort(np.random.default_rng(2024).choice(a.size, cap, replace=False))]
+        np.save(os.path.join(dirname, name + ".npy"), a)
+
+
 def traffic_from_profiles():
     """dram bytes per launch of the dominant kernel from the committed ncu capture, if any"""
     p = os.path.join(ROOT, "profiles", "traffic.json")
@@ -211,11 +226,11 @@ def time_cpu_vcycles(H, n, steps, warmup, budget_s=25.0):
     t_all = time.perf_counter()
     for _ in range(steps):
         t0 = time.perf_counter()
-        H.mult(r)
+        z = H.mult(r)
         ts.append(time.perf_counter() - t0)
         if time.perf_counter() - t_all > budget_s:
             break
-    return float(np.mean(ts)), len(ts)
+    return float(np.mean(ts)), len(ts), z
 
 
 def host_threads():
@@ -378,7 +393,9 @@ def run_reference(args, rank):
         n_s, deformed = min(n_s, 32), False              # the numpy coarsening oracle: minutes beyond that
     levels = levels_for(n_s, args.levels)
     H, ndofs = cpu_vcycle_setup(n_s, levels, cores, inputs)
-    t, done = time_cpu_vcycles(H, ndofs, args.steps, min(args.warmup, 1), budget_s=120.0)
+    t, done, z = time_cpu_vcycles(H, ndofs, args.steps, min(args.warmup, 1), budget_s=120.0)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"z": z})
     value = ndofs / t
     setup = None if args.no_cpu_setup else cpu_setup_baseline()
     sample = ("H(div) AMGe V-cycle (Hiptmair l1-GS, PCG-GS coarse) on %d^3 hexahedra, %d RT0 dofs, %d levels (level operators "
@@ -441,7 +458,14 @@ def main():
                     help="multi-GPU halo exchange: NVLink peer-memory stores (default) or ncclSend/ncclRecv")
     ap.add_argument("--profile-range", action="store_true",
                     help="bracket 2 extra V-cycles with cudaProfilerStart/Stop (ncu --profile-from-start off) and exit")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned (the preconditioned vector z; z_rank<r> per "
+                         "rank when N > 1) as DIR/<name>.npy in float64, at most 64 MB in all: a longer vector is stored at a "
+                         "fixed, seeded sample of its entries.  The inputs depend on the arguments only, so two builds can be "
+                         "compared file by file")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -679,6 +703,8 @@ def main():
     barrier()
     launches = ctx.launch_count() - l0
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"z" if world == 1 else "z_rank%d" % rank: z_dev.download()}, DUMP_MAX_BYTES // world)
     ms = max_over_ranks(ms)
     ms_per_step = ms / args.steps
     value = ndofs_global / (ms_per_step * 1e-3)
@@ -803,7 +829,7 @@ def main():
             orc.set_threads(1)
             lv = levels_for(args.cpu_n, levels)
             H, nd = cpu_vcycle_setup(args.cpu_n, lv, 1, lambda ns, lvv: product_level_operators(ctx, ns, lvv))
-            t_cpu, done = time_cpu_vcycles(H, nd, 30, 1, budget_s=20.0)
+            t_cpu, done, _ = time_cpu_vcycles(H, nd, 30, 1, budget_s=20.0)
             cpu_baseline = {"value": nd / t_cpu, "unit": UNIT, "cores": 1, "kind": "port",
                             "sample": "same H(div) AMGe V-cycle (Hiptmair l1-GS natural order, PCG-GS coarse) on a "
                                       "%d^3-hexahedra sample (%d RT0 dofs, %d levels), %d cycles of %.3f s on one host core; "

@@ -5,12 +5,14 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
-def test_reference_arm_prints_one_json_line():
+def test_reference_arm_prints_one_json_line(tmp_path):
     r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "2", "--warmup", "1",
-                        "--ref-n", "16"], cwd=ROOT,
+                        "--ref-n", "16", "--dump-outputs", str(tmp_path)], cwd=ROOT,
                        env=dict(os.environ, OMP_NUM_THREADS="1"),      # what torchrun exports: the arm must override it
                        capture_output=True, text=True, timeout=600)
     assert r.returncode == 0, r.stderr[-2000:]
@@ -24,6 +26,22 @@ def test_reference_arm_prints_one_json_line():
     assert d["cpu_baseline"]["cores"] == threads and d["cpu_baseline"]["omp_threads"] == threads
     assert d["cpu_baseline"]["setup"]["seconds"] > 0
     assert d["e2e"] == {"value": d["value"], "unit": "DOFs/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
+    assert d["steps"] == 2
+    assert sorted(os.listdir(tmp_path)) == ["z.npy"]
+    z = np.load(tmp_path / "z.npy")
+    assert z.dtype == np.float64 and z.ndim == 1 and np.isfinite(z).all() and np.abs(z).max() > 0
+
+
+def test_dump_outputs_samples_a_long_array_within_the_budget(tmp_path):
+    import bench
+    a = np.arange(10000, dtype=np.float64)
+    bench.dump_outputs(str(tmp_path / "one"), {"short": a[:100], "long": a}, budget=8192)
+    bench.dump_outputs(str(tmp_path / "two"), {"short": a[:100], "long": a}, budget=8192)
+    assert os.path.getsize(tmp_path / "one" / "short.npy") + os.path.getsize(tmp_path / "one" / "long.npy") <= 8192
+    assert np.array_equal(np.load(tmp_path / "one" / "short.npy"), a[:100])
+    s = np.load(tmp_path / "one" / "long.npy")
+    assert s.size == (4096 - 128) // 8 and np.all(np.diff(s) > 0) and np.array_equal(s, np.floor(s))
+    assert np.array_equal(np.load(tmp_path / "two" / "long.npy"), s)         # the same entries from run to run
 
 
 def test_reference_arm_other_ranks_exit_quietly():

@@ -111,11 +111,33 @@ int pe_ctx_profile_get(pe_ctx *ctx, int kernel_id, int64_t *count, double *total
  * The idea: the iterate of one slab stays in L2 across its C colour launches instead of being re-read from HBM by
  * every colour (each colour gathers (C-1)/C of the vector: the 1.2x DRAM traffic over the algorithmic bytes).  Measured
  * (round 2): 4 slabs 9.38 ms, 8 slabs 9.76 ms against 7.46 ms -- the smaller launches cost more than the gathers save
- * and the L2 hit rate of the gathers did not rise; default off.  Read when a smoother is created. */
+ * and the L2 hit rate of the gathers did not rise; default off.  Read when a smoother is created.
+ * PE_TUNE_LOCAL_SMEM_BYTES [0 = built-in limits]: workspace bytes above which an agglomerate of the batched local solves
+ * of Coarsen() leaves shared memory for a global-memory slab (k_traces_gmem, k_extension_gmem).  The built-in limits are
+ * 200 KB (traces) and 220 KB (extension); a value > 0 replaces both and is clamped to them, so 1 sends every
+ * agglomerate to the global-memory kernels.  Results do not depend on it (same arithmetic, same order). */
 enum { PE_TUNE_SELL_MIN_ROWS = 0, PE_TUNE_SELL_GROUP = 1, PE_TUNE_PDL = 2, PE_TUNE_GATHER_KEEP_PCT = 3, PE_TUNE_P2P_HALO = 4,
-       PE_TUNE_FUSED_GS_MAX_MB = 5, PE_TUNE_GS_SLABS = 6, PE_TUNE_COUNT = 7 };
+       PE_TUNE_FUSED_GS_MAX_MB = 5, PE_TUNE_GS_SLABS = 6, PE_TUNE_LOCAL_SMEM_BYTES = 7, PE_TUNE_COUNT = 8 };
 int pe_set_tuning(int key, int value);
 int pe_get_tuning(int key);
+/* process-wide counts of the work each size-dispatched kernel variant was given, kept on the host at the place that
+ * chooses the variant (no device work, no synchronisation).  Units: rows for SpMV (per call), SpGEMM (per bin of the
+ * symbolic / numeric pass) and relaxation (per launch of k_jacobi_update<TPR> / k_gs_set<TPR>), agglomerates for the
+ * batched local solves.  An operation recorded into a persistent program or captured into a CUDA graph counts once,
+ * when it is recorded.  Three slots refine the local solves: EXT_SPLIT_SMEM counts the agglomerates of the listed
+ * shared-memory extension launch of a batch split between both kernels (also counted in EXT_SMEM); TRACES_GMEM_REUSE and
+ * EXT_GMEM_REUSE count the agglomerates a global-workspace CTA takes after its first one (a launch with more agglomerates
+ * than CTAs reuses each workspace slab).  out: n slots (slots past PE_VARIANT_COUNT are set to 0; NULL with n = 0 copies nothing);
+ * reset != 0 zeroes every counter after the copy. */
+enum { PE_VARIANT_SPMV_SELL = 0, PE_VARIANT_SPMV_STREAM = 1, PE_VARIANT_SPMV_VECTOR = 2,
+       PE_VARIANT_SPGEMM_SYM_T128 = 3, PE_VARIANT_SPGEMM_SYM_T1024 = 4, PE_VARIANT_SPGEMM_SYM_T8192 = 5, PE_VARIANT_SPGEMM_SYM_GMEM = 6,
+       PE_VARIANT_SPGEMM_NUM_T128 = 7, PE_VARIANT_SPGEMM_NUM_T1024 = 8, PE_VARIANT_SPGEMM_NUM_T8192 = 9, PE_VARIANT_SPGEMM_NUM_GMEM = 10,
+       PE_VARIANT_RELAX_TPR_1 = 11, PE_VARIANT_RELAX_TPR_2 = 12, PE_VARIANT_RELAX_TPR_4 = 13, PE_VARIANT_RELAX_TPR_8 = 14,
+       PE_VARIANT_RELAX_TPR_16 = 15, PE_VARIANT_RELAX_TPR_32 = 16,
+       PE_VARIANT_TRACES_SMEM = 17, PE_VARIANT_TRACES_GMEM = 18, PE_VARIANT_EXT_SMEM = 19, PE_VARIANT_EXT_GMEM = 20,
+       PE_VARIANT_EXT_SPLIT_SMEM = 21, PE_VARIANT_TRACES_GMEM_REUSE = 22, PE_VARIANT_EXT_GMEM_REUSE = 23,
+       PE_VARIANT_COUNT = 24 };
+int pe_variant_counts(int64_t *out, int n, int reset);
 /* write a scratch buffer larger than L2 (bench hygiene) */
 int pe_ctx_flush_l2(pe_ctx *ctx);
 

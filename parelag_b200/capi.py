@@ -136,6 +136,7 @@ TUNE_GATHER_KEEP_PCT = 3
 TUNE_P2P_HALO = 4
 TUNE_FUSED_GS_MAX_MB = 5
 TUNE_GS_SLABS = 6
+TUNE_LOCAL_SMEM_BYTES = 7
 
 
 def set_tuning(key, value):
@@ -144,6 +145,29 @@ def set_tuning(key, value):
 
 def get_tuning(key):
     return lib().pe_get_tuning(key)
+
+
+# slots of pe_variant_counts (include/parelag_b200.h)
+VARIANT_SLOTS = ("SPMV_SELL", "SPMV_STREAM", "SPMV_VECTOR",
+                 "SPGEMM_SYM_T128", "SPGEMM_SYM_T1024", "SPGEMM_SYM_T8192", "SPGEMM_SYM_GMEM",
+                 "SPGEMM_NUM_T128", "SPGEMM_NUM_T1024", "SPGEMM_NUM_T8192", "SPGEMM_NUM_GMEM",
+                 "RELAX_TPR_1", "RELAX_TPR_2", "RELAX_TPR_4", "RELAX_TPR_8", "RELAX_TPR_16", "RELAX_TPR_32",
+                 "TRACES_SMEM", "TRACES_GMEM", "EXT_SMEM", "EXT_GMEM",
+                 "EXT_SPLIT_SMEM", "TRACES_GMEM_REUSE", "EXT_GMEM_REUSE")
+(SPMV_SELL, SPMV_STREAM, SPMV_VECTOR,
+ SPGEMM_SYM_T128, SPGEMM_SYM_T1024, SPGEMM_SYM_T8192, SPGEMM_SYM_GMEM,
+ SPGEMM_NUM_T128, SPGEMM_NUM_T1024, SPGEMM_NUM_T8192, SPGEMM_NUM_GMEM,
+ RELAX_TPR_1, RELAX_TPR_2, RELAX_TPR_4, RELAX_TPR_8, RELAX_TPR_16, RELAX_TPR_32,
+ TRACES_SMEM, TRACES_GMEM, EXT_SMEM, EXT_GMEM,
+ EXT_SPLIT_SMEM, TRACES_GMEM_REUSE, EXT_GMEM_REUSE) = range(len(VARIANT_SLOTS))
+
+
+def variant_counts(reset=False):
+    """Rows / agglomerates each size-dispatched kernel variant was given since the last reset (process-wide):
+    int64 array indexed by the slot constants above.  reset: zero the counters after reading them."""
+    out = np.zeros(len(VARIANT_SLOTS), dtype=np.int64)
+    _chk(lib().pe_variant_counts(_ptr(out), len(VARIANT_SLOTS), 1 if reset else 0))
+    return out
 
 
 def nccl_unique_id():

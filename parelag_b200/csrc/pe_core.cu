@@ -2,6 +2,7 @@
 #include "pe_core.cuh"
 #include "pe_stream.cuh"
 #include <dlfcn.h>
+#include <atomic>
 #include <cstring>
 #include <cstdio>
 
@@ -128,7 +129,7 @@ extern "C" int pe_ctx_destroy(pe_ctx *c)
     return 0;
 }
 
-static int g_tuning[PE_TUNE_COUNT] = {200000, 0, 1, 0, 1, 0, 0};
+static int g_tuning[PE_TUNE_COUNT] = {200000, 0, 1, 0, 1, 0, 0, 0};
 extern "C" int pe_set_tuning(int key, int value)
 {
     PE_CHECK(key >= 0 && key < PE_TUNE_COUNT, "bad tuning key");
@@ -136,6 +137,17 @@ extern "C" int pe_set_tuning(int key, int value)
     return 0;
 }
 extern "C" int pe_get_tuning(int key) { return key >= 0 && key < PE_TUNE_COUNT ? g_tuning[key] : 0; }
+
+static std::atomic<int64_t> g_variant[PE_VARIANT_COUNT];
+void pe_variant_add(int slot, int64_t count) { g_variant[slot].fetch_add(count, std::memory_order_relaxed); }
+extern "C" int pe_variant_counts(int64_t *out, int n, int reset)
+{
+    PE_CHECK(n >= 0 && (out || n == 0), "pe_variant_counts: bad arguments");
+    for (int k = 0; k < n; ++k) out[k] = k < PE_VARIANT_COUNT ? g_variant[k].load(std::memory_order_relaxed) : 0;
+    if (reset)
+        for (auto &c : g_variant) c.store(0, std::memory_order_relaxed);
+    return 0;
+}
 
 extern "C" int pe_ctx_sync(pe_ctx *c)
 {

@@ -243,6 +243,7 @@ int pe_halo_wait(pe_mat *A);                           // compute stream waits f
 int pe_devcsr_transpose(pe_ctx *ctx, const DevCSR &A, DevCSR &T);
 int pe_devcsr_spgemm(pe_ctx *ctx, const DevCSR &A, const DevCSR &B, DevCSR &C);
 int pe_choose_tpr(int64_t nnz, int32_t nrows);
+void pe_variant_add(int slot, int64_t count);   // pe_variant_counts: rows / agglomerates handed to one kernel variant
 int pe_mat_wrap_local(pe_ctx *ctx, DevCSR &diag, pe_mat **out);  // takes ownership of diag
 int pe_allreduce_sum(pe_ctx *ctx, double *d, int count);
 

@@ -824,6 +824,13 @@ namespace
 // [1] kernel, [2] D2H of the results, [3] bytes uploaded, [4] bytes downloaded, [5] calls
 static double g_stage[6] = {0, 0, 0, 0, 0, 0};
 static double now_s() { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); }
+// workspace bytes above which an agglomerate goes to the global-memory kernel: the built-in limit, or PE_TUNE_LOCAL_SMEM_BYTES
+// when that is set (clamped to the built-in limit)
+static size_t local_smem_limit(size_t builtin)
+{
+    const int v = pe_get_tuning(PE_TUNE_LOCAL_SMEM_BYTES);
+    return v > 0 ? std::min(builtin, (size_t)v) : builtin;
+}
 // Device copies of inputs that stay constant over one Coarsen() (entity mass pools, agglomerate tables, the
 // fine D_j): uploaded once per pe_local_cache(1) ... pe_local_cache(0) scope and shared by the per-form,
 // per-codimension batched calls, keyed by host address and size.  At 144^3 hexahedra the 24 extension
@@ -978,15 +985,18 @@ extern "C" int pe_batched_traces(pe_ctx *ctx, const pe_trace_batch *b)
     const int nT1 = b->nT > 0 ? b->nT : 1, ncm = b->nT + 1;
     size_t smem = sizeof(double) * ((size_t)max_m * nT1 + 2 * (size_t)max_m + nT1 + 2 * (size_t)max_m * ncm + (size_t)ncm * ncm + (size_t)max_m * ncm
                                     + 3 * (size_t)a.max_md * a.max_md + (size_t)a.max_md);
-    if (smem <= 200 * 1024)
+    if (smem <= local_smem_limit(200 * 1024))
     {
+        pe_variant_add(PE_VARIANT_TRACES_SMEM, b->nAE);
         PE_CUDA(cudaFuncSetAttribute(k_traces, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         k_traces<<<b->nAE, 32, smem, st>>>(a);
     }
     else
     {
+        pe_variant_add(PE_VARIANT_TRACES_GMEM, b->nAE);
         // agglomerated entity too large for shared memory (coarse levels with many dofs per entity): global workspace
         const int grid = std::min(b->nAE, 148 * 16);
+        pe_variant_add(PE_VARIANT_TRACES_GMEM_REUSE, b->nAE - grid);
         const size_t stride = (smem / sizeof(double) + 31) & ~(size_t)31;
         double *work = nullptr;
         PE_TRY(D.alloc(stride * (size_t)grid, &work));
@@ -1098,7 +1108,7 @@ extern "C" int pe_batched_extension(pe_ctx *ctx, const pe_extension_batch *b)
                           + (size_t)std::max(B.mxu, B.mxp) * (lbmax > 0 ? lbmax : 1) + lbmax * lbmax + (size_t)B.mxq * B.mxq + 2 * (size_t)B.mxq * B.mxpi + nT1;
         return sizeof(double) * nd + sizeof(int) * ((size_t)B.mxu + B.mxp + B.mxq + B.mxcb) + 16;
     };
-    const size_t SMEM_LIMIT = 220 * 1024;
+    const size_t SMEM_LIMIT = local_smem_limit(220 * 1024);
     Bounds all, fit, big;
     std::vector<int> fit_list, big_list;
     for (int e = 0; e < nAE; ++e) grow(all, e);
@@ -1118,6 +1128,8 @@ extern "C" int pe_batched_extension(pe_ctx *ctx, const pe_extension_batch *b)
     auto set_bounds = [&](const Bounds &B) { a.mxu = B.mxu; a.mxp = B.mxp; a.mxq = B.mxq; a.mxui = B.mxui; a.mxpi = B.mxpi; a.mxcb = B.mxcb; a.mxrt = B.mxrt; };
     PE_CUDA(cudaStreamSynchronize(st));
     const double t_up = now_s();
+    pe_variant_add(PE_VARIANT_EXT_SMEM, big_list.empty() ? nAE : (int64_t)fit_list.size());
+    pe_variant_add(PE_VARIANT_EXT_GMEM, (int64_t)big_list.size());
     if (big_list.empty())
     {
         set_bounds(all);
@@ -1133,6 +1145,7 @@ extern "C" int pe_batched_extension(pe_ctx *ctx, const pe_extension_batch *b)
             set_bounds(fit);
             const size_t smem = bytes_of(fit);
             PE_TRY(D.up(fit_list.data(), fit_list.size(), &list_d));
+            pe_variant_add(PE_VARIANT_EXT_SPLIT_SMEM, (int64_t)fit_list.size());
             PE_CUDA(cudaFuncSetAttribute(k_extension, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
             k_extension<<<(int)fit_list.size(), LT, smem, st>>>(a, list_d, (int)fit_list.size());
             PE_LAUNCHED(ctx);
@@ -1140,6 +1153,7 @@ extern "C" int pe_batched_extension(pe_ctx *ctx, const pe_extension_batch *b)
         set_bounds(big);
         const size_t stride = (bytes_of(big) / sizeof(double) + 31) & ~(size_t)31;
         const int grid = std::min((int)big_list.size(), 148 * 4);
+        pe_variant_add(PE_VARIANT_EXT_GMEM_REUSE, (int64_t)big_list.size() - grid);
         double *work = nullptr;
         PE_TRY(D.alloc(stride * (size_t)grid, &work));
         PE_TRY(D.up(big_list.data(), big_list.size(), &list_d));

@@ -962,6 +962,7 @@ static int launch_gs_set(pe_smoother *s, int k0, int k1, const double *f, double
         return 0;
     }
     int tpr = s->tpr;
+    pe_variant_add(PE_VARIANT_RELAX_TPR_1 + __builtin_ctz(tpr), rows);
     int grid = pe_grid_for((int64_t)rows * tpr, 256);
     int ncd = s->A->diag.ncols;
 #define LAUNCH(T) PE_CUDA(pe_launch_k(ctx, k_gs_set<T, GENERAL>, grid, 256, k0, k1, s->P.I, s->P.J, s->P.A, s->perm_d, ncd, f, u, s->A->x_ext_d, s->l1_d, s->before_d, forward, s->w_d, c1, c2))
@@ -1036,6 +1037,7 @@ extern "C" int pe_smoother_apply(pe_smoother *s, const pe_vec *b, pe_vec *x, int
         if (s->type == 0 || s->type == 1 || s->type == 5) {
             PE_TRY(sweep_halo(A, x->d, !iterative_mode && sweep == 0));
             int tpr = A->tpr;
+            pe_variant_add(PE_VARIANT_RELAX_TPR_1 + __builtin_ctz(tpr), n);
             int64_t threads = (int64_t)n * tpr;
             int grid = (int)std::min<int64_t>((threads + 255) / 256, (int64_t)PE_SM_COUNT * 64);
             if (grid < 1) grid = 1;

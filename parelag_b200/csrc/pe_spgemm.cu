@@ -228,6 +228,7 @@ static int run_bins(pe_ctx *ctx, int n, const int *size_d, const DevCSR &A, cons
     int counts[4];
     PE_CUDA(cudaMemcpyAsync(counts, counts_d, sizeof(int) * 4, cudaMemcpyDeviceToHost, st));
     PE_CUDA(cudaStreamSynchronize(st));
+    for (int b = 0; b < 4; ++b) pe_variant_add((NUMERIC ? PE_VARIANT_SPGEMM_NUM_T128 : PE_VARIANT_SPGEMM_SYM_T128) + b, counts[b]);
     const int *CI = C ? C->I : nullptr;
     int *CJ = C ? C->J : nullptr;
     double *CA = C ? C->A : nullptr;

@@ -112,6 +112,7 @@ int pe_launch_spmv(pe_ctx *ctx, const DevCSR &diag, const DevCSR *offd, int tpr,
     if (!oI && diag.sell_state == 0) PE_TRY(pe_sell_for_spmv(ctx, const_cast<DevCSR &>(diag)));
     if (!oI && diag.sell)
     {
+        pe_variant_add(PE_VARIANT_SPMV_SELL, n);
         PE_TRY(pe_prof_begin(ctx, 0, 12.0 * (double)diag.nnz + 4.0 * (n + 1) + 8.0 * diag.ncols + 8.0 * n + (beta != 0.0 ? 8.0 * n : 0.0)));
         PE_TRY(pe_launch_sell_spmv(ctx, *diag.sell, alpha, x, beta, yin, yout));
         PE_TRY(pe_prof_end(ctx));
@@ -120,6 +121,7 @@ int pe_launch_spmv(pe_ctx *ctx, const DevCSR &diag, const DevCSR *offd, int tpr,
     if (ctx->rec && !oI)
     {
         // persistent program: CSR-vector op (the CTA-tiled streaming kernel has no op equivalent)
+        pe_variant_add(PE_VARIANT_SPMV_VECTOR, n);
         PeOp o = pe_op(PE_OP_CSR_SPMV); o.i0 = n; o.i1 = pe_choose_tpr(diag.nnz, n); o.a = alpha; o.b = beta;
         o.p[0] = diag.I; o.p[1] = diag.J; o.p[2] = diag.A; o.p[3] = x; o.p[4] = yin; o.p[5] = yout;
         pe_rec_push(ctx, o, 12.0 * (double)diag.nnz + 4.0 * (n + 1) + 8.0 * diag.ncols + 8.0 * n + (beta != 0.0 ? 8.0 * n : 0.0));
@@ -128,12 +130,14 @@ int pe_launch_spmv(pe_ctx *ctx, const DevCSR &diag, const DevCSR *offd, int tpr,
     if (!oI && diag.nrb == 0 && diag.nnz > 0) PE_TRY(pe_build_row_blocks(ctx, const_cast<DevCSR &>(diag), nullptr));
     if (!oI && diag.nrb > 0)
     {
+        pe_variant_add(PE_VARIANT_SPMV_STREAM, n);
         PE_TRY(pe_prof_begin(ctx, 0, 12.0 * (double)diag.nnz + 4.0 * (n + 1) + 8.0 * diag.ncols + 8.0 * n + (beta != 0.0 ? 8.0 * n : 0.0)));
         PE_CUDA(pe_launch_k(ctx, k_spmv_stream, diag.nrb, 256, diag.rb, diag.I, diag.J, diag.A, x, alpha, beta, yin, yout));
         PE_LAUNCHED(ctx);
         PE_TRY(pe_prof_end(ctx));
         return 0;
     }
+    pe_variant_add(PE_VARIANT_SPMV_VECTOR, n);
     int64_t threads = (int64_t)n * tpr;
     int64_t cap = (int64_t)PE_SM_COUNT * 8 * 8;     // 8 CTAs of 256 threads per SM, x8 waves
     int grid = (int)std::min<int64_t>((threads + 255) / 256, cap);

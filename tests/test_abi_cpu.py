@@ -23,3 +23,25 @@ def test_no_cpu_fallback_without_device():
         assert "no CUDA device" in str(e) or "CUDA" in str(e)
     else:
         raise AssertionError("context creation must fail loudly without a CUDA device")
+
+
+def _header_enum(first, last):
+    """name -> value of an enum in include/parelag_b200.h, from `first` to `last`"""
+    import re
+    text = open(capi.HEADER_PATHS[1]).read()
+    body = text[text.index(first):text.index(last)]
+    return {m.group(1): int(m.group(2)) for m in re.finditer(r"PE_(?:VARIANT|TUNE)_(\w+)\s*=\s*(\d+)", body)}
+
+
+def test_variant_counter_slots_match_the_header():
+    """capi's slot constants are the header's enum; the counters are host integers, readable and resettable without a
+    device"""
+    slots = _header_enum("PE_VARIANT_SPMV_SELL", "int pe_variant_counts")
+    assert slots.pop("COUNT") == len(capi.VARIANT_SLOTS)
+    assert slots == {name: getattr(capi, name) for name in capi.VARIANT_SLOTS}
+    assert [slots[n] for n in capi.VARIANT_SLOTS] == list(range(len(capi.VARIANT_SLOTS)))
+    capi.variant_counts(reset=True)
+    assert not capi.variant_counts().any()
+    tune = _header_enum("PE_TUNE_SELL_MIN_ROWS", "int pe_set_tuning")
+    assert tune["LOCAL_SMEM_BYTES"] == capi.TUNE_LOCAL_SMEM_BYTES and tune["COUNT"] == capi.TUNE_LOCAL_SMEM_BYTES + 1
+    assert capi.get_tuning(capi.TUNE_LOCAL_SMEM_BYTES) == 0

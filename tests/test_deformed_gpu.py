@@ -9,7 +9,7 @@ import pytest
 import scipy.sparse as sp
 import scipy.sparse.linalg as spl
 
-from parelag_b200 import api
+from parelag_b200 import api, capi
 from oracle import amge
 from tests.test_coarsen_gpu import compare_levels
 
@@ -79,7 +79,9 @@ def test_deformed_mesh_hcurl_levels_take_the_dense_weighted_trace_svd():
     finally:
         amge.svd_on_weighted = orig
     assert dense["n"] > 0                                       # the oracle really takes the dense-weighted path
+    capi.variant_counts(reset=True)
     S = api.Sequence.hex(dims, nlev, jstart=1, alpha=alpha, beta=beta, coords=mesh.vertex_coords())
+    assert capi.variant_counts()[capi.EXT_GMEM] > 0
     assert S.stat(2, "trace_dense_mass_1") + S.stat(2, "trace_dense_mass_2") == dense["n"]
     compare_levels(S, seqs, tol=1e-10, null_tol=1e-7)
     # CheckInvariants on the product's own operators (DeRhamSequence.cpp:694-970)

@@ -265,13 +265,17 @@ def test_rap_pattern_bit_exact_values_1e12(ctx, dims):
 
 
 def test_spgemm_long_rows_use_bigger_tables(ctx):
-    """rows with hundreds / thousands of products exercise the 1024- and 8192-slot
-    shared tables and the global-memory table."""
+    """rows with ~60 000 products and ~5 000 distinct columns: more than the 8192-slot shared table takes, so every
+    row of both passes uses the global-memory table (the shared tables: tests/test_variants_gpu.py)."""
     rng = np.random.default_rng(8)
     A = sp.random(40, 3000, density=0.2, random_state=rng, format="csr")
     B = sp.random(3000, 5000, density=0.02, random_state=rng, format="csr")
     dA, dB = capi.Mat.from_scipy(ctx, A), capi.Mat.from_scipy(ctx, B)
+    capi.variant_counts(reset=True)
     Cg = capi.spgemm(ctx, dA, dB).to_scipy()
+    c = capi.variant_counts()
+    assert list(c[[capi.SPGEMM_SYM_T128, capi.SPGEMM_SYM_T1024, capi.SPGEMM_SYM_T8192, capi.SPGEMM_SYM_GMEM]]) == [0, 0, 0, 40]
+    assert list(c[[capi.SPGEMM_NUM_T128, capi.SPGEMM_NUM_T1024, capi.SPGEMM_NUM_T8192, capi.SPGEMM_NUM_GMEM]]) == [0, 0, 0, 40]
     Co = orc.spgemm(A, B)
     assert np.array_equal(Cg.indptr, Co.indptr) and np.array_equal(Cg.indices, Co.indices)
     assert np.max(np.abs(Cg.data - Co.data)) <= 1e-12 * np.max(np.abs(Co.data))

@@ -205,6 +205,11 @@ int pe_api_solver_num_levels(const pe_solver *s, int *nlevels);
 /* Hierarchy solvers: the persistent program the V-cycle was recorded into (NULL until the third
  * preconditioner application with the same buffers, or when recording was not possible) */
 int pe_api_solver_program(const pe_solver *s, pe_program **out);
+/* Hierarchy solvers: how the last preconditioner-mode V-cycle (Mult with iterative_mode off, e.g.
+ * pe_api_solver_prec_mult_device) ran: 0 directly, 1 as a replayed or just-recorded CUDA graph, 2 as the
+ * persistent program.  A host-side value: no device work, no synchronisation. */
+enum { PE_REPLAY_DIRECT = 0, PE_REPLAY_GRAPH = 1, PE_REPLAY_PROGRAM = 2 };
+int pe_api_solver_replay_mode(const pe_solver *s, int *mode);
 int pe_api_solver_level_info(const pe_solver *s, int level, int64_t *nrows, int64_t *nnz, int64_t *nnz_P);
 /* download A (diag block) of a hierarchy level for parity tests; arrays sized from level_info */
 int pe_api_solver_level_matrix(const pe_solver *s, int level, int32_t *I, int32_t *J, double *A);

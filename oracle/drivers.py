@@ -40,25 +40,36 @@ def bdr_mask(dofhandler):
     return mask
 
 
+# "Type" of the Hypre smoother factory -> hypre relaxation type (ParELAG_HypreSmootherFactory.cpp:27-31)
+SMOOTHER_TYPES = {"Jacobi": 0, "L1 Jacobi": 1, "L1 Gauss-Seidel": 2, "L1 Gauss-Seidel Truncated": 4, "Lumped Jacobi": 5,
+                  "Gauss-Seidel": 6, "Chebyshev": 16, "Hypre Jacobi": 413}
+
+
 def gs_order(A, ordering):
     return None if ordering == "natural" else orc.multicolor_order(A)[0]
 
 
 def amge_pcg_solver(seqs, form, ess_attr, A, ordering="natural", smoother_type=2,
-                    coarse_its=3, coarse_tol=1e-4, hiptmair=None):
-    """Returns (prec, info): prec(r) = one AMGe V-cycle.  hiptmair defaults to form>0."""
+                    coarse_its=3, coarse_tol=1e-4, hiptmair=None, damping=1.0, omega=1.0, cheby_order=2):
+    """Returns (prec, info): prec(r) = one AMGe V-cycle.  hiptmair defaults to form>0.  smoother_type: a hypre
+    relaxation type or a name of SMOOTHER_TYPES; damping, omega and cheby_order as "Damping Factor", "Omega" and
+    "Cheby Poly Order" of library_entries."""
     hiptmair = (form > 0) if hiptmair is None else hiptmair
+    stype = SMOOTHER_TYPES[smoother_type] if isinstance(smoother_type, str) else smoother_type
     nl = len(seqs)
     Ps = [seqs[l].get_P(form, ess_attr) for l in range(nl - 1)]
 
+    def kw(M):
+        return dict(type=stype, damping=damping, omega=omega, cheby_order=cheby_order,
+                    order=gs_order(M, ordering) if stype in (2, 4, 6) else None)
+
     def hypre(Al):
-        return orc.Smoother(Al, type=smoother_type, order=gs_order(Al, ordering))
+        return orc.Smoother(Al, **kw(Al))
 
     def make_smoother(l, Al):
         if not hiptmair:
             return hypre(Al)
         Dl = seqs[l].get_D(form - 1, ess_attr)
-        kw = lambda M: dict(type=smoother_type, order=gs_order(M, ordering))
         return orc.Hiptmair(Al, Dl, kw, kw)
 
     def make_coarse(Ac):
@@ -73,12 +84,13 @@ def amge_pcg_solver(seqs, form, ess_attr, A, ordering="natural", smoother_type=2
 
 
 def library_entries(form, ordering="natural", smoother="L1 Gauss-Seidel", coarse_its=3, coarse_tol=1e-4,
-                    rtol=1e-6, atol=1e-6, max_iter=300):
-    """The same solver as a ParElag 'Preconditioner Library' (dict for api.library_xml)."""
-    hyp = ("Hypre", {"Type": smoother, "Sweeps": 1, "Damping Factor": 1.0, "Omega": 1.0,
-                     "Cheby Poly Order": 2, "Cheby Poly Fraction": 0.3, "GS ordering": ordering})
+                    rtol=1e-6, atol=1e-6, max_iter=300, damping=1.0, omega=1.0, cheby_order=2, hiptmair=None):
+    """The same solver as a ParElag 'Preconditioner Library' (dict for api.library_xml).  hiptmair defaults to form>0."""
+    hiptmair = (form > 0) if hiptmair is None else hiptmair
+    hyp = ("Hypre", {"Type": smoother, "Sweeps": 1, "Damping Factor": float(damping), "Omega": float(omega),
+                     "Cheby Poly Order": int(cheby_order), "Cheby Poly Fraction": 0.3, "GS ordering": ordering})
     lib = {"Gauss-Seidel": hyp}
-    if form > 0:
+    if hiptmair:
         lib["Hiptmair-GS-GS"] = ("Hiptmair", {"Primary Smoother": "Gauss-Seidel", "Auxiliary Smoother": "Gauss-Seidel"})
         smoo = "Hiptmair-GS-GS"
     else:

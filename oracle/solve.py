@@ -176,7 +176,9 @@ def hypre_rand_vector(n, seed=1):
 
 
 class Smoother:
-    """mfem::HypreSmoother as configured by parelag::HypreSmootherWrapper."""
+    """mfem::HypreSmoother as configured by parelag::HypreSmootherWrapper.  type 413 ("Hypre Jacobi") is
+    mfem::HypreDiagScale: x = diag(A)^{-1} b, one unit-weight Jacobi sweep from a zero guess whatever the
+    initial guess, sweeps and damping."""
 
     def __init__(self, A, type=2, sweeps=1, damping=1.0, omega=1.0, cheby_order=2,
                  cheby_fraction=0.3, order=None, ranks=1):
@@ -188,7 +190,9 @@ class Smoother:
         self.A = A.tocsr()
         self.n, self.I, self.J, self.D = _csr(self.A)
         self.type, self.sweeps, self.w, self.omega = type, sweeps, damping, omega
-        l1opt = 0 if type in (0, 6, 16) else type
+        if type == 413:
+            self.sweeps, self.w = 1, 1.0
+        l1opt = 0 if type in (0, 6, 16, 413) else type
         self.l1 = l1_norms(self.A, l1opt)
         if ranks > 1:
             assert type == 2 and order is None
@@ -218,6 +222,9 @@ class Smoother:
             s = r.copy()
             gamma_old = gamma
             gamma = float(r @ s)
+            if i > 0 and gamma < 2.220446049250313e-16:     # residual gone: the Lanczos matrix so far
+                max_iter = i
+                break
             if i == 0:
                 beta = 1.0
                 p = s.copy()
@@ -241,11 +248,11 @@ class Smoother:
     def apply(self, b, x, iterative_mode=True):
         b = np.ascontiguousarray(b, dtype=np.float64)
         x = np.ascontiguousarray(x, dtype=np.float64).copy()
-        if not iterative_mode:
+        if not iterative_mode or self.type == 413:
             x[:] = 0.0
         n = self.n
         for _ in range(self.sweeps):
-            if self.type in (0, 1, 5):
+            if self.type in (0, 1, 5, 413):
                 v = np.empty(n)
                 lib().orc_relax_jacobi(n, _p(self.I), _p(self.J), _p(self.D), None, None, None,
                                        _p(self.l1), C.c_double(self.w), _p(b), _p(x), None, _p(v))
@@ -381,7 +388,8 @@ def pcg(A, prec, b, rtol=1e-6, atol=1e-6, max_iter=300, x0=None):
         return x, 0, True, hist
     z = Amul(d)
     den = float(z @ d)
-    if den <= 0:
+    # a negative (Ad, d) is only reported by MFEM and the iteration goes on; an exact zero stops it
+    if den == 0:
         return x, 0, False, hist
     i = 1
     converged = False
@@ -402,7 +410,7 @@ def pcg(A, prec, b, rtol=1e-6, atol=1e-6, max_iter=300, x0=None):
         d = z + beta * d
         z = Amul(d)
         den = float(d @ z)
-        if den <= 0:
+        if den == 0:
             break
         nom = betanom
     return x, min(i, max_iter), converged, hist

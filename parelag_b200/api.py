@@ -416,6 +416,12 @@ class Solver:
         _chk(lib().pe_program_info(h, C.byref(n), C.byref(b)))
         return n.value, b.value
 
+    def replay_mode(self):
+        """How the last preconditioner-mode V-cycle ran: "direct", "graph" or "program" (capi.REPLAY_*)."""
+        m = C.c_int()
+        _chk(lib().pe_api_solver_replay_mode(self.h, C.byref(m)))
+        return capi.REPLAY_MODE_NAMES[m.value]
+
     def program_profile(self, ctx):
         """One extra program launch with per-op device timestamps: (types, usec, bytes) arrays."""
         h = C.c_void_p()

@@ -147,6 +147,12 @@ def get_tuning(key):
     return lib().pe_get_tuning(key)
 
 
+# pe_api_solver_replay_mode values (include/parelag_b200_api.h): how the last preconditioner-mode V-cycle ran
+REPLAY_DIRECT = 0
+REPLAY_GRAPH = 1
+REPLAY_PROGRAM = 2
+REPLAY_MODE_NAMES = {REPLAY_DIRECT: "direct", REPLAY_GRAPH: "graph", REPLAY_PROGRAM: "program"}
+
 # slots of pe_variant_counts (include/parelag_b200.h)
 VARIANT_SLOTS = ("SPMV_SELL", "SPMV_STREAM", "SPMV_VECTOR",
                  "SPGEMM_SYM_T128", "SPGEMM_SYM_T1024", "SPGEMM_SYM_T8192", "SPGEMM_SYM_GMEM",

@@ -731,6 +731,9 @@ static int cheby_setup(pe_smoother *s)
     for (int i = 0; i < max_iter; ++i) {
         gamma_old = gamma;
         PE_TRY(dot_dev(ctx, n, r, r, &gamma));
+        // stop once the residual vanishes (the start vector spans fewer than max_iter eigenvectors, as on
+        // a small coarse level); the Lanczos matrix of the steps taken holds the estimate.  Going on divides 0 by 0.
+        if (i > 0 && gamma < 2.220446049250313e-16) { max_iter = i; break; }
         pe_vec vr{ctx, n, r}, vp{ctx, n, p}, vs{ctx, n, sv};
         if (i == 0) { beta = 1.0; PE_TRY(pe_vec_copy(&vr, &vp)); }
         else { beta = gamma / gamma_old; PE_TRY(pe_vec_axpby(1.0, &vr, beta, &vp)); }

@@ -55,6 +55,9 @@ __device__ __forceinline__ double ld_nc_f64_pro(const double *p)
 // scalar recurrences of mfem::CGSolver::Mult, one phase per call (single thread)
 //  phase 0: DOT = (d, r) before the loop        phase 1: DOT = (z, d) before the loop
 //  phase 2: DOT = (r, z) in iteration `iter`    phase 3: DOT = (d, z) in iteration `iter`
+// As in mfem (and KrylovSolver::Mult on the host): a negative initial (B r, r) stops at once (FetchStats
+// reports it as the final norm, unsquared); a negative (Ad, d) continues with a negative step; only an
+// exact zero (Ad, d) stops, unconverged, with final_iter the iteration that computed it.
 __device__ __forceinline__ void pe_pcg_scalar_step_dev(double *s, int phase, int iter, int max_iter, double rel, double abs_tol)
 {
     const double dot = s[PE_PCG_DOT];
@@ -75,7 +78,7 @@ __device__ __forceinline__ void pe_pcg_scalar_step_dev(double *s, int phase, int
         if (!done)
         {
             s[PE_PCG_DEN] = dot;
-            if (dot <= 0.0) done = true;
+            if (dot == 0.0) done = true;
             else s[PE_PCG_ALPHA] = s[PE_PCG_NOM] / dot;
         }
     }
@@ -95,7 +98,7 @@ __device__ __forceinline__ void pe_pcg_scalar_step_dev(double *s, int phase, int
         if (!done)
         {
             s[PE_PCG_DEN] = dot;
-            if (dot <= 0.0) { done = true; s[PE_PCG_FINAL_ITER] = (double)max_iter; }
+            if (dot == 0.0) { done = true; s[PE_PCG_FINAL_ITER] = (double)(iter + 1); }
             else { s[PE_PCG_NOM] = s[PE_PCG_BETANOM]; s[PE_PCG_ALPHA] = s[PE_PCG_BETANOM] / dot; }
         }
     }

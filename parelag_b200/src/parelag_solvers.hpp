@@ -664,7 +664,8 @@ private:
         history_.assign(h.begin() + PE_PCG_HIST, h.begin() + PE_PCG_HIST + nh);
         converged_ = h[PE_PCG_CONVERGED] != 0.0;
         final_iter_ = (int)h[PE_PCG_FINAL_ITER];
-        final_norm_ = std::sqrt(std::fabs(h[PE_PCG_BETANOM]));
+        // a negative initial (B r, r) stops at once and is reported as it is, as Mult does
+        final_norm_ = h[PE_PCG_NOM0] < 0.0 ? h[PE_PCG_NOM0] : std::sqrt(std::fabs(h[PE_PCG_BETANOM]));
         stats_on_device_ = false;
     }
     void _do_set_operator(const Op_Ptr &op) override { A_ = op; }
@@ -765,6 +766,8 @@ public:
     bool UsesGraph() const noexcept { return graph_ != nullptr; }
     bool UsesProgram() const noexcept { return program_ != nullptr; }
     pe_program *GetProgram() const noexcept { return program_; }
+    /// how the last preconditioner-mode Mult ran: 0 directly, 1 as a CUDA graph, 2 as the persistent program
+    int LastReplayMode() const noexcept { return last_mode_; }
     bool CaptureSafe() const override
     {
         for (auto &lev : Levels_)
@@ -854,6 +857,7 @@ private:
     bool ReplayGraph(const mfem::Vector &rhs, mfem::Vector &sol) const
     {
         pe_ctx *ctx = Device::Get();
+        last_mode_ = 0;
         if ((!use_graph_ || graph_failed_) && (!use_program_ || program_failed_)) return false;
         if (pe_ctx_is_capturing(ctx) || pe_ctx_is_recording(ctx) || pe_ctx_is_profiling(ctx)) return false;
         // multi-rank: the NCCL halo exchanges and all-reduces are captured with the kernels (every
@@ -866,11 +870,13 @@ private:
         if (program_ && graph_rhs_ == rp && graph_sol_ == sp)
         {
             PE_CALL(pe_program_launch(ctx, program_));
+            last_mode_ = 2;
             return true;
         }
         if (graph_ && graph_rhs_ == rp && graph_sol_ == sp)
         {
             PE_CALL(pe_graph_launch(ctx, graph_));
+            last_mode_ = 1;
             return true;
         }
         if (warm_rhs_ != rp || warm_sol_ != sp) { warm_rhs_ = rp; warm_sol_ = sp; return false; }
@@ -889,6 +895,7 @@ private:
             {
                 program_ = p; graph_rhs_ = rp; graph_sol_ = sp;
                 PE_CALL(pe_program_launch(ctx, program_));
+                last_mode_ = 2;
                 return true;
             }
             pe_program_free(p);
@@ -908,6 +915,7 @@ private:
         }
         graph_ = g; graph_rhs_ = rp; graph_sol_ = sp;
         PE_CALL(pe_graph_launch(ctx, graph_));
+        last_mode_ = 1;
         return true;
     }
     void DropRecordedCycle() const
@@ -925,6 +933,7 @@ private:
     mutable bool graph_failed_ = false, program_failed_ = false;
     mutable pe_program *program_ = nullptr;
     mutable int capture_safe_ = -1;
+    mutable int last_mode_ = 0;                 // LastReplayMode()
     mutable pe_graph *graph_ = nullptr;
     mutable const void *graph_rhs_ = nullptr, *graph_sol_ = nullptr, *warm_rhs_ = nullptr, *warm_sol_ = nullptr;
 };

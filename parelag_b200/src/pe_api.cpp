@@ -741,6 +741,12 @@ extern "C" int pe_api_solver_program(const pe_solver *s, pe_program **out)
     *out = as_hierarchy(s)->GetProgram();
     API_CATCH
 }
+extern "C" int pe_api_solver_replay_mode(const pe_solver *s, int *mode)
+{
+    API_TRY
+    *mode = as_hierarchy(s)->LastReplayMode();
+    API_CATCH
+}
 extern "C" int pe_api_solver_level_info(const pe_solver *s, int level, int64_t *nrows, int64_t *nnz, int64_t *nnz_P)
 {
     API_TRY

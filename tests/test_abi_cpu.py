@@ -9,6 +9,7 @@ def test_library_exports_every_declared_symbol():
     lib = capi.lib()
     names = capi.declared_symbols()
     assert len(names) > 30
+    assert "pe_api_solver_replay_mode" in names
     missing = [n for n in names if not hasattr(lib, n)]
     assert not missing, "declared in include/*.h but not exported: %s" % missing
 
@@ -45,3 +46,12 @@ def test_variant_counter_slots_match_the_header():
     tune = _header_enum("PE_TUNE_SELL_MIN_ROWS", "int pe_set_tuning")
     assert tune["LOCAL_SMEM_BYTES"] == capi.TUNE_LOCAL_SMEM_BYTES and tune["COUNT"] == capi.TUNE_LOCAL_SMEM_BYTES + 1
     assert capi.get_tuning(capi.TUNE_LOCAL_SMEM_BYTES) == 0
+
+
+def test_replay_mode_values_match_the_header():
+    """the mode names api.Solver.replay_mode() returns are keyed by the header's PE_REPLAY_* values"""
+    import re
+    text = open(capi.HEADER_PATHS[2]).read()
+    vals = {m.group(1): int(m.group(2)) for m in re.finditer(r"PE_REPLAY_(\w+)\s*=\s*(\d+)", text)}
+    assert vals == {"DIRECT": capi.REPLAY_DIRECT, "GRAPH": capi.REPLAY_GRAPH, "PROGRAM": capi.REPLAY_PROGRAM}
+    assert sorted(capi.REPLAY_MODE_NAMES) == sorted(vals.values())

@@ -127,7 +127,8 @@ int pe_get_tuning(int key);
  * when it is recorded.  Three slots refine the local solves: EXT_SPLIT_SMEM counts the agglomerates of the listed
  * shared-memory extension launch of a batch split between both kernels (also counted in EXT_SMEM); TRACES_GMEM_REUSE and
  * EXT_GMEM_REUSE count the agglomerates a global-workspace CTA takes after its first one (a launch with more agglomerates
- * than CTAs reuses each workspace slab).  out: n slots (slots past PE_VARIANT_COUNT are set to 0; NULL with n = 0 copies nothing);
+ * than CTAs reuses each workspace slab).  SPMV_SELL_SIGNS counts the rows of SELL SpMVs whose values are stored as int8
+ * sign codes (every value -1, 0 or +1; also counted in SPMV_SELL).  out: n slots (slots past PE_VARIANT_COUNT are set to 0; NULL with n = 0 copies nothing);
  * reset != 0 zeroes every counter after the copy. */
 enum { PE_VARIANT_SPMV_SELL = 0, PE_VARIANT_SPMV_STREAM = 1, PE_VARIANT_SPMV_VECTOR = 2,
        PE_VARIANT_SPGEMM_SYM_T128 = 3, PE_VARIANT_SPGEMM_SYM_T1024 = 4, PE_VARIANT_SPGEMM_SYM_T8192 = 5, PE_VARIANT_SPGEMM_SYM_GMEM = 6,
@@ -136,7 +137,7 @@ enum { PE_VARIANT_SPMV_SELL = 0, PE_VARIANT_SPMV_STREAM = 1, PE_VARIANT_SPMV_VEC
        PE_VARIANT_RELAX_TPR_16 = 15, PE_VARIANT_RELAX_TPR_32 = 16,
        PE_VARIANT_TRACES_SMEM = 17, PE_VARIANT_TRACES_GMEM = 18, PE_VARIANT_EXT_SMEM = 19, PE_VARIANT_EXT_GMEM = 20,
        PE_VARIANT_EXT_SPLIT_SMEM = 21, PE_VARIANT_TRACES_GMEM_REUSE = 22, PE_VARIANT_EXT_GMEM_REUSE = 23,
-       PE_VARIANT_COUNT = 24 };
+       PE_VARIANT_SPMV_SELL_SIGNS = 24, PE_VARIANT_COUNT = 25 };
 int pe_variant_counts(int64_t *out, int n, int reset);
 /* write a scratch buffer larger than L2 (bench hygiene) */
 int pe_ctx_flush_l2(pe_ctx *ctx);

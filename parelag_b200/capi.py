@@ -159,13 +159,13 @@ VARIANT_SLOTS = ("SPMV_SELL", "SPMV_STREAM", "SPMV_VECTOR",
                  "SPGEMM_NUM_T128", "SPGEMM_NUM_T1024", "SPGEMM_NUM_T8192", "SPGEMM_NUM_GMEM",
                  "RELAX_TPR_1", "RELAX_TPR_2", "RELAX_TPR_4", "RELAX_TPR_8", "RELAX_TPR_16", "RELAX_TPR_32",
                  "TRACES_SMEM", "TRACES_GMEM", "EXT_SMEM", "EXT_GMEM",
-                 "EXT_SPLIT_SMEM", "TRACES_GMEM_REUSE", "EXT_GMEM_REUSE")
+                 "EXT_SPLIT_SMEM", "TRACES_GMEM_REUSE", "EXT_GMEM_REUSE", "SPMV_SELL_SIGNS")
 (SPMV_SELL, SPMV_STREAM, SPMV_VECTOR,
  SPGEMM_SYM_T128, SPGEMM_SYM_T1024, SPGEMM_SYM_T8192, SPGEMM_SYM_GMEM,
  SPGEMM_NUM_T128, SPGEMM_NUM_T1024, SPGEMM_NUM_T8192, SPGEMM_NUM_GMEM,
  RELAX_TPR_1, RELAX_TPR_2, RELAX_TPR_4, RELAX_TPR_8, RELAX_TPR_16, RELAX_TPR_32,
  TRACES_SMEM, TRACES_GMEM, EXT_SMEM, EXT_GMEM,
- EXT_SPLIT_SMEM, TRACES_GMEM_REUSE, EXT_GMEM_REUSE) = range(len(VARIANT_SLOTS))
+ EXT_SPLIT_SMEM, TRACES_GMEM_REUSE, EXT_GMEM_REUSE, SPMV_SELL_SIGNS) = range(len(VARIANT_SLOTS))
 
 
 def variant_counts(reset=False):

@@ -52,7 +52,7 @@ void pe_set_error(const std::string &msg);
 enum PeOpType : int32_t {
     PE_OP_SELL_SPMV = 1, PE_OP_SELL_GS, PE_OP_CSR_SPMV, PE_OP_PERM_IN, PE_OP_PERM_OUT, PE_OP_AXPBY, PE_OP_ADD3,
     PE_OP_FILL, PE_OP_COPY, PE_OP_SCALE, PE_OP_MUL, PE_OP_DOT, PE_OP_DOT_FIN, PE_OP_AXPY_DEV, PE_OP_XPBY_DEV,
-    PE_OP_PCG_STEP
+    PE_OP_PCG_STEP, PE_OP_PERM_IN_GS0
 };
 struct PeOp {               // 128 bytes, copied to shared memory by the interpreter
     int32_t type, i0, i1, i2, i3, i4, i5, flags;
@@ -155,7 +155,8 @@ struct DevSELL {
     int64_t nstored = 0;              // stored entries incl. padding
     int32_t *soff = nullptr;          // nslices+1 slice offsets, in units of 32 entries
     int32_t *J = nullptr;
-    double *A = nullptr;
+    double *A = nullptr;              // null when the values are sign-encoded
+    int8_t *S = nullptr;              // SpMV copies whose values are all -1, 0 or +1 (discrete derivatives): 1 B per entry
 };
 
 struct DevCSR {
@@ -185,6 +186,8 @@ int pe_launch_sell_gs(pe_ctx *ctx, const DevSELL &S, int s0, int s1, int wmax, i
 int pe_make_gather_policy(pe_ctx *ctx, int keep_pct, uint64_t *pol);
 int pe_launch_perm_in(pe_ctx *ctx, int n, const int *pos, const double *b, const double *x, double *fp, double *up);
 int pe_launch_perm_out(pe_ctx *ctx, int n, const int *pos, const double *up, double *x);
+int pe_launch_perm_in_gs0(pe_ctx *ctx, int n, const int *pos, const double *b, int r0, int r1, const double *l1,
+                          double *fp, double *up);
 #define PE_STREAM_NNZ 2048      // target non-zeros per CTA
 #define PE_STREAM_CAP 2560      // shared-memory capacity (target + longest admissible row)
 #define PE_STREAM_MAXROW 512

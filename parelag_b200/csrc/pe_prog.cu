@@ -50,12 +50,16 @@ __device__ __forceinline__ unsigned long long globaltimer_ns()
 // ---------------------------------------------------------------------------------------------
 // ops.  gw: global warp index (consecutive indices sit on different SMs), W: warps in the grid
 // ---------------------------------------------------------------------------------------------
-// p: soff J A x yin yout | i0 nslices i1 nrows | a alpha b beta
-__device__ __noinline__ void op_sell_spmv(const PeOp &o, int gw, int W, int lane)
+__device__ __forceinline__ double op_ld_value(const double *a, uint64_t pol) { return ld_stream_f64(a, pol); }
+__device__ __forceinline__ double op_ld_value(const int8_t *a, uint64_t pol) { return ld_stream_s8(a, pol); }
+
+// p: soff J A x yin yout S | i0 nslices i1 nrows | a alpha b beta      (S: sign codes in place of A, or null)
+template <typename V>
+__device__ __forceinline__ void sell_spmv_body(const PeOp &o, const V *A, int gw, int W, int lane)
 {
     const int nslices = o.i0, nrows = o.i1;
     const int *soff = (const int *)o.p[0], *J = (const int *)o.p[1];
-    const double *A = (const double *)o.p[2], *x = (const double *)o.p[3], *yin = (const double *)o.p[4];
+    const double *x = (const double *)o.p[3], *yin = (const double *)o.p[4];
     double *yout = (double *)o.p[5];
     const double alpha = o.a, beta = o.b;
     const uint64_t pol = l2_evict_first_policy();
@@ -63,19 +67,19 @@ __device__ __noinline__ void op_sell_spmv(const PeOp &o, int gw, int W, int lane
     {
         const int o0 = __ldg(soff + s), w = __ldg(soff + s + 1) - o0;
         const int *j = J + (int64_t)o0 * 32 + lane;
-        const double *a = A + (int64_t)o0 * 32 + lane;
+        const V *a = A + (int64_t)o0 * 32 + lane;
         double acc = 0.0;
         int q = 0;
         for (; q + 4 <= w; q += 4)
         {
             const int c0 = ld_stream_s32(j + (q + 0) * 32, pol), c1 = ld_stream_s32(j + (q + 1) * 32, pol);
             const int c2 = ld_stream_s32(j + (q + 2) * 32, pol), c3 = ld_stream_s32(j + (q + 3) * 32, pol);
-            const double a0 = ld_stream_f64(a + (q + 0) * 32, pol), a1 = ld_stream_f64(a + (q + 1) * 32, pol);
-            const double a2 = ld_stream_f64(a + (q + 2) * 32, pol), a3 = ld_stream_f64(a + (q + 3) * 32, pol);
+            const double a0 = op_ld_value(a + (q + 0) * 32, pol), a1 = op_ld_value(a + (q + 1) * 32, pol);
+            const double a2 = op_ld_value(a + (q + 2) * 32, pol), a3 = op_ld_value(a + (q + 3) * 32, pol);
             const double x0 = __ldcg(x + c0), x1 = __ldcg(x + c1), x2 = __ldcg(x + c2), x3 = __ldcg(x + c3);
             acc += a0 * x0; acc += a1 * x1; acc += a2 * x2; acc += a3 * x3;
         }
-        for (; q < w; ++q) acc += ld_stream_f64(a + q * 32, pol) * __ldcg(x + ld_stream_s32(j + q * 32, pol));
+        for (; q < w; ++q) acc += op_ld_value(a + q * 32, pol) * __ldcg(x + ld_stream_s32(j + q * 32, pol));
         const int row = s * 32 + lane;
         if (row < nrows)
         {
@@ -84,6 +88,11 @@ __device__ __noinline__ void op_sell_spmv(const PeOp &o, int gw, int W, int lane
             yout[row] = v;
         }
     }
+}
+__device__ __noinline__ void op_sell_spmv(const PeOp &o, int gw, int W, int lane)
+{
+    if (o.p[6]) sell_spmv_body(o, (const int8_t *)o.p[6], gw, W, lane);
+    else sell_spmv_body(o, (const double *)o.p[2], gw, W, lane);
 }
 
 // one colour of (l1-)Gauss-Seidel, slices [i0, i1) -- same arithmetic as k_sell_gs (pe_sell.cu)
@@ -189,6 +198,21 @@ __device__ __noinline__ void op_elementwise(const PeOp &o, int64_t gt, int64_t T
         const double *bv = (const double *)o.p[1], *x = (const double *)o.p[2];
         double *fp = (double *)o.p[3], *up = (double *)o.p[4];
         for (int64_t i = gt; i < n; i += T) { const int p = __ldg(pos + i); fp[p] = __ldcg(bv + i); up[p] = x ? __ldcg(x + i) : 0.0; }
+        break;
+    }
+    case PE_OP_PERM_IN_GS0:   // PERM_IN from a zero guess + the first colour, rows [r0, r1) (k_sell_perm_in_gs0)
+    {                         //                                                    p: pos b l1 fp up | i0 r0 i1 r1
+        const int *pos = (const int *)o.p[0];
+        const double *bv = (const double *)o.p[1], *l1 = (const double *)o.p[2];
+        double *fp = (double *)o.p[3], *up = (double *)o.p[4];
+        for (int64_t i = gt; i < n; i += T)
+        {
+            const int p = __ldg(pos + i);
+            const double d = (p >= o.i0 && p < o.i1) ? __ldcg(l1 + p) : 0.0;
+            const double fr = __ldcg(bv + i), ur = 0.0, acc = 0.0;
+            fp[p] = fr;
+            up[p] = d != 0.0 ? ur + (fr - acc) / d : ur;
+        }
         break;
     }
     case PE_OP_PERM_OUT:      // x[i] = up[pos[i]]                                  p: pos up x

@@ -1019,12 +1019,21 @@ extern "C" int pe_smoother_apply(pe_smoother *s, const pe_vec *b, pe_vec *x, int
             const bool zero_guess = !iterative_mode && sweep == 0;
             PE_TRY(sweep_halo(A, x->d, zero_guess));
             if (s->fused && !ctx->rec) { PE_TRY(launch_fused_sweep(s, b->d, x->d, zero_guess)); continue; }
-            PE_TRY(pe_launch_perm_in(ctx, n, s->pos_d, b->d, zero_guess ? nullptr : x->d, s->fp_d, s->up_d));
+            // from a zero guess the first colour only sees zeros: it is done by the renumbering pass
+            int first = -1;
+            if (zero_guess && s->nsets > 0)
+            {
+                first = 0;
+                while (first < s->nsets - 1 && s->slice_starts[first + 1] == s->slice_starts[first]) ++first;
+                PE_TRY(pe_launch_perm_in_gs0(ctx, n, s->pos_d, b->d, 32 * s->slice_starts[first], 32 * s->slice_starts[first + 1],
+                                             s->l1p_d, s->fp_d, s->up_d));
+            }
+            else PE_TRY(pe_launch_perm_in(ctx, n, s->pos_d, b->d, zero_guess ? nullptr : x->d, s->fp_d, s->up_d));
             for (int pass = 0; pass < 2; ++pass)
                 for (int cc = (pass == 1 && s->skip_turn) ? 1 : 0; cc < s->nsets; ++cc)
                 {
                     const int c = pass == 0 ? cc : s->nsets - 1 - cc;
-                    if (s->slice_starts[c + 1] == s->slice_starts[c]) continue;
+                    if (s->slice_starts[c + 1] == s->slice_starts[c] || (pass == 0 && c == first)) continue;
                     PE_TRY(pe_prof_begin(ctx, s->set_bytes[c] >= 64e6 ? 1 : 3, s->set_bytes[c]));
                     PE_TRY(pe_launch_sell_gs(ctx, s->S, s->slice_starts[c], s->slice_starts[c + 1], s->set_wmax[c], s->npad, s->fp_d, s->up_d,
                                              ghosts ? A->x_ext_d : nullptr, s->l1p_d, s->pol_gather));

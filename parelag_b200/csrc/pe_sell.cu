@@ -72,6 +72,7 @@ void pe_sell_free(DevSELL &m)
     if (m.soff) cudaFree(m.soff);
     if (m.J) cudaFree(m.J);
     if (m.A) cudaFree(m.A);
+    if (m.S) cudaFree(m.S);
     m = DevSELL();
 }
 
@@ -116,6 +117,38 @@ int pe_sell_build(pe_ctx *ctx, const DevCSR &diag, const DevCSR *offd, const int
     return 0;
 }
 
+// sign codes of the stored values; *bad is set when a value is not -1, 0 or +1 (-0.0 counts as 0: the row sum starts
+// at +0.0 and an fma only returns -0.0 from a -0.0 addend, so a +0 or -0 product leaves every sum bit-identical)
+__global__ void k_sell_signs(int64_t n, const double *__restrict__ A, int8_t *S, int *bad)
+{
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const double v = A[i];
+    const int8_t c = v == 1.0 ? 1 : (v == -1.0 ? -1 : 0);
+    if (c == 0 && v != 0.0) *bad = 1;
+    S[i] = c;
+}
+
+// Replace the values of a SELL copy by sign codes when all of them are -1, 0 or +1 (the discrete derivatives of the
+// fine de Rham sequence): 5 B per stored entry instead of 12, decoded to the same doubles.
+static int sell_encode_signs(pe_ctx *ctx, DevSELL &s)
+{
+    if (s.nstored == 0) return 0;
+    cudaStream_t st = ctx->stream;
+    int *bad_d = nullptr, bad = 0;
+    PE_CUDA(cudaMalloc(&s.S, (size_t)s.nstored));
+    PE_CUDA(cudaMalloc(&bad_d, sizeof(int)));
+    PE_CUDA(cudaMemsetAsync(bad_d, 0, sizeof(int), st));
+    k_sell_signs<<<pe_grid_for(s.nstored, 256), 256, 0, st>>>(s.nstored, s.A, s.S, bad_d);
+    PE_LAUNCHED(ctx);
+    PE_CUDA(cudaMemcpyAsync(&bad, bad_d, sizeof(int), cudaMemcpyDeviceToHost, st));
+    PE_CUDA(cudaStreamSynchronize(st));
+    cudaFree(bad_d);
+    if (bad) { cudaFree(s.S); s.S = nullptr; }
+    else { cudaFree(s.A); s.A = nullptr; }
+    return 0;
+}
+
 // Lazily attach a SELL copy to a CSR block used by SpMV.  Rejected (state -1) when padding
 // would add more than 25 % to the stream.
 int pe_sell_for_spmv(pe_ctx *ctx, DevCSR &m)
@@ -127,6 +160,8 @@ int pe_sell_for_spmv(pe_ctx *ctx, DevCSR &m)
     int rc = pe_sell_build(ctx, m, nullptr, nullptr, 0, nullptr, 0, *s);
     if (rc) { delete s; return rc; }
     if ((double)s->nstored > 1.25 * (double)m.nnz) { pe_sell_free(*s); delete s; return 0; }
+    rc = sell_encode_signs(ctx, *s);
+    if (rc) { pe_sell_free(*s); delete s; return rc; }
     m.sell = s;
     m.sell_state = 1;
     return 0;
@@ -141,8 +176,15 @@ int pe_sell_for_spmv(pe_ctx *ctx, DevCSR &m)
 // what short rows (RT0: 11, D: 2, D^T: 4) need to keep enough bytes in flight.  The products are
 // accumulated in entry order in every variant, so the result does not depend on G.
 // ---------------------------------------------------------------------------
-template <int G, bool PRO = false>
-__device__ __forceinline__ void sell_load_group(const int *j, const double *a, int q, int w, uint64_t pol,
+template <bool PRO>
+__device__ __forceinline__ double sell_load_value(const double *a, uint64_t pol)
+{ return PRO ? ld_stream_f64_pro(a, pol) : ld_stream_f64(a, pol); }
+template <bool PRO>
+__device__ __forceinline__ double sell_load_value(const int8_t *a, uint64_t pol)
+{ return PRO ? ld_stream_s8_pro(a, pol) : ld_stream_s8(a, pol); }
+
+template <int G, bool PRO = false, typename V>
+__device__ __forceinline__ void sell_load_group(const int *j, const V *a, int q, int w, uint64_t pol,
                                                 int (&c)[G], double (&v)[G])
 {
 #pragma unroll
@@ -150,7 +192,7 @@ __device__ __forceinline__ void sell_load_group(const int *j, const double *a, i
         if (q + k < w)
         {
             c[k] = PRO ? ld_stream_s32_pro(j + (q + k) * 32, pol) : ld_stream_s32(j + (q + k) * 32, pol);
-            v[k] = PRO ? ld_stream_f64_pro(a + (q + k) * 32, pol) : ld_stream_f64(a + (q + k) * 32, pol);
+            v[k] = sell_load_value<PRO>(a + (q + k) * 32, pol);
         }
 }
 
@@ -169,12 +211,12 @@ __device__ __forceinline__ void sell_pin_group_then_wait(const int (&c)[G], cons
 }
 
 // ---------------------------------------------------------------------------
-// SpMV: yout = alpha * A x + beta * yin   (thread per row, warp per slice)
+// SpMV: yout = alpha * A x + beta * yin   (thread per row, warp per slice; V: double values or int8 sign codes)
 // ---------------------------------------------------------------------------
-template <int G, bool SINGLE>
+template <int G, bool SINGLE, typename V>
 __global__ void __launch_bounds__(256, ((SINGLE || G <= 4) ? 4 : 2))
 k_sell_spmv(int nslices, int nrows, const int *__restrict__ soff, const int *__restrict__ J,
-            const double *__restrict__ A, const double *x, double alpha, double beta,
+            const V *__restrict__ A, const double *x, double alpha, double beta,
             const double *yin, double *yout)
 {
     // x, yin, f, u, uext are written by preceding kernels that may still be draining when this one
@@ -184,7 +226,7 @@ k_sell_spmv(int nslices, int nrows, const int *__restrict__ soff, const int *__r
     if (s >= nslices) { pdl_wait(); return; }
     const int o0 = ld_nc_s32_pro(soff + s), w = ld_nc_s32_pro(soff + s + 1) - o0;
     const int *j = J + (int64_t)o0 * 32 + lane;
-    const double *a = A + (int64_t)o0 * 32 + lane;
+    const V *a = A + (int64_t)o0 * 32 + lane;
     const uint64_t pol = l2_evict_first_policy();
     double acc = 0.0;
     int c[G]; double v[G];
@@ -266,18 +308,20 @@ int pe_launch_sell_spmv(pe_ctx *ctx, const DevSELL &S, double alpha, const doubl
     if (ctx->rec)
     {
         PeOp o = pe_op(PE_OP_SELL_SPMV); o.i0 = S.nslices; o.i1 = S.nrows; o.a = alpha; o.b = beta;
-        o.p[0] = S.soff; o.p[1] = S.J; o.p[2] = S.A; o.p[3] = x; o.p[4] = yin; o.p[5] = yout;
+        o.p[0] = S.soff; o.p[1] = S.J; o.p[2] = S.A; o.p[3] = x; o.p[4] = yin; o.p[5] = yout; o.p[6] = S.S;
         pe_rec_push(ctx, o, -1.0);
         return 0;
     }
     const int grid = pe_grid_for((int64_t)S.nslices * 32, 256);
     int G; bool single;
     sell_pick_group(S.wmax, G, single);
-#define PE_SPMV(GG, SS) PE_CUDA(pe_launch_k(ctx, k_sell_spmv<GG, SS>, grid, 256, S.nslices, S.nrows, S.soff, S.J, S.A, x, alpha, beta, yin, yout))
+#define PE_SPMV_V(GG, SS, VV, AA) PE_CUDA(pe_launch_k(ctx, k_sell_spmv<GG, SS, VV>, grid, 256, S.nslices, S.nrows, S.soff, S.J, AA, x, alpha, beta, yin, yout))
+#define PE_SPMV(GG, SS) do { if (S.S) PE_SPMV_V(GG, SS, int8_t, (const int8_t *)S.S); else PE_SPMV_V(GG, SS, double, (const double *)S.A); } while (0)
     if (G == 4) { if (single) PE_SPMV(4, true); else PE_SPMV(4, false); }
     else if (G == 8) { if (single) PE_SPMV(8, true); else PE_SPMV(8, false); }
     else { if (single) PE_SPMV(12, true); else PE_SPMV(12, false); }
 #undef PE_SPMV
+#undef PE_SPMV_V
     PE_LAUNCHED(ctx);
     return 0;
 }
@@ -378,6 +422,39 @@ int pe_launch_perm_in(pe_ctx *ctx, int n, const int *pos, const double *b, const
         return 0;
     }
     PE_CUDA(pe_launch_k(ctx, k_sell_perm_in, pe_grid_for(n, 256), 256, n, pos, b, x, fp, up));
+    PE_LAUNCHED(ctx);
+    return 0;
+}
+
+// Zero initial guess: perm_in of f, and the first colour of the sweep in the same pass.  u is +0 everywhere (ghosts
+// too), so every gather of that colour returns +0 and its row sum is +0 (fma(a, +0, +0) = +0 for finite a): the rows
+// [r0, r1) of that colour get k_sell_gs's update with acc = 0 -- the same expression, so the same bits, signed zeros
+// included -- and every other row gets the 0 perm_in writes.
+__global__ void k_sell_perm_in_gs0(int n, const int *__restrict__ pos, const double *b, int r0, int r1,
+                                   const double *__restrict__ l1, double *fp, double *up)
+{
+    pdl_trigger();
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    const int p = i < n ? pos[i] : 0;
+    const double d = (i < n && p >= r0 && p < r1) ? l1[p] : 0.0;
+    pdl_wait();
+    if (i >= n) return;
+    const double fr = b[i], ur = 0.0, acc = 0.0;
+    fp[p] = fr;
+    up[p] = d != 0.0 ? ur + (fr - acc) / d : ur;
+}
+int pe_launch_perm_in_gs0(pe_ctx *ctx, int n, const int *pos, const double *b, int r0, int r1, const double *l1,
+                          double *fp, double *up)
+{
+    if (n == 0) return 0;
+    if (ctx->rec)
+    {
+        PeOp o = pe_op(PE_OP_PERM_IN_GS0); o.n = n; o.i0 = r0; o.i1 = r1;
+        o.p[0] = pos; o.p[1] = b; o.p[2] = l1; o.p[3] = fp; o.p[4] = up;
+        pe_rec_push(ctx, o, 0.0);
+        return 0;
+    }
+    PE_CUDA(pe_launch_k(ctx, k_sell_perm_in_gs0, pe_grid_for(n, 256), 256, n, pos, b, r0, r1, l1, fp, up));
     PE_LAUNCHED(ctx);
     return 0;
 }

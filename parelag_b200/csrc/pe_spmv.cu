@@ -113,7 +113,9 @@ int pe_launch_spmv(pe_ctx *ctx, const DevCSR &diag, const DevCSR *offd, int tpr,
     if (!oI && diag.sell)
     {
         pe_variant_add(PE_VARIANT_SPMV_SELL, n);
-        PE_TRY(pe_prof_begin(ctx, 0, 12.0 * (double)diag.nnz + 4.0 * (n + 1) + 8.0 * diag.ncols + 8.0 * n + (beta != 0.0 ? 8.0 * n : 0.0)));
+        if (diag.sell->S) pe_variant_add(PE_VARIANT_SPMV_SELL_SIGNS, n);
+        const double per_nnz = diag.sell->S ? 5.0 : 12.0;     // sign-encoded values: 1 B instead of 8
+        PE_TRY(pe_prof_begin(ctx, 0, per_nnz * (double)diag.nnz + 4.0 * (n + 1) + 8.0 * diag.ncols + 8.0 * n + (beta != 0.0 ? 8.0 * n : 0.0)));
         PE_TRY(pe_launch_sell_spmv(ctx, *diag.sell, alpha, x, beta, yin, yout));
         PE_TRY(pe_prof_end(ctx));
         return 0;

@@ -39,6 +39,19 @@ __device__ __forceinline__ int ld_stream_s32_pro(const int *p, uint64_t pol)
     asm volatile("ld.global.nc.L1::no_allocate.L2::cache_hint.s32 %0, [%1], %2;" : "=r"(v) : "l"(p), "l"(pol));
     return v;
 }
+// sign-encoded SELL values (-1, 0, +1 stored as int8): decoded to the same double
+__device__ __forceinline__ double ld_stream_s8(const int8_t *p, uint64_t pol)
+{
+    int v;
+    asm("ld.global.nc.L1::no_allocate.L2::cache_hint.s8 %0, [%1], %2;" : "=r"(v) : "l"(p), "l"(pol));
+    return (double)v;
+}
+__device__ __forceinline__ double ld_stream_s8_pro(const int8_t *p, uint64_t pol)
+{
+    int v;
+    asm volatile("ld.global.nc.L1::no_allocate.L2::cache_hint.s8 %0, [%1], %2;" : "=r"(v) : "l"(p), "l"(pol));
+    return (double)v;
+}
 __device__ __forceinline__ int ld_nc_s32_pro(const int *p)
 {
     int v;

@@ -156,22 +156,30 @@ public:
         D_op_->MultTranspose(PrimaryVec_, AuxB_);
         PARELAG_ASSERT(!AuxiliarySolver_->iterative_mode);
         AuxiliarySolver_->Mult(AuxB_, AuxX_);
-        D_op_->Mult(AuxX_, PrimaryVec_);
-        X += PrimaryVec_;
+        AddAuxiliaryCorrection(X);
     }
     void MultTranspose(const mfem::Vector &B, mfem::Vector &X) const override
     {
         if (this->IsPreconditioner()) { X = 0.0; D_op_->MultTranspose(B, AuxB_); }
         else { mg_utils::ComputeResidual(*A_, X, B, PrimaryVec_); D_op_->MultTranspose(PrimaryVec_, AuxB_); }
         AuxiliarySolver_->Mult(AuxB_, AuxX_);
-        D_op_->Mult(AuxX_, PrimaryVec_);
-        X += PrimaryVec_;
+        AddAuxiliaryCorrection(X);
         PrimarySolver_->Mult(B, X);
     }
     Op_Ptr GetAuxiliaryOperator() const { return A_aux_; }
     bool CaptureSafe() const override
     { return SolverCaptureSafe(PrimarySolver_.get()) && SolverCaptureSafe(AuxiliarySolver_.get()); }
 private:
+    /// X += D AuxX_.  On one rank the add rides in the product (beta = 1): acc + X rounds like X + (D AuxX_), so the
+    /// bits are those of the separate pass.  With a halo, D's diagonal and off-diagonal blocks are two passes, and
+    /// adding X before the second would change the order of the sum, so the separate add stays.
+    void AddAuxiliaryCorrection(mfem::Vector &X) const
+    {
+        auto D_hyp = dynamic_cast<const mfem::HypreParMatrix *>(D_op_.get());
+        if (D_hyp && pe_ctx_nranks(Device::Get()) == 1) { D_hyp->Mult(1.0, AuxX_, 1.0, X); return; }
+        D_op_->Mult(AuxX_, PrimaryVec_);
+        X += PrimaryVec_;
+    }
     void _do_set_operator(const Op_Ptr &) override { PARELAG_NOT_IMPLEMENTED(); }
     Op_Ptr A_, A_aux_, D_op_;
     std::shared_ptr<mfem::Solver> PrimarySolver_, AuxiliarySolver_;

@@ -128,7 +128,12 @@ int pe_get_tuning(int key);
  * shared-memory extension launch of a batch split between both kernels (also counted in EXT_SMEM); TRACES_GMEM_REUSE and
  * EXT_GMEM_REUSE count the agglomerates a global-workspace CTA takes after its first one (a launch with more agglomerates
  * than CTAs reuses each workspace slab).  SPMV_SELL_SIGNS counts the rows of SELL SpMVs whose values are stored as int8
- * sign codes (every value -1, 0 or +1; also counted in SPMV_SELL).  out: n slots (slots past PE_VARIANT_COUNT are set to 0; NULL with n = 0 copies nothing);
+ * sign codes (every value -1, 0 or +1; also counted in SPMV_SELL).  SELL_GS_* and SELL_SPMV_* count the entry-group variant
+ * of each k_sell_gs (one colour of a multicolour sweep) and k_sell_spmv launch: G = 4, 8 or 12 entries per group, SINGLE
+ * when every slice of the launch fits one group, PIPE otherwise; the unit is padded slice rows (32 per slice of the
+ * launch, padding rows of a partly filled slice included).  Recording a persistent program pushes an op and picks no
+ * variant, so it counts nothing; capturing a CUDA graph counts once, at capture, and a replay counts nothing.
+ * out: n slots (slots past PE_VARIANT_COUNT are set to 0; NULL with n = 0 copies nothing);
  * reset != 0 zeroes every counter after the copy. */
 enum { PE_VARIANT_SPMV_SELL = 0, PE_VARIANT_SPMV_STREAM = 1, PE_VARIANT_SPMV_VECTOR = 2,
        PE_VARIANT_SPGEMM_SYM_T128 = 3, PE_VARIANT_SPGEMM_SYM_T1024 = 4, PE_VARIANT_SPGEMM_SYM_T8192 = 5, PE_VARIANT_SPGEMM_SYM_GMEM = 6,
@@ -137,7 +142,12 @@ enum { PE_VARIANT_SPMV_SELL = 0, PE_VARIANT_SPMV_STREAM = 1, PE_VARIANT_SPMV_VEC
        PE_VARIANT_RELAX_TPR_16 = 15, PE_VARIANT_RELAX_TPR_32 = 16,
        PE_VARIANT_TRACES_SMEM = 17, PE_VARIANT_TRACES_GMEM = 18, PE_VARIANT_EXT_SMEM = 19, PE_VARIANT_EXT_GMEM = 20,
        PE_VARIANT_EXT_SPLIT_SMEM = 21, PE_VARIANT_TRACES_GMEM_REUSE = 22, PE_VARIANT_EXT_GMEM_REUSE = 23,
-       PE_VARIANT_SPMV_SELL_SIGNS = 24, PE_VARIANT_COUNT = 25 };
+       PE_VARIANT_SPMV_SELL_SIGNS = 24,
+       PE_VARIANT_SELL_GS_G4_SINGLE = 25, PE_VARIANT_SELL_GS_G4_PIPE = 26, PE_VARIANT_SELL_GS_G8_SINGLE = 27,
+       PE_VARIANT_SELL_GS_G8_PIPE = 28, PE_VARIANT_SELL_GS_G12_SINGLE = 29, PE_VARIANT_SELL_GS_G12_PIPE = 30,
+       PE_VARIANT_SELL_SPMV_G4_SINGLE = 31, PE_VARIANT_SELL_SPMV_G4_PIPE = 32, PE_VARIANT_SELL_SPMV_G8_SINGLE = 33,
+       PE_VARIANT_SELL_SPMV_G8_PIPE = 34, PE_VARIANT_SELL_SPMV_G12_SINGLE = 35, PE_VARIANT_SELL_SPMV_G12_PIPE = 36,
+       PE_VARIANT_COUNT = 37 };
 int pe_variant_counts(int64_t *out, int n, int reset);
 /* write a scratch buffer larger than L2 (bench hygiene) */
 int pe_ctx_flush_l2(pe_ctx *ctx);

@@ -159,13 +159,26 @@ VARIANT_SLOTS = ("SPMV_SELL", "SPMV_STREAM", "SPMV_VECTOR",
                  "SPGEMM_NUM_T128", "SPGEMM_NUM_T1024", "SPGEMM_NUM_T8192", "SPGEMM_NUM_GMEM",
                  "RELAX_TPR_1", "RELAX_TPR_2", "RELAX_TPR_4", "RELAX_TPR_8", "RELAX_TPR_16", "RELAX_TPR_32",
                  "TRACES_SMEM", "TRACES_GMEM", "EXT_SMEM", "EXT_GMEM",
-                 "EXT_SPLIT_SMEM", "TRACES_GMEM_REUSE", "EXT_GMEM_REUSE", "SPMV_SELL_SIGNS")
+                 "EXT_SPLIT_SMEM", "TRACES_GMEM_REUSE", "EXT_GMEM_REUSE", "SPMV_SELL_SIGNS",
+                 "SELL_GS_G4_SINGLE", "SELL_GS_G4_PIPE", "SELL_GS_G8_SINGLE", "SELL_GS_G8_PIPE",
+                 "SELL_GS_G12_SINGLE", "SELL_GS_G12_PIPE",
+                 "SELL_SPMV_G4_SINGLE", "SELL_SPMV_G4_PIPE", "SELL_SPMV_G8_SINGLE", "SELL_SPMV_G8_PIPE",
+                 "SELL_SPMV_G12_SINGLE", "SELL_SPMV_G12_PIPE")
 (SPMV_SELL, SPMV_STREAM, SPMV_VECTOR,
  SPGEMM_SYM_T128, SPGEMM_SYM_T1024, SPGEMM_SYM_T8192, SPGEMM_SYM_GMEM,
  SPGEMM_NUM_T128, SPGEMM_NUM_T1024, SPGEMM_NUM_T8192, SPGEMM_NUM_GMEM,
  RELAX_TPR_1, RELAX_TPR_2, RELAX_TPR_4, RELAX_TPR_8, RELAX_TPR_16, RELAX_TPR_32,
  TRACES_SMEM, TRACES_GMEM, EXT_SMEM, EXT_GMEM,
- EXT_SPLIT_SMEM, TRACES_GMEM_REUSE, EXT_GMEM_REUSE, SPMV_SELL_SIGNS) = range(len(VARIANT_SLOTS))
+ EXT_SPLIT_SMEM, TRACES_GMEM_REUSE, EXT_GMEM_REUSE, SPMV_SELL_SIGNS,
+ SELL_GS_G4_SINGLE, SELL_GS_G4_PIPE, SELL_GS_G8_SINGLE, SELL_GS_G8_PIPE, SELL_GS_G12_SINGLE, SELL_GS_G12_PIPE,
+ SELL_SPMV_G4_SINGLE, SELL_SPMV_G4_PIPE, SELL_SPMV_G8_SINGLE, SELL_SPMV_G8_PIPE, SELL_SPMV_G12_SINGLE,
+ SELL_SPMV_G12_PIPE) = range(len(VARIANT_SLOTS))
+
+
+def sell_group_slot(kernel, G, single):
+    """slot of the (G, single) entry-group variant of k_sell_gs (kernel "gs") or k_sell_spmv ("spmv")"""
+    base = SELL_GS_G4_SINGLE if kernel == "gs" else SELL_SPMV_G4_SINGLE
+    return base + 2 * (G // 4 - 1) + (0 if single else 1)
 
 
 def variant_counts(reset=False):

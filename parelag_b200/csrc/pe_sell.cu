@@ -301,6 +301,12 @@ static void sell_pick_group(int wmax, int &G, bool &single)
     single = wmax <= G;
 }
 
+// pe_variant_counts slot of a (G, single) choice: base = PE_VARIANT_SELL_GS_G4_SINGLE or PE_VARIANT_SELL_SPMV_G4_SINGLE
+static int sell_group_slot(int base, int G, bool single)
+{
+    return base + 2 * (G / 4 - 1) + (single ? 0 : 1);
+}
+
 int pe_launch_sell_spmv(pe_ctx *ctx, const DevSELL &S, double alpha, const double *x, double beta,
                         const double *yin, double *yout)
 {
@@ -315,6 +321,7 @@ int pe_launch_sell_spmv(pe_ctx *ctx, const DevSELL &S, double alpha, const doubl
     const int grid = pe_grid_for((int64_t)S.nslices * 32, 256);
     int G; bool single;
     sell_pick_group(S.wmax, G, single);
+    pe_variant_add(sell_group_slot(PE_VARIANT_SELL_SPMV_G4_SINGLE, G, single), (int64_t)S.nslices * 32);
 #define PE_SPMV_V(GG, SS, VV, AA) PE_CUDA(pe_launch_k(ctx, k_sell_spmv<GG, SS, VV>, grid, 256, S.nslices, S.nrows, S.soff, S.J, AA, x, alpha, beta, yin, yout))
 #define PE_SPMV(GG, SS) do { if (S.S) PE_SPMV_V(GG, SS, int8_t, (const int8_t *)S.S); else PE_SPMV_V(GG, SS, double, (const double *)S.A); } while (0)
     if (G == 4) { if (single) PE_SPMV(4, true); else PE_SPMV(4, false); }
@@ -381,6 +388,7 @@ int pe_launch_sell_gs(pe_ctx *ctx, const DevSELL &S, int s0, int s1, int wmax, i
     const int grid = pe_grid_for((int64_t)(s1 - s0) * 32, 256);
     int G; bool single;
     sell_pick_group(wmax > 0 ? wmax : S.wmax, G, single);
+    pe_variant_add(sell_group_slot(PE_VARIANT_SELL_GS_G4_SINGLE, G, single), (int64_t)(s1 - s0) * 32);
 #define PE_GS(GG, SS, OO) PE_CUDA(pe_launch_k(ctx, k_sell_gs<GG, SS, OO>, grid, 256, s0, s1, S.soff, S.J, S.A, ext_base, f, u, uext, l1, pol_gather))
 #define PE_GS2(GG, SS) do { if (uext) PE_GS(GG, SS, true); else PE_GS(GG, SS, false); } while (0)
     if (G == 4) { if (single) PE_GS2(4, true); else PE_GS2(4, false); }

@@ -41,6 +41,12 @@ def test_variant_counter_slots_match_the_header():
     assert slots.pop("COUNT") == len(capi.VARIANT_SLOTS)
     assert slots == {name: getattr(capi, name) for name in capi.VARIANT_SLOTS}
     assert [slots[n] for n in capi.VARIANT_SLOTS] == list(range(len(capi.VARIANT_SLOTS)))
+    # the SELL entry-group slots: one per (kernel, G, single) choice, in the order sell_group_slot (pe_sell.cu) indexes
+    for kernel in ("gs", "spmv"):
+        for G in (4, 8, 12):
+            for single in (True, False):
+                name = "SELL_%s_G%d_%s" % (kernel.upper(), G, "SINGLE" if single else "PIPE")
+                assert capi.sell_group_slot(kernel, G, single) == slots[name], name
     capi.variant_counts(reset=True)
     assert not capi.variant_counts().any()
     tune = _header_enum("PE_TUNE_SELL_MIN_ROWS", "int pe_set_tuning")

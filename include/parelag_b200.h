@@ -252,6 +252,14 @@ int pe_mat_abs_row_sums(const pe_mat *A, pe_vec *d);
 int pe_spmv(pe_ctx *ctx, double alpha, pe_mat *A, const pe_vec *x, double beta, pe_vec *y);
 int pe_spmv_t(pe_ctx *ctx, double alpha, pe_mat *A, const pe_vec *x, double beta, pe_vec *y);
 int pe_residual(pe_ctx *ctx, pe_mat *A, const pe_vec *x, const pe_vec *b, pe_vec *r);
+/* Renumbered copy of A (transpose != 0: of A^T) for products on vectors in other numberings, single rank: row i of A
+ * becomes row rpos[i] of a matrix of nrows_out rows, column j becomes column cpos[j] of ncols_out; NULL keeps the
+ * natural numbering of that side.  rpos / cpos are device arrays, e.g. the colour numbering of
+ * pe_smoother_colour_numbering.  Each row keeps its entries, their order, and A's SpMV format, so every mapped entry
+ * of a product equals the natural product's bit for bit; rows no row of A maps to are empty (their result is
+ * beta * y).  Free with pe_mat_free. */
+int pe_mat_renumbered(pe_ctx *ctx, pe_mat *A, int transpose, const int32_t *rpos, int32_t nrows_out,
+                      const int32_t *cpos, int32_t ncols_out, pe_mat **out);
 
 /* ---- K3/K4/K5: hypre relaxation (mfem::HypreSmoother behind
  * parelag::HypreSmootherWrapper, src/linalg/solver_ops/ParELAG_HypreSmootherWrapper.cpp:20-35;
@@ -272,6 +280,18 @@ int pe_smoother_get_l1(const pe_smoother *s, double *l1_host);
 int pe_smoother_get_order(const pe_smoother *s, int32_t *order_host, int32_t *num_sets,
                           int32_t *set_starts_host /* num_sets+1, may be NULL */);
 int pe_smoother_get_eig(const pe_smoother *s, double *max_eig, double *min_eig);
+/* Colour numbering of a multicolour SELL Gauss-Seidel smoother (one rank): *npad = padded length of the colour-ordered
+ * vectors, *pos_d = device array row -> position (owned by the smoother).  *npad = 0 and *pos_d = NULL when the
+ * smoother has no such numbering (other types, CSR path, fused sweeps). */
+int pe_smoother_colour_numbering(const pe_smoother *s, int32_t *npad, const int32_t **pos_d);
+/* The smoother on colour-numbered vectors f, u of npad entries, no renumbering passes.  Padding entries of f must be 0;
+ * those of u stay 0.  mode 0: u holds the initial guess; 1: zero initial guess (u's content is ignored); 2: u is what
+ * pe_smoother_colour_in left (the first colour of a sweep from a zero guess is done). */
+int pe_smoother_apply_colour(pe_smoother *s, const pe_vec *f, pe_vec *u, int mode);
+/* b (natural) -> f (colour order) and u = the first colour of a sweep from a zero guess, in one pass; then
+ * pe_smoother_apply_colour(mode 2).  pe_smoother_colour_out: x (natural) = u (colour order). */
+int pe_smoother_colour_in(pe_smoother *s, const pe_vec *b, pe_vec *f, pe_vec *u);
+int pe_smoother_colour_out(pe_smoother *s, const pe_vec *u, pe_vec *x);
 
 /* ---- K8/K9: sparse products
  * C = A*B (mfem::ParMult / hypre_ParMatmul; SchurComplementFactory.cpp:51-166)

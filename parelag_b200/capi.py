@@ -324,6 +324,13 @@ class Mat:
     def residual(self, x, b, r):
         _chk(lib().pe_residual(self.ctx.h, self.h, x.h, b.h, r.h))
 
+    def renumbered(self, transpose=False, rpos=None, nrows_out=0, cpos=None, ncols_out=0):
+        """pe_mat_renumbered: rpos / cpos are device pointers (Smoother.colour_numbering) or None"""
+        out = Mat(self.ctx)
+        _chk(lib().pe_mat_renumbered(self.ctx.h, self.h, 1 if transpose else 0, C.c_void_p(rpos), C.c_int32(nrows_out),
+                                     C.c_void_p(cpos), C.c_int32(ncols_out), C.byref(out.h)))
+        return out
+
     def fix_zero_rows(self):
         n = C.c_int32()
         _chk(lib().pe_fix_zero_rows(self.ctx.h, self.h, C.byref(n)))
@@ -398,6 +405,21 @@ class Smoother:
 
     def apply(self, b, x, iterative_mode=True):
         _chk(lib().pe_smoother_apply(self.h, b.h, x.h, 1 if iterative_mode else 0))
+
+    def colour_numbering(self):
+        """(npad, device pointer of row -> colour position); (0, None) without a colour numbering"""
+        npad, pos = C.c_int32(), C.c_void_p()
+        _chk(lib().pe_smoother_colour_numbering(self.h, C.byref(npad), C.byref(pos)))
+        return npad.value, pos.value
+
+    def apply_colour(self, f, u, mode):
+        _chk(lib().pe_smoother_apply_colour(self.h, f.h, u.h, mode))
+
+    def colour_in(self, b, f, u):
+        _chk(lib().pe_smoother_colour_in(self.h, b.h, f.h, u.h))
+
+    def colour_out(self, u, x):
+        _chk(lib().pe_smoother_colour_out(self.h, u.h, x.h))
 
     def l1(self):
         n = self.A.info()[0]

@@ -176,7 +176,7 @@ void pe_sell_free(DevSELL &m);
 int pe_sell_build(pe_ctx *ctx, const DevCSR &diag, const DevCSR *offd, const int32_t *rowmap_d, int32_t nslices,
                   const int32_t *colpos_d, int32_t ext_base, DevSELL &out,
                   std::vector<int32_t> *soff_host = nullptr);
-int pe_sell_for_spmv(pe_ctx *ctx, DevCSR &m);
+int pe_sell_for_spmv(pe_ctx *ctx, DevCSR &m, bool force = false);
 void pe_mat_values_changed(struct pe_mat *A);   // drop cached transposes / SELL copies after an in-place edit
 int pe_launch_sell_spmv(pe_ctx *ctx, const DevSELL &S, double alpha, const double *x, double beta,
                         const double *yin, double *yout);

@@ -200,17 +200,17 @@ __device__ __noinline__ void op_elementwise(const PeOp &o, int64_t gt, int64_t T
         for (int64_t i = gt; i < n; i += T) { const int p = __ldg(pos + i); fp[p] = __ldcg(bv + i); up[p] = x ? __ldcg(x + i) : 0.0; }
         break;
     }
-    case PE_OP_PERM_IN_GS0:   // PERM_IN from a zero guess + the first colour, rows [r0, r1) (k_sell_perm_in_gs0)
-    {                         //                                                    p: pos b l1 fp up | i0 r0 i1 r1
+    case PE_OP_PERM_IN_GS0:   // PERM_IN from a zero guess + the first colour, rows [r0, r1) (k_sell_perm_in_gs0;
+    {                         // pos null: b already in colour order, only up written)  p: pos b l1 fp up | i0 r0 i1 r1
         const int *pos = (const int *)o.p[0];
         const double *bv = (const double *)o.p[1], *l1 = (const double *)o.p[2];
         double *fp = (double *)o.p[3], *up = (double *)o.p[4];
         for (int64_t i = gt; i < n; i += T)
         {
-            const int p = __ldg(pos + i);
+            const int p = pos ? __ldg(pos + i) : (int)i;
             const double d = (p >= o.i0 && p < o.i1) ? __ldcg(l1 + p) : 0.0;
-            const double fr = __ldcg(bv + i), ur = 0.0, acc = 0.0;
-            fp[p] = fr;
+            const double fr = (fp || d != 0.0) ? __ldcg(bv + i) : 0.0, ur = 0.0, acc = 0.0;
+            if (fp) fp[p] = fr;
             up[p] = d != 0.0 ? ur + (fr - acc) / d : ur;
         }
         break;

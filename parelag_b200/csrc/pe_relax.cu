@@ -1003,6 +1003,86 @@ static int sweep_halo(pe_mat *A, const double *x_d, bool all_zero)
     return pe_halo_wait(A);
 }
 
+// first colour with rows (the one a sweep from a zero guess does without gathers)
+static int first_colour(const pe_smoother *s)
+{
+    int first = 0;
+    while (first < s->nsets - 1 && s->slice_starts[first + 1] == s->slice_starts[first]) ++first;
+    return first;
+}
+
+// one symmetric sweep of the colour-ordered SELL path on f, u in colour order; skip_first: the first forward colour is
+// done (zero-guess start)
+static int sell_sweep(pe_smoother *s, const double *f, double *u, bool skip_first)
+{
+    pe_ctx *ctx = s->ctx;
+    pe_mat *A = s->A;
+    const int first = skip_first ? first_colour(s) : -1;
+    for (int pass = 0; pass < 2; ++pass)
+        for (int cc = (pass == 1 && s->skip_turn) ? 1 : 0; cc < s->nsets; ++cc)
+        {
+            const int c = pass == 0 ? cc : s->nsets - 1 - cc;
+            if (s->slice_starts[c + 1] == s->slice_starts[c] || (pass == 0 && c == first)) continue;
+            PE_TRY(pe_prof_begin(ctx, s->set_bytes[c] >= 64e6 ? 1 : 3, s->set_bytes[c]));
+            PE_TRY(pe_launch_sell_gs(ctx, s->S, s->slice_starts[c], s->slice_starts[c + 1], s->set_wmax[c], s->npad, f, u,
+                                     A->offd.nnz > 0 ? A->x_ext_d : nullptr, s->l1p_d, s->pol_gather));
+            PE_TRY(pe_prof_end(ctx));
+        }
+    return 0;
+}
+
+static bool has_colour_numbering(const pe_smoother *s)
+{
+    return s->use_sell && !s->fused && s->nsets > 0 && s->ctx->nranks == 1 && s->A->offd.nnz == 0;
+}
+
+extern "C" int pe_smoother_colour_numbering(const pe_smoother *s, int32_t *npad, const int32_t **pos_d)
+{
+    PE_CHECK(s && npad && pos_d, "bad arguments");
+    const bool on = has_colour_numbering(s);
+    *npad = on ? s->npad : 0;
+    *pos_d = on ? s->pos_d : nullptr;
+    return 0;
+}
+
+extern "C" int pe_smoother_apply_colour(pe_smoother *s, const pe_vec *f, pe_vec *u, int mode)
+{
+    PE_CHECK(s && f && u && mode >= 0 && mode <= 2, "bad arguments");
+    PE_CHECK(has_colour_numbering(s), "pe_smoother_apply_colour: the smoother has no colour numbering");
+    PE_CHECK(f->n == s->npad && u->n == s->npad, "pe_smoother_apply_colour: size mismatch");
+    for (int sweep = 0; sweep < s->sweeps; ++sweep)
+    {
+        if (sweep == 0 && mode == 1)
+        {
+            const int first = first_colour(s);
+            PE_TRY(pe_launch_perm_in_gs0(s->ctx, s->npad, nullptr, f->d, 32 * s->slice_starts[first], 32 * s->slice_starts[first + 1],
+                                         s->l1p_d, nullptr, u->d));
+        }
+        PE_TRY(sell_sweep(s, f->d, u->d, sweep == 0 && mode != 0));
+    }
+    return 0;
+}
+
+extern "C" int pe_smoother_colour_in(pe_smoother *s, const pe_vec *b, pe_vec *f, pe_vec *u)
+{
+    PE_CHECK(s && b && f && u, "bad arguments");
+    PE_CHECK(has_colour_numbering(s), "pe_smoother_colour_in: the smoother has no colour numbering");
+    const int n = s->A->diag.nrows;
+    PE_CHECK(b->n == n && f->n == s->npad && u->n == s->npad, "pe_smoother_colour_in: size mismatch");
+    const int first = first_colour(s);
+    return pe_launch_perm_in_gs0(s->ctx, n, s->pos_d, b->d, 32 * s->slice_starts[first], 32 * s->slice_starts[first + 1],
+                                 s->l1p_d, f->d, u->d);
+}
+
+extern "C" int pe_smoother_colour_out(pe_smoother *s, const pe_vec *u, pe_vec *x)
+{
+    PE_CHECK(s && u && x, "bad arguments");
+    PE_CHECK(has_colour_numbering(s), "pe_smoother_colour_out: the smoother has no colour numbering");
+    const int n = s->A->diag.nrows;
+    PE_CHECK(x->n == n && u->n == s->npad, "pe_smoother_colour_out: size mismatch");
+    return pe_launch_perm_out(s->ctx, n, s->pos_d, u->d, x->d);
+}
+
 extern "C" int pe_smoother_apply(pe_smoother *s, const pe_vec *b, pe_vec *x, int iterative_mode)
 {
     pe_ctx *ctx = s->ctx;
@@ -1013,32 +1093,21 @@ extern "C" int pe_smoother_apply(pe_smoother *s, const pe_vec *b, pe_vec *x, int
     if (s->use_sell)
     {
         // colour-ordered SELL path: f and u are carried in colour order across the whole sweep
-        const bool ghosts = A->offd.nnz > 0;
         for (int sweep = 0; sweep < s->sweeps; ++sweep)
         {
             const bool zero_guess = !iterative_mode && sweep == 0;
             PE_TRY(sweep_halo(A, x->d, zero_guess));
             if (s->fused && !ctx->rec) { PE_TRY(launch_fused_sweep(s, b->d, x->d, zero_guess)); continue; }
             // from a zero guess the first colour only sees zeros: it is done by the renumbering pass
-            int first = -1;
-            if (zero_guess && s->nsets > 0)
+            const bool fold = zero_guess && s->nsets > 0;
+            if (fold)
             {
-                first = 0;
-                while (first < s->nsets - 1 && s->slice_starts[first + 1] == s->slice_starts[first]) ++first;
+                const int first = first_colour(s);
                 PE_TRY(pe_launch_perm_in_gs0(ctx, n, s->pos_d, b->d, 32 * s->slice_starts[first], 32 * s->slice_starts[first + 1],
                                              s->l1p_d, s->fp_d, s->up_d));
             }
             else PE_TRY(pe_launch_perm_in(ctx, n, s->pos_d, b->d, zero_guess ? nullptr : x->d, s->fp_d, s->up_d));
-            for (int pass = 0; pass < 2; ++pass)
-                for (int cc = (pass == 1 && s->skip_turn) ? 1 : 0; cc < s->nsets; ++cc)
-                {
-                    const int c = pass == 0 ? cc : s->nsets - 1 - cc;
-                    if (s->slice_starts[c + 1] == s->slice_starts[c] || (pass == 0 && c == first)) continue;
-                    PE_TRY(pe_prof_begin(ctx, s->set_bytes[c] >= 64e6 ? 1 : 3, s->set_bytes[c]));
-                    PE_TRY(pe_launch_sell_gs(ctx, s->S, s->slice_starts[c], s->slice_starts[c + 1], s->set_wmax[c], s->npad, s->fp_d, s->up_d,
-                                             ghosts ? A->x_ext_d : nullptr, s->l1p_d, s->pol_gather));
-                    PE_TRY(pe_prof_end(ctx));
-                }
+            PE_TRY(sell_sweep(s, s->fp_d, s->up_d, fold));
             PE_TRY(pe_launch_perm_out(ctx, n, s->pos_d, s->up_d, x->d));
         }
         return 0;

@@ -151,7 +151,8 @@ static int sell_encode_signs(pe_ctx *ctx, DevSELL &s)
 
 // Lazily attach a SELL copy to a CSR block used by SpMV.  Rejected (state -1) when padding
 // would add more than 25 % to the stream.
-int pe_sell_for_spmv(pe_ctx *ctx, DevCSR &m)
+// force: keep the copy whatever its padding (a renumbered copy takes the format of its source: pe_mat_renumbered).
+int pe_sell_for_spmv(pe_ctx *ctx, DevCSR &m, bool force)
 {
     if (m.sell_state != 0) return 0;
     m.sell_state = -1;
@@ -159,7 +160,7 @@ int pe_sell_for_spmv(pe_ctx *ctx, DevCSR &m)
     DevSELL *s = new DevSELL();
     int rc = pe_sell_build(ctx, m, nullptr, nullptr, 0, nullptr, 0, *s);
     if (rc) { delete s; return rc; }
-    if ((double)s->nstored > 1.25 * (double)m.nnz) { pe_sell_free(*s); delete s; return 0; }
+    if (!force && (double)s->nstored > 1.25 * (double)m.nnz) { pe_sell_free(*s); delete s; return 0; }
     rc = sell_encode_signs(ctx, *s);
     if (rc) { pe_sell_free(*s); delete s; return rc; }
     m.sell = s;
@@ -438,17 +439,19 @@ int pe_launch_perm_in(pe_ctx *ctx, int n, const int *pos, const double *b, const
 // too), so every gather of that colour returns +0 and its row sum is +0 (fma(a, +0, +0) = +0 for finite a): the rows
 // [r0, r1) of that colour get k_sell_gs's update with acc = 0 -- the same expression, so the same bits, signed zeros
 // included -- and every other row gets the 0 perm_in writes.
+// pos == null: b is already in colour order (n = the padded length) and only u is written -- the zero-guess start of a
+// smoother application on a colour-numbered level.
 __global__ void k_sell_perm_in_gs0(int n, const int *__restrict__ pos, const double *b, int r0, int r1,
                                    const double *__restrict__ l1, double *fp, double *up)
 {
     pdl_trigger();
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    const int p = i < n ? pos[i] : 0;
+    const int p = pos ? (i < n ? pos[i] : 0) : i;
     const double d = (i < n && p >= r0 && p < r1) ? l1[p] : 0.0;
     pdl_wait();
     if (i >= n) return;
-    const double fr = b[i], ur = 0.0, acc = 0.0;
-    fp[p] = fr;
+    const double fr = (fp || d != 0.0) ? b[i] : 0.0, ur = 0.0, acc = 0.0;
+    if (fp) fp[p] = fr;
     up[p] = d != 0.0 ? ur + (fr - acc) / d : ur;
 }
 int pe_launch_perm_in_gs0(pe_ctx *ctx, int n, const int *pos, const double *b, int r0, int r1, const double *l1,

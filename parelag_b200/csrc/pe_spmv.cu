@@ -124,7 +124,7 @@ int pe_launch_spmv(pe_ctx *ctx, const DevCSR &diag, const DevCSR *offd, int tpr,
     {
         // persistent program: CSR-vector op (the CTA-tiled streaming kernel has no op equivalent)
         pe_variant_add(PE_VARIANT_SPMV_VECTOR, n);
-        PeOp o = pe_op(PE_OP_CSR_SPMV); o.i0 = n; o.i1 = pe_choose_tpr(diag.nnz, n); o.a = alpha; o.b = beta;
+        PeOp o = pe_op(PE_OP_CSR_SPMV); o.i0 = n; o.i1 = tpr; o.a = alpha; o.b = beta;
         o.p[0] = diag.I; o.p[1] = diag.J; o.p[2] = diag.A; o.p[3] = x; o.p[4] = yin; o.p[5] = yout;
         pe_rec_push(ctx, o, 12.0 * (double)diag.nnz + 4.0 * (n + 1) + 8.0 * diag.ncols + 8.0 * n + (beta != 0.0 ? 8.0 * n : 0.0));
         return 0;
@@ -265,6 +265,69 @@ extern "C" int pe_spmv_t(pe_ctx *ctx, double alpha, pe_mat *A, const pe_vec *x, 
     if (A->distributed) return pe_spmv_t_distributed(ctx, alpha, A, x, beta, y);
     if (!A->T) PE_TRY(pe_mat_transpose(ctx, A, &A->T));
     return pe_spmv(ctx, alpha, A->T, x, beta, y);
+}
+
+// ---------------------------------------------------------------------------
+// Renumbered copies: row i of the source becomes row rpos[i] of a matrix of nrows_out rows (rows no source row maps to
+// stay empty), column j becomes column cpos[j]; the entries of a row and their order are kept.  On vectors in the colour
+// numbering of a multicolour SELL level the product is then the natural one, permuted, bit for bit: every row runs the
+// same sum in the same order, with the same kernel -- the copy takes its source's format (SELL or CSR, as decided on the
+// source) and lane count, since a SELL row sums with fma and a CSR row with separate products.  Rows in colour order
+// write and read y contiguously; measured against natural rows with a scattered row map (B200, configs[1] 144^3), the
+// V-cycle's SpMV time was 94 ms instead of 106 ms per 50 cycles.
+// ---------------------------------------------------------------------------
+__global__ void k_renumber_row_lens(int n, const int *__restrict__ I, const int *__restrict__ rpos, int *len)
+{
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) len[(rpos ? rpos[i] : i) + 1] = I[i + 1] - I[i];
+}
+__global__ void k_renumber_fill(int n, const int *__restrict__ I, const int *__restrict__ J, const double *__restrict__ A,
+                                const int *__restrict__ rpos, const int *__restrict__ cpos, const int *__restrict__ RI,
+                                int *RJ, double *RA)
+{
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    int q = RI[rpos ? rpos[i] : i];
+    for (int k = I[i]; k < I[i + 1]; ++k, ++q) { RJ[q] = cpos ? cpos[J[k]] : J[k]; RA[q] = A[k]; }
+}
+
+extern "C" int pe_mat_renumbered(pe_ctx *ctx, pe_mat *A, int transpose, const int32_t *rpos, int32_t nrows_out,
+                                 const int32_t *cpos, int32_t ncols_out, pe_mat **out)
+{
+    PE_CHECK(ctx && A && out, "bad arguments");
+    PE_CHECK(!A->distributed && A->offd.nnz == 0 && ctx->nranks == 1, "pe_mat_renumbered: single-rank matrices only");
+    if (transpose && !A->T) PE_TRY(pe_mat_transpose(ctx, A, &A->T));
+    pe_mat *S = transpose ? A->T : A;
+    DevCSR &src = S->diag;
+    PE_CHECK(!rpos || nrows_out >= src.nrows, "pe_mat_renumbered: row numbering shorter than the matrix");
+    PE_CHECK(!cpos || ncols_out >= src.ncols, "pe_mat_renumbered: column numbering shorter than the matrix");
+    PE_TRY(pe_sell_for_spmv(ctx, src));
+    cudaStream_t st = ctx->stream;
+    const int32_t nr = rpos ? nrows_out : src.nrows;
+    DevCSR M;
+    PE_TRY(devcsr_alloc(M, nr, cpos ? ncols_out : src.ncols, src.nnz));
+    PE_CUDA(cudaMemsetAsync(M.I, 0, sizeof(int32_t) * (size_t)(nr + 1), st));
+    if (src.nrows > 0)
+    {
+        k_renumber_row_lens<<<pe_grid_for(src.nrows, 256), 256, 0, st>>>(src.nrows, src.I, rpos, M.I);
+        PE_LAUNCHED(ctx);
+        void *tmp = nullptr; size_t tb = 0;
+        cub::DeviceScan::InclusiveSum(nullptr, tb, M.I, M.I, nr + 1, st);
+        PE_CUDA(cudaMalloc(&tmp, tb));
+        PE_CUDA(cub::DeviceScan::InclusiveSum(tmp, tb, M.I, M.I, nr + 1, st));
+        ctx->launches++;
+        k_renumber_fill<<<pe_grid_for(src.nrows, 256), 256, 0, st>>>(src.nrows, src.I, src.J, src.A, rpos, cpos, M.I, M.J, M.A);
+        PE_LAUNCHED(ctx);
+        PE_CUDA(cudaStreamSynchronize(st));
+        cudaFree(tmp);
+    }
+    PE_TRY(pe_mat_wrap_local(ctx, M, out));
+    pe_mat *R = *out;
+    R->tpr = S->tpr;
+    if (src.sell) PE_TRY(pe_sell_for_spmv(ctx, R->diag, true));
+    else R->diag.sell_state = -1;
+    PE_CUDA(cudaStreamSynchronize(st));
+    return 0;
 }
 
 // ---------------------------------------------------------------------------

@@ -34,6 +34,23 @@ inline void ComputeResidual(const mfem::Operator &A, const mfem::Vector &x, cons
 }
 } // namespace mg_utils
 
+/// the colour numbering of a multicolour SELL level (pe_smoother_colour_numbering): padded length and the device
+/// array row -> position; npad == 0: natural numbering
+struct ColourNumbering
+{
+    int32_t npad = 0;
+    const int32_t *pos = nullptr;
+};
+using MatHandle = std::shared_ptr<pe_mat>;
+/// copy of A (or of A^T) whose products read columns at cols.pos and write rows at rows.pos (natural where npad == 0)
+inline MatHandle RenumberedCopy(const mfem::HypreParMatrix &A, bool transpose, const ColourNumbering &rows,
+                                const ColourNumbering &cols)
+{
+    pe_mat *m = nullptr;
+    PE_CALL(pe_mat_renumbered(Device::Get(), A.Handle(), transpose ? 1 : 0, rows.pos, rows.npad, cols.pos, cols.npad, &m));
+    return MatHandle(m, [](pe_mat *p) { pe_mat_free(p); });
+}
+
 inline bool SolverCaptureSafe(const mfem::Solver *s)
 {
     auto p = dynamic_cast<const Solver *>(s);
@@ -70,6 +87,20 @@ public:
     /// all supported relaxations are symmetric operators
     void MultTranspose(const mfem::Vector &rhs, mfem::Vector &sol) const override { Mult(rhs, sol); }
     bool CaptureSafe() const override { return true; }
+    pe_smoother *Handle() const noexcept { return smoo_; }
+    /// colour numbering of a multicolour SELL Gauss-Seidel smoother on one rank (npad == 0: none)
+    ColourNumbering Numbering() const
+    {
+        ColourNumbering c;
+        PE_CALL(pe_smoother_colour_numbering(smoo_, &c.npad, &c.pos));
+        return c;
+    }
+    /// Mult on colour-numbered vectors (Numbering().npad entries); mode 0: sol is the initial guess, 1: zero initial
+    /// guess, 2: sol is what pe_smoother_colour_in left
+    void MultColour(const mfem::Vector &rhs, mfem::Vector &sol, int mode) const
+    {
+        PE_CALL(pe_smoother_apply_colour(smoo_, rhs.Read(), mode == 1 ? sol.Write() : sol.ReadWrite(), mode));
+    }
 private:
     void _do_set_operator(const Op_Ptr &) override { PARELAG_NOT_IMPLEMENTED(); }
     std::shared_ptr<mfem::HypreParMatrix> A_;
@@ -169,6 +200,38 @@ public:
     Op_Ptr GetAuxiliaryOperator() const { return A_aux_; }
     bool CaptureSafe() const override
     { return SolverCaptureSafe(PrimarySolver_.get()) && SolverCaptureSafe(AuxiliarySolver_.get()); }
+    pe_smoother *PrimaryHandle() const { return dynamic_cast<const HypreSmootherWrapper &>(*PrimarySolver_).Handle(); }
+    /// colour numbering of the primary smoother when both smoothers have one (npad == 0: none)
+    ColourNumbering Numbering() const
+    {
+        auto pri = dynamic_cast<const HypreSmootherWrapper *>(PrimarySolver_.get());
+        auto aux = dynamic_cast<const HypreSmootherWrapper *>(AuxiliarySolver_.get());
+        if (!pri || !aux || !dynamic_cast<const mfem::HypreParMatrix *>(D_op_.get()) || aux->Numbering().npad == 0) return {};
+        return pri->Numbering();
+    }
+    /// Build the renumbered D (primary <- auxiliary numbering) and D^T; residual: A in the primary numbering (borrowed).
+    void SetupColour(const MatHandle &residual)
+    {
+        auto pri = dynamic_cast<const HypreSmootherWrapper *>(PrimarySolver_.get());
+        auto aux = dynamic_cast<const HypreSmootherWrapper *>(AuxiliarySolver_.get());
+        auto &D = dynamic_cast<const mfem::HypreParMatrix &>(*D_op_);
+        const ColourNumbering p = pri->Numbering(), a = aux->Numbering();
+        cres_ = residual;
+        cDt_ = RenumberedCopy(D, true, a, p);
+        cD_ = RenumberedCopy(D, false, p, a);
+        cPrimaryVec_.SetSize(p.npad); cAuxB_.SetSize(a.npad); cAuxX_.SetSize(a.npad);
+    }
+    /// Mult on vectors in the primary colour numbering (after SetupColour): the same products as Mult, on renumbered
+    /// copies, and no renumbering passes; mode as HypreSmootherWrapper::MultColour
+    void MultColour(const mfem::Vector &B, mfem::Vector &X, int mode) const
+    {
+        pe_ctx *ctx = Device::Get();
+        dynamic_cast<const HypreSmootherWrapper &>(*PrimarySolver_).MultColour(B, X, mode);
+        PE_CALL(pe_residual(ctx, cres_.get(), X.Read(), B.Read(), cPrimaryVec_.Write()));
+        PE_CALL(pe_spmv(ctx, 1.0, cDt_.get(), cPrimaryVec_.Read(), 0.0, cAuxB_.Write()));
+        dynamic_cast<const HypreSmootherWrapper &>(*AuxiliarySolver_).MultColour(cAuxB_, cAuxX_, 1);
+        PE_CALL(pe_spmv(ctx, 1.0, cD_.get(), cAuxX_.Read(), 1.0, X.ReadWrite()));
+    }
 private:
     /// X += D AuxX_.  On one rank the add rides in the product (beta = 1): acc + X rounds like X + (D AuxX_), so the
     /// bits are those of the separate pass.  With a halo, D's diagonal and off-diagonal blocks are two passes, and
@@ -184,6 +247,8 @@ private:
     Op_Ptr A_, A_aux_, D_op_;
     std::shared_ptr<mfem::Solver> PrimarySolver_, AuxiliarySolver_;
     mutable mfem::Vector AuxB_, AuxX_, PrimaryVec_;
+    MatHandle cres_, cDt_, cD_;                             // colour-numbered products (SetupColour)
+    mutable mfem::Vector cPrimaryVec_, cAuxB_, cAuxX_;
 };
 
 class HiptmairSmootherFactory : public SolverFactory
@@ -788,11 +853,11 @@ public:
     /// one V-cycle (the "Cycle type" parameter is never read by the reference, SURVEY fact 4)
     void Mult(const mfem::Vector &rhs, mfem::Vector &sol) const override
     {
+        SetupColour();
         if (this->IsPreconditioner())
         {
             if (ReplayGraph(rhs, sol)) return;
-            sol = 0.0;
-            Iterate(rhs, sol, 0, 1, false);
+            Cycle(rhs, sol);
         }
         else
         {
@@ -800,12 +865,14 @@ public:
             Levels_.front()->Get<Op_Ptr>("A")->Mult(sol, rhs_view);
             rhs_view *= -1.0;
             rhs_view += rhs;
-            sol_view = 0.0;
-            Iterate(rhs_view, sol_view, 0, 1, false);
+            Cycle(rhs_view, sol_view);
             sol += sol_view;
         }
     }
-    void Iterate(const mfem::Vector &RHS, mfem::Vector &SOL, int StartLevel, int NumIterations, bool CycleThisLevel) const
+    /// Levels are visited as in the reference.  On a colour-numbered level (SetupColour) RHS and SOL are in the level's
+    /// colour numbering and SolMode tells the pre-smoother what SOL holds (HypreSmootherWrapper::MultColour).
+    void Iterate(const mfem::Vector &RHS, mfem::Vector &SOL, int StartLevel, int NumIterations, bool CycleThisLevel,
+                 int SolMode = 0) const
     {
         for (int iteration = 1; iteration <= NumIterations; ++iteration)
         {
@@ -822,28 +889,38 @@ public:
             }
             Level &Fine = *Levels_[StartLevel];
             Level &Coarse = *Levels_[StartLevel + 1];
-            if (Fine.IsValidKey("PreSmoother")) Fine.Get<Op_Ptr>("PreSmoother")->Mult(RHS, SOL);
+            const int l = StartLevel;
+            const bool fine_c = IsColourLevel(l), coarse_c = IsColourLevel(l + 1);
+            pe_ctx *ctx = Device::Get();
+            if (fine_c) SmoothColour(*Fine.Get<Op_Ptr>("PreSmoother"), RHS, SOL, iteration == 1 ? SolMode : 0);
+            else if (Fine.IsValidKey("PreSmoother")) Fine.Get<Op_Ptr>("PreSmoother")->Mult(RHS, SOL);
             // residual (K1+K7 fused: r = b - A x in one pass)
             tmp_resid_[StartLevel].SetSize(RHS.Size());
-            mg_utils::ComputeResidual(*Fine.Get<Op_Ptr>("A"), SOL, RHS, tmp_resid_[StartLevel]);
+            if (fine_c) PE_CALL(pe_residual(ctx, cres_[l].get(), SOL.Read(), RHS.Read(), tmp_resid_[l].Write()));
+            else mg_utils::ComputeResidual(*Fine.Get<Op_Ptr>("A"), SOL, RHS, tmp_resid_[StartLevel]);
             auto &P = Coarse.Get<Op_Ptr>("P");
-            if (ImplicitTranspose_ || !Fine.IsKey("R")) P->MultTranspose(tmp_resid_[StartLevel], CoarseResids_[StartLevel + 1]);
+            if (fine_c || coarse_c) PE_CALL(pe_spmv(ctx, 1.0, crestrict_[l].get(), tmp_resid_[l].Read(), 0.0, CoarseResids_[l + 1].Write()));
+            else if (ImplicitTranspose_ || !Fine.IsKey("R")) P->MultTranspose(tmp_resid_[StartLevel], CoarseResids_[StartLevel + 1]);
             else Fine.Get<Op_Ptr>("R")->Mult(tmp_resid_[StartLevel], CoarseResids_[StartLevel + 1]);
-            CoarseSols_[StartLevel + 1] = 0.0;
+            // a colour-numbered coarse level starts from a zero guess without the fill (SolMode 1)
+            if (!coarse_c) CoarseSols_[StartLevel + 1] = 0.0;
             int cycle_times = 0;
             if (CycleThisLevel && CycleMu_.size() > 1) cycle_times = CycleMu_[StartLevel];
             for (int cycle = 0; cycle <= cycle_times; ++cycle)
-                Iterate(CoarseResids_[StartLevel + 1], CoarseSols_[StartLevel + 1], StartLevel + 1, 1, false);
+                Iterate(CoarseResids_[StartLevel + 1], CoarseSols_[StartLevel + 1], StartLevel + 1, 1, false,
+                        coarse_c && cycle == 0 ? 1 : 0);
             // SOL += P * e  (K1 with beta = 1: prolongation and correction in one pass)
             auto P_hyp = std::dynamic_pointer_cast<mfem::HypreParMatrix>(P);
-            if (P_hyp) P_hyp->Mult(1.0, CoarseSols_[StartLevel + 1], 1.0, SOL);
+            if (fine_c || coarse_c) PE_CALL(pe_spmv(ctx, 1.0, cprolong_[l].get(), CoarseSols_[l + 1].Read(), 1.0, SOL.ReadWrite()));
+            else if (P_hyp) P_hyp->Mult(1.0, CoarseSols_[StartLevel + 1], 1.0, SOL);
             else
             {
                 tmp_correct_[StartLevel].SetSize(P->Height());
                 P->Mult(CoarseSols_[StartLevel + 1], tmp_correct_[StartLevel]);
                 SOL += tmp_correct_[StartLevel];
             }
-            if (Fine.IsValidKey("PostSmoother")) Fine.Get<Op_Ptr>("PostSmoother")->Mult(RHS, SOL);
+            if (fine_c) SmoothColour(*Fine.Get<Op_Ptr>("PostSmoother"), RHS, SOL, 0);
+            else if (Fine.IsValidKey("PostSmoother")) Fine.Get<Op_Ptr>("PostSmoother")->Mult(RHS, SOL);
         }
     }
     void Finalize()
@@ -858,6 +935,86 @@ public:
         }
     }
 private:
+    bool IsColourLevel(int l) const { return colour_state_ > 0 && l < (int)colour_.size() && colour_[l].npad > 0; }
+    static void SmoothColour(const mfem::Operator &S, const mfem::Vector &B, mfem::Vector &X, int mode)
+    {
+        if (auto h = dynamic_cast<const HiptmairSmoother *>(&S)) h->MultColour(B, X, mode);
+        else dynamic_cast<const HypreSmootherWrapper &>(S).MultColour(B, X, mode);
+    }
+    static ColourNumbering SmootherNumbering(const mfem::Operator &S)
+    {
+        if (auto h = dynamic_cast<const HiptmairSmoother *>(&S)) return h->Numbering();
+        if (auto w = dynamic_cast<const HypreSmootherWrapper *>(&S)) return w->Numbering();
+        return {};
+    }
+    /// sol = one V-cycle from a zero guess.  With a colour-numbered fine level the right-hand side is renumbered on
+    /// entry, in the same pass as the first colour of the pre-smoother's first sweep, and the solution on exit.
+    void Cycle(const mfem::Vector &rhs, mfem::Vector &sol) const
+    {
+        if (!IsColourLevel(0))
+        {
+            sol = 0.0;
+            Iterate(rhs, sol, 0, 1, false);
+            return;
+        }
+        pe_smoother *s = PrimaryHandle(*Levels_[0]->Get<Op_Ptr>("PreSmoother"));
+        PE_CALL(pe_smoother_colour_in(s, rhs.Read(), CoarseResids_[0].Write(), CoarseSols_[0].Write()));
+        Iterate(CoarseResids_[0], CoarseSols_[0], 0, 1, false, 2);
+        PE_CALL(pe_smoother_colour_out(s, CoarseSols_[0].Read(), sol.Write()));
+    }
+    static pe_smoother *PrimaryHandle(const mfem::Operator &S)
+    {
+        if (auto h = dynamic_cast<const HiptmairSmoother *>(&S)) return h->PrimaryHandle();
+        return dynamic_cast<const HypreSmootherWrapper &>(S).Handle();
+    }
+    /// Colour-numbered levels (one rank): a level whose pre- and post-smoother are one multicolour SELL Gauss-Seidel
+    /// smoother, or one Hiptmair smoother of two, keeps its vectors in that smoother's colour numbering for the whole
+    /// cycle.  Its residual, restriction, prolongation (and Hiptmair's D, D^T) run on renumbered copies built here, so
+    /// the smoothers need no renumbering passes.  Every other level keeps the natural numbering.
+    void SetupColour() const
+    {
+        if (colour_state_ != 0) return;
+        colour_state_ = -1;
+        pe_ctx *ctx = Device::Get();
+        if (pe_ctx_nranks(ctx) != 1 || pe_ctx_is_capturing(ctx) || pe_ctx_is_recording(ctx)) return;
+        const int L = (int)Levels_.size();
+        colour_.assign(L, ColourNumbering());
+        cres_.assign(L, nullptr); crestrict_.assign(L, nullptr); cprolong_.assign(L, nullptr);
+        bool any = false;
+        for (int l = 0; l + 1 < L; ++l)
+        {
+            Level &lev = *Levels_[l];
+            if (!lev.IsValidKey("PreSmoother") || !lev.IsValidKey("PostSmoother")) continue;
+            auto pre = lev.Get<Op_Ptr>("PreSmoother");
+            if (pre != lev.Get<Op_Ptr>("PostSmoother")) continue;
+            auto A = std::dynamic_pointer_cast<mfem::HypreParMatrix>(lev.Get<Op_Ptr>("A"));
+            auto P = std::dynamic_pointer_cast<mfem::HypreParMatrix>(Levels_[l + 1]->Get<Op_Ptr>("P"));
+            if (!A || !P || !(ImplicitTranspose_ || !lev.IsKey("R"))) continue;
+            const ColourNumbering c = SmootherNumbering(*pre);
+            if (c.npad == 0) continue;
+            colour_[l] = c;
+            cres_[l] = RenumberedCopy(*A, false, c, c);
+            if (auto h = dynamic_cast<HiptmairSmoother *>(pre.get())) h->SetupColour(cres_[l]);
+            any = true;
+        }
+        if (!any) return;
+        for (int l = 0; l + 1 < L; ++l)
+        {
+            if (colour_[l].npad == 0 && colour_[l + 1].npad == 0) continue;
+            auto &P = dynamic_cast<const mfem::HypreParMatrix &>(*Levels_[l + 1]->Get<Op_Ptr>("P"));
+            crestrict_[l] = RenumberedCopy(P, true, colour_[l + 1], colour_[l]);
+            cprolong_[l] = RenumberedCopy(P, false, colour_[l], colour_[l + 1]);
+        }
+        for (int l = 0; l < L; ++l)
+            if (colour_[l].npad > 0)
+            {
+                // padding entries are allocated zeroed and never written
+                CoarseResids_[l] = mfem::Vector(); CoarseResids_[l].SetSize(colour_[l].npad);
+                CoarseSols_[l] = mfem::Vector(); CoarseSols_[l].SetSize(colour_[l].npad);
+                tmp_resid_[l] = mfem::Vector(); tmp_resid_[l].SetSize(colour_[l].npad);
+            }
+        colour_state_ = 1;
+    }
     /// Preconditioner-mode V-cycle through a CUDA graph: the first call with a given (rhs, sol)
     /// buffer pair runs directly (it allocates work vectors and builds lazy matrix formats), the
     /// second call records the cycle, later calls replay it.  Returns false when the cycle has to
@@ -896,7 +1053,7 @@ private:
         {
             // record the cycle: every C-ABI call below appends an op instead of launching
             bool rec_ok = true;
-            try { sol = 0.0; Iterate(rhs, sol, 0, 1, false); }
+            try { Cycle(rhs, sol); }
             catch (...) { rec_ok = false; }
             pe_program *p = nullptr;
             if (pe_program_end(ctx, &p) == 0 && rec_ok)
@@ -912,7 +1069,7 @@ private:
         if (!use_graph_ || graph_failed_) return false;
         if (pe_graph_begin(ctx) != 0) { graph_failed_ = true; return false; }
         bool ok = true;
-        try { sol = 0.0; Iterate(rhs, sol, 0, 1, false); }
+        try { Cycle(rhs, sol); }
         catch (...) { ok = false; }
         pe_graph *g = nullptr;
         if (pe_graph_end(ctx, &g) != 0 || !ok)
@@ -944,6 +1101,9 @@ private:
     mutable int last_mode_ = 0;                 // LastReplayMode()
     mutable pe_graph *graph_ = nullptr;
     mutable const void *graph_rhs_ = nullptr, *graph_sol_ = nullptr, *warm_rhs_ = nullptr, *warm_sol_ = nullptr;
+    mutable int colour_state_ = 0;              // SetupColour: 0 not yet, 1 some level colour-numbered, -1 none
+    mutable std::vector<ColourNumbering> colour_;
+    mutable std::vector<MatHandle> cres_, crestrict_, cprolong_;   // per level: A_l, P_{l+1}^T, P_{l+1} renumbered
 };
 
 /// Hierarchy.cpp:282-383: per coarse level P = ComputeTrueP(form, ess); A <- P^T A P; FixZeroRows

@@ -231,6 +231,8 @@ int pe_mat_download(const pe_mat *A, int32_t *diag_i, int32_t *diag_j, double *d
                     int32_t *offd_i, int32_t *offd_j, double *offd_data,
                     int64_t *col_map_offd);
 int pe_mat_free(pe_mat *A);
+/* copy of a single-rank matrix: its row pointers, columns and values (no cached transpose or SELL copy) */
+int pe_mat_clone(pe_ctx *ctx, const pe_mat *A, pe_mat **out);
 /* explicit local transpose (counting-sort order: ascending columns per row).
  * mfem::Transpose / hypre_ParCSRMatrixTranspose2 (src/hypreExtension/par_Tmatmul.c:41-79) */
 int pe_mat_transpose(pe_ctx *ctx, const pe_mat *A, pe_mat **out);
@@ -260,6 +262,12 @@ int pe_residual(pe_ctx *ctx, pe_mat *A, const pe_vec *x, const pe_vec *b, pe_vec
  * beta * y).  Free with pe_mat_free. */
 int pe_mat_renumbered(pe_ctx *ctx, pe_mat *A, int transpose, const int32_t *rpos, int32_t nrows_out,
                       const int32_t *cpos, int32_t ncols_out, pe_mat **out);
+/* Values only: R, made by pe_mat_renumbered(ctx, B, 0, rpos, ...) from a matrix B with A's pattern, takes A's values
+ * (the same row map rpos); its pattern is kept and its products equal those of pe_mat_renumbered(A) bit for bit. */
+int pe_mat_renumbered_values(pe_ctx *ctx, pe_mat *A, const int32_t *rpos, pe_mat *R);
+/* *same = 1 when A and B (single rank) have the same sizes, row pointers and column indices: one device pass, one
+ * flag downloaded */
+int pe_mat_same_pattern(pe_ctx *ctx, const pe_mat *A, const pe_mat *B, int32_t *same);
 
 /* ---- K3/K4/K5: hypre relaxation (mfem::HypreSmoother behind
  * parelag::HypreSmootherWrapper, src/linalg/solver_ops/ParELAG_HypreSmootherWrapper.cpp:20-35;
@@ -292,6 +300,12 @@ int pe_smoother_apply_colour(pe_smoother *s, const pe_vec *f, pe_vec *u, int mod
  * pe_smoother_apply_colour(mode 2).  pe_smoother_colour_out: x (natural) = u (colour order). */
 int pe_smoother_colour_in(pe_smoother *s, const pe_vec *b, pe_vec *f, pe_vec *u);
 int pe_smoother_colour_out(pe_smoother *s, const pe_vec *u, pe_vec *x);
+/* New values for a smoother (mfem::Solver::SetOperator on a built HypreSmootherWrapper): A (borrowed) must have the
+ * size and sparsity pattern of the smoother's matrix, else the call fails and changes nothing.  The smoother then
+ * works on A, with everything recomputed that a pe_smoother_create on A would compute from the values (l1 norms,
+ * diagonal, the values of its set-ordered CSR / colour-ordered SELL copy, Chebyshev bounds and coefficients), and
+ * with its colouring, level sets, copy layouts and colour numbering (pos_d) kept. */
+int pe_smoother_update(pe_smoother *s, pe_mat *A);
 
 /* ---- K8/K9: sparse products
  * C = A*B (mfem::ParMult / hypre_ParMatmul; SchurComplementFactory.cpp:51-166)
@@ -304,6 +318,15 @@ int pe_smoother_colour_out(pe_smoother *s, const pe_vec *u, pe_vec *x);
 int pe_spgemm(pe_ctx *ctx, const pe_mat *A, const pe_mat *B, pe_mat **C);
 int pe_rap(pe_ctx *ctx, const pe_mat *R_or_null, const pe_mat *A, const pe_mat *P, pe_mat **Ac);
 int pe_fix_zero_rows(pe_ctx *ctx, pe_mat *A, int32_t *num_fixed);
+/* Numeric pass only (single rank): C / Ac already hold the pattern of the product (row pointers, ascending columns),
+ * e.g. from an earlier pe_spgemm / pe_rap with operands of the same patterns; only their values are overwritten, with
+ * the summation order of the two-pass product, so the values are those pe_spgemm / pe_rap compute, bit for bit.
+ * pe_rap_numeric recomputes the intermediate A*P with the two-pass product and uses P's cached transpose. */
+int pe_spgemm_numeric(pe_ctx *ctx, const pe_mat *A, const pe_mat *B, pe_mat *C);
+int pe_rap_numeric(pe_ctx *ctx, const pe_mat *A, const pe_mat *P, pe_mat *Ac);
+/* The rows pe_fix_zero_rows rewrites (l1 norm below DBL_EPSILON).  changed == NULL: mask (length = rows of A) becomes
+ * 1.0 on those rows and 0.0 elsewhere.  Otherwise mask is only read and *changed = 1 when that set differs from it. */
+int pe_mat_zero_rows(pe_ctx *ctx, const pe_mat *A, pe_vec *mask, int32_t *changed);
 int pe_spadd(pe_ctx *ctx, double a, const pe_mat *A, double b, const pe_mat *B, pe_mat **C);
 /* mfem::SparseMatrix::EliminateRowCol(rc, DIAG_ONE) for every marked dof (marker_host[n],
  * non-zero = essential): marked rows become unit rows, marked columns are zeroed; entries

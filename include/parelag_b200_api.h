@@ -213,6 +213,14 @@ int pe_api_solver_replay_mode(const pe_solver *s, int *mode);
 int pe_api_solver_level_info(const pe_solver *s, int level, int64_t *nrows, int64_t *nnz, int64_t *nnz_P);
 /* download A (diag block) of a hierarchy level for parity tests; arrays sized from level_info */
 int pe_api_solver_level_matrix(const pe_solver *s, int level, int32_t *I, int32_t *J, double *A);
+/* solver->SetOperator(A) (mfem::Solver::SetOperator, ParELAG_Solver.hpp:57-65): new values with the held operator's size
+ * and sparsity pattern, e.g. the next time step of M + dt K.  The solver is left as a build on A would leave it (one
+ * rank, single-form AMGe hierarchies: numeric-only Galerkin products, smoothers and coarse solver refreshed; the recorded
+ * V-cycle is dropped and recorded again).  Ownership of A passes to the solver; it is released when the call is refused:
+ * a different size or pattern, a changed FixZeroRows row set on a coarse level or of a Hiptmair auxiliary operator, a
+ * blocked operator, more than one rank.  A refused call leaves the solver as it was.  Krylov solvers: the preconditioner
+ * takes A first, then the Krylov solver. */
+int pe_api_solver_set_operator(pe_solver *s, pe_mat *A);
 int pe_api_solver_free(pe_solver *s);
 
 /* TimeManager: seconds accumulated under a timer name; clear all timers */

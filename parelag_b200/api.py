@@ -363,6 +363,12 @@ class Solver:
         _chk(lib().pe_api_solver_build(xml.encode(), name.encode(), C.byref(H), None if seq is None else seq.h,
                                        start_level, form, _ptr(ess), 0 if ess is None else len(ess), C.byref(self.h)))
 
+    def set_operator(self, A):
+        """SetOperator on the built solver: A (capi.Mat) has the held operator's size and sparsity pattern and new
+        values.  Ownership of A passes to the solver, also when the call is refused (capi.PEError)."""
+        h, A.h = A.h, None
+        _chk(lib().pe_api_solver_set_operator(self.h, h))
+
     def mult(self, b, x0=None):
         b = _f64(b)
         x = np.zeros(self.n) if x0 is None else _f64(x0).copy()

@@ -331,6 +331,11 @@ class Mat:
                                      C.c_void_p(cpos), C.c_int32(ncols_out), C.byref(out.h)))
         return out
 
+    def same_pattern(self, other):
+        same = C.c_int32()
+        _chk(lib().pe_mat_same_pattern(self.ctx.h, self.h, other.h, C.byref(same)))
+        return bool(same.value)
+
     def fix_zero_rows(self):
         n = C.c_int32()
         _chk(lib().pe_fix_zero_rows(self.ctx.h, self.h, C.byref(n)))
@@ -383,6 +388,16 @@ def rap(ctx, A, P, R=None):
     return out
 
 
+def spgemm_numeric(ctx, A, B, Cm):
+    """pe_spgemm_numeric: Cm (pattern of A*B) takes the values of A*B"""
+    _chk(lib().pe_spgemm_numeric(ctx.h, A.h, B.h, Cm.h))
+
+
+def rap_numeric(ctx, A, P, Ac):
+    """pe_rap_numeric: Ac (pattern of P^T A P) takes the values of P^T A P"""
+    _chk(lib().pe_rap_numeric(ctx.h, A.h, P.h, Ac.h))
+
+
 def spadd(ctx, a, A, b, B):
     out = Mat(ctx)
     _chk(lib().pe_spadd(ctx.h, C.c_double(a), A.h, C.c_double(b), B.h, C.byref(out.h)))
@@ -405,6 +420,11 @@ class Smoother:
 
     def apply(self, b, x, iterative_mode=True):
         _chk(lib().pe_smoother_apply(self.h, b.h, x.h, 1 if iterative_mode else 0))
+
+    def update(self, A):
+        """pe_smoother_update: the smoother takes A's values (same size and pattern; A stays owned by the caller)"""
+        _chk(lib().pe_smoother_update(self.h, A.h))
+        self.A = A
 
     def colour_numbering(self):
         """(npad, device pointer of row -> colour position); (0, None) without a colour numbering"""

@@ -802,6 +802,27 @@ int pe_mat_wrap_local(pe_ctx *ctx, DevCSR &diag, pe_mat **out)
     return 0;
 }
 
+extern "C" int pe_mat_clone(pe_ctx *ctx, const pe_mat *A, pe_mat **out)
+{
+    PE_CHECK(ctx && A && out, "bad arguments");
+    PE_CHECK(!A->distributed && A->offd.nnz == 0, "pe_mat_clone: single-rank matrices only");
+    DevCSR c;
+    PE_TRY(devcsr_alloc(c, A->diag.nrows, A->diag.ncols, A->diag.nnz));
+    cudaStream_t st = ctx->stream;
+    PE_CUDA(cudaMemcpyAsync(c.I, A->diag.I, sizeof(int32_t) * (size_t)(c.nrows + 1), cudaMemcpyDeviceToDevice, st));
+    if (c.nnz > 0)
+    {
+        PE_CUDA(cudaMemcpyAsync(c.J, A->diag.J, sizeof(int32_t) * (size_t)c.nnz, cudaMemcpyDeviceToDevice, st));
+        PE_CUDA(cudaMemcpyAsync(c.A, A->diag.A, sizeof(double) * (size_t)c.nnz, cudaMemcpyDeviceToDevice, st));
+    }
+    PE_TRY(pe_mat_wrap_local(ctx, c, out));
+    (*out)->global_num_rows = A->global_num_rows;
+    (*out)->global_num_cols = A->global_num_cols;
+    (*out)->tpr = A->tpr;
+    PE_CUDA(cudaStreamSynchronize(st));
+    return 0;
+}
+
 extern "C" int pe_mat_info(const pe_mat *A, int32_t *num_rows, int32_t *num_cols_diag,
                            int32_t *num_cols_offd, int64_t *nnz_diag, int64_t *nnz_offd)
 {

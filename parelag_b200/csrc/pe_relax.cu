@@ -46,7 +46,8 @@ struct pe_smoother {
     std::vector<int32_t> set_wmax;      // widest slice of every colour (selects the kernel's entry-group size)
     std::vector<double> set_bytes;      // algorithmic bytes of one colour launch
     uint64_t pol_gather = 0;            // L2 policy word of the u-gathers (PE_TUNE_GATHER_KEEP_PCT at creation)
-    bool skip_turn = false;             // the backward pass may start at the second-to-last colour (see build_gs_schedule)
+    bool skip_turn = false;             // the backward pass may start at the second-to-last colour (see set_skip_turn)
+    int32_t *last_rows_d = nullptr;     // rows of the last set, for set_skip_turn
     int32_t *pos_d = nullptr;           // row -> colour-ordered position
     double *l1p_d = nullptr, *fp_d = nullptr, *up_d = nullptr;
     // fused sweep (PE_TUNE_FUSED_GS_MAX_MB): all colours of a symmetric sweep in one cooperative kernel
@@ -334,13 +335,41 @@ __global__ void k_perm_fill(int n, const int *__restrict__ perm, const int *__re
     int i = perm[k];
     int q = pI[k];
     for (int t = dI[i]; t < dI[i + 1]; ++t, ++q) {
-        pJ[q] = dJ[t]; pA[q] = dA[t];
+        if (pJ) pJ[q] = dJ[t];
+        pA[q] = dA[t];
         if (before) before[q] = pos[dJ[t]] < k ? 1 : 0;
     }
     if (oI) for (int t = oI[i]; t < oI[i + 1]; ++t, ++q) {
-        pJ[q] = ncd + oJ[t]; pA[q] = oA[t];
+        if (pJ) pJ[q] = ncd + oJ[t];
+        pA[q] = oA[t];
         if (before) before[q] = 0;
     }
+}
+// values of the colour-ordered SELL copy (pe_smoother_update): row i sits on lane pos[i] % 32 of slice pos[i] / 32, its
+// diag then offd entries in CSR order (k_sell_fill); padding entries keep their 0
+__global__ void k_sell_refill(int n, const int *__restrict__ pos, const int *__restrict__ soff,
+                              const int *__restrict__ dI, const double *__restrict__ dA,
+                              const int *__restrict__ oI, const double *__restrict__ oA, double *SA)
+{
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const int p = pos[i];
+    int64_t q = (int64_t)soff[p >> 5] * 32 + (p & 31);
+    for (int t = dI[i]; t < dI[i + 1]; ++t, q += 32) SA[q] = dA[t];
+    if (oI) for (int t = oI[i]; t < oI[i + 1]; ++t, q += 32) SA[q] = oA[t];
+}
+// the rule of build_gs_schedule for skipping the second visit of the last set: every row of it has a positive diagonal
+// equal to its l1 norm and no ghost entries.  *bad = 1 when a row breaks it.
+__global__ void k_last_set_check(int m, const int *__restrict__ rows, const int *__restrict__ dI, const int *__restrict__ dJ,
+                                 const double *__restrict__ dA, const int *__restrict__ oI, const double *__restrict__ l1,
+                                 int *bad)
+{
+    const int k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= m) return;
+    const int i = rows[k];
+    double aii = 0.0;
+    for (int q = dI[i]; q < dI[i + 1]; ++q) if (dJ[q] == i) aii = dA[q];
+    if (!(aii > 0.0 && l1[i] == aii && (!oI || oI[i + 1] == oI[i]))) *bad = 1;
 }
 
 // host: schedule construction -------------------------------------------------
@@ -415,6 +444,36 @@ static void build_slabs(int n, const int *I, const int *J, int nslabs, std::vect
 #include <cub/cub.cuh>
 
 static int fused_setup(pe_smoother *s);
+// The forward pass ends and the backward pass starts with the LAST set.  Its rows are mutually independent, so right
+// after the forward update row i has residual f_i - sum_j a_ij u_j = (1 - a_ii / d_i) r_i, which is exactly 0 when
+// d_i == a_ii: the repeated update adds only the rounding error of that zero.  When every row of the last set has
+// d_i == a_ii (no ghost entries, l1 == diagonal) the second visit is skipped -- 1/nsets of the matrix traffic of a sweep.
+// Depends on the values: evaluated when the smoother is built and when its matrix takes new values.
+static int set_skip_turn(pe_smoother *s)
+{
+    s->skip_turn = false;
+    const int nsets = s->nsets;
+    if (!(nsets >= 2 && s->type == 2 && s->ordering == PE_GS_ORDER_MULTICOLOR && s->weight == 1.0 && s->omega == 1.0)) return 0;
+    pe_ctx *ctx = s->ctx;
+    pe_mat *A = s->A;
+    const int m = s->set_starts[nsets] - s->set_starts[nsets - 1];
+    if (m == 0) { s->skip_turn = true; return 0; }
+    int *bad = reinterpret_cast<int *>(ctx->scalar_d + 4), h = 0;
+    if (!s->last_rows_d)
+    {
+        PE_CUDA(cudaMalloc(&s->last_rows_d, sizeof(int32_t) * (size_t)m));
+        PE_CUDA(cudaMemcpyAsync(s->last_rows_d, s->order.data() + s->set_starts[nsets - 1], sizeof(int32_t) * (size_t)m,
+                                cudaMemcpyHostToDevice, ctx->stream));
+    }
+    PE_CUDA(cudaMemsetAsync(bad, 0, sizeof(int), ctx->stream));
+    k_last_set_check<<<pe_grid_for(m, 256), 256, 0, ctx->stream>>>(m, s->last_rows_d, A->diag.I, A->diag.J, A->diag.A,
+                                                                   A->offd.nnz > 0 ? A->offd.I : nullptr, s->l1_d, bad);
+    PE_LAUNCHED(ctx);
+    PE_CUDA(cudaMemcpyAsync(&h, bad, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+    PE_CUDA(cudaStreamSynchronize(ctx->stream));
+    s->skip_turn = h == 0;
+    return 0;
+}
 static int build_gs_schedule(pe_smoother *s)
 {
     pe_ctx *ctx = s->ctx;
@@ -462,28 +521,7 @@ static int build_gs_schedule(pe_smoother *s)
     std::vector<int> next(s->set_starts.begin(), s->set_starts.end() - 1), pos(n);
     for (int i = 0; i < n; ++i) { int p = next[key[i]]++; s->order[p] = i; pos[i] = p; }
 
-    // The forward pass ends and the backward pass starts with the LAST set.  Its rows are mutually
-    // independent, so right after the forward update row i has residual f_i - sum_j a_ij u_j =
-    // (1 - a_ii / d_i) r_i, which is exactly 0 when d_i == a_ii: the repeated update adds only the
-    // rounding error of that zero.  When every row of the last set has d_i == a_ii (no ghost entries,
-    // l1 == diagonal) the second visit is skipped -- 1/nsets of the matrix traffic of a sweep.
-    if (nsets >= 2 && s->type == 2 && s->ordering == PE_GS_ORDER_MULTICOLOR && s->weight == 1.0 && s->omega == 1.0)
-    {
-        std::vector<double> l1h(n), Ah((size_t)A->diag.nnz);
-        std::vector<int> oIt;
-        PE_CUDA(cudaMemcpy(l1h.data(), s->l1_d, sizeof(double) * (size_t)n, cudaMemcpyDeviceToHost));
-        if (A->diag.nnz) PE_CUDA(cudaMemcpy(Ah.data(), A->diag.A, sizeof(double) * (size_t)A->diag.nnz, cudaMemcpyDeviceToHost));
-        if (A->offd.nnz > 0) { oIt.resize(n + 1); PE_CUDA(cudaMemcpy(oIt.data(), A->offd.I, sizeof(int) * (size_t)(n + 1), cudaMemcpyDeviceToHost)); }
-        bool ok = true;
-        for (int k = s->set_starts[nsets - 1]; k < s->set_starts[nsets] && ok; ++k)
-        {
-            const int i = s->order[k];
-            double aii = 0.0;
-            for (int q = I[i]; q < I[i + 1]; ++q) if (J[q] == i) aii = Ah[q];
-            ok = aii > 0.0 && l1h[i] == aii && (oIt.empty() || oIt[i + 1] == oIt[i]);
-        }
-        s->skip_turn = ok;
-    }
+    PE_TRY(set_skip_turn(s));
 
     bool general = !(s->weight == 1.0 && s->omega == 1.0);
     // Colour-ordered SELL streaming (thread per row) for bandwidth-bound levels; below
@@ -715,7 +753,7 @@ static int cheby_setup(pe_smoother *s)
     pe_mat *A = s->A;
     int n = A->diag.nrows;
     cudaStream_t st = ctx->stream;
-    PE_CUDA(cudaMalloc(&s->ds_d, sizeof(double) * (size_t)(n > 0 ? n : 1)));
+    if (!s->ds_d) PE_CUDA(cudaMalloc(&s->ds_d, sizeof(double) * (size_t)(n > 0 ? n : 1)));
     k_inv_sqrt_diag<<<pe_grid_for(n, 256), 256, 0, st>>>(n, A->diag.I, A->diag.J, A->diag.A, s->ds_d);
     PE_LAUNCHED(ctx);
     // hypre_ParCSRMaxEigEstimateCG(A, scale=1, max_iter=10)
@@ -832,9 +870,65 @@ extern "C" int pe_smoother_free(pe_smoother *s)
     if (s->up_d) cudaFree(s->up_d);
     if (s->fused_steps_d) cudaFree(s->fused_steps_d);
     if (s->fused_bar_d) cudaFree(s->fused_bar_d);
+    if (s->last_rows_d) cudaFree(s->last_rows_d);
     pe_sell_free(s->S);
     devcsr_free(s->P);
     delete s;
+    return 0;
+}
+
+// New values, same pattern: what depends on the values is recomputed (l1 norms / diagonal, the values of the set-ordered
+// CSR or colour-ordered SELL copy, the colour-ordered l1, the last-set rule, the Chebyshev bounds and coefficients);
+// the schedule, the copies' layouts, pos_d and the fused-step tables are kept.
+extern "C" int pe_smoother_update(pe_smoother *s, pe_mat *A)
+{
+    PE_CHECK(s && A, "bad arguments");
+    pe_ctx *ctx = s->ctx;
+    PE_CHECK(!ctx->rec && !ctx->capturing, "pe_smoother_update: not while a program or graph is being recorded");
+    int32_t same = 0;
+    PE_TRY(pe_mat_same_pattern(ctx, s->A, A, &same));
+    PE_CHECK(same, "pe_smoother_update: the new matrix has a different size or sparsity pattern");
+    s->A = A;
+    cudaStream_t st = ctx->stream;
+    const int n = A->diag.nrows;
+    const int type = s->type;
+    const int l1opt = (type == 0 || type == 6 || type == 16) ? 0 : type;
+    const int *oI = A->offd.nnz > 0 ? A->offd.I : nullptr;
+    k_l1_norms<<<pe_grid_for(n, 256), 256, 0, st>>>(n, A->diag.I, A->diag.J, A->diag.A, oI, A->offd.A, l1opt, s->l1_d);
+    PE_LAUNCHED(ctx);
+    if (type == 2 || type == 4 || type == 6)
+    {
+        if (s->use_sell)
+        {
+            if (n > 0)
+            {
+                k_sell_refill<<<pe_grid_for(n, 256), 256, 0, st>>>(n, s->pos_d, s->S.soff, A->diag.I, A->diag.A, oI,
+                                                                    A->offd.A, s->S.A);
+                PE_LAUNCHED(ctx);
+            }
+            PE_TRY(pe_launch_perm_in(ctx, n, s->pos_d, s->l1_d, nullptr, s->l1p_d, s->up_d));
+        }
+        else if (n > 0)
+        {
+            k_perm_fill<<<pe_grid_for(n, 256), 256, 0, st>>>(n, s->perm_d, nullptr, A->diag.I, A->diag.J, A->diag.A,
+                                                             oI, A->offd.J, A->offd.A, A->diag.ncols,
+                                                             s->P.I, nullptr, s->P.A, nullptr);
+            PE_LAUNCHED(ctx);
+        }
+        const bool skip_before = s->skip_turn;
+        PE_TRY(set_skip_turn(s));
+        if (s->fused && s->skip_turn != skip_before)
+        {
+            // the fused-step table lists the colours of the backward pass
+            PE_CUDA(cudaStreamSynchronize(st));
+            cudaFree(s->fused_steps_d); cudaFree(s->fused_bar_d);
+            s->fused_steps_d = nullptr; s->fused_bar_d = nullptr;
+            s->fused = false;
+            PE_TRY(fused_setup(s));
+        }
+    }
+    else if (type == 16) PE_TRY(cheby_setup(s));
+    PE_CUDA(cudaStreamSynchronize(st));
     return 0;
 }
 

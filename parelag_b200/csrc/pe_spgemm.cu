@@ -363,6 +363,191 @@ extern "C" int pe_rap(pe_ctx *ctx, const pe_mat *R, const pe_mat *A, const pe_ma
 }
 
 // ---------------------------------------------------------------------------
+// Numeric pass into a known pattern (pe_spgemm_numeric / pe_rap_numeric): the sorted columns of a row of C are its slot
+// table, and a product a_ik * b_kj lands on the slot of column j found by binary search.  The group finishes entry ka of
+// A's row before any thread starts ka+1, and every slot gets at most one add per ka (the columns of a B row are
+// distinct), so every entry of C is summed in the order of k_spgemm_smem / k_spgemm_gmem, starting from 0.0, and the
+// values are theirs bit for bit.  The product and the add are rounded separately, as the atomicAdd of those kernels.
+// CAP > 0: the row is staged in shared memory (CAP slots per group); CAP == 0: one CTA per row, in place in C.
+__global__ void k_row_len(int n, const int *__restrict__ I, int *len)
+{
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) len[i] = I[i + 1] - I[i];
+}
+
+template <int GT, int CAP>
+__global__ void __launch_bounds__(256)
+k_spgemm_refill(int nlist, const int *__restrict__ list,
+                const int *__restrict__ AI, const int *__restrict__ AJ, const double *__restrict__ AA,
+                const int *__restrict__ BI, const int *__restrict__ BJ, const double *__restrict__ BA,
+                const int *__restrict__ CI, const int *__restrict__ CJ, double *CA)
+{
+    extern __shared__ unsigned char smem_raw[];
+    constexpr int GROUPS = 256 / GT;
+    const int g = threadIdx.x / GT, tid = threadIdx.x % GT;
+    const int li = blockIdx.x * GROUPS + g;
+    const bool active = li < nlist;   // whole group is uniform
+    const int row = active ? list[li] : 0;
+    const int c0 = active ? CI[row] : 0, m = active ? CI[row + 1] - c0 : 0;
+    const int *keys;
+    double *vals;
+    if (CAP > 0)
+    {
+        vals = reinterpret_cast<double *>(smem_raw) + g * CAP;
+        int *k = reinterpret_cast<int *>(smem_raw + sizeof(double) * CAP * GROUPS) + g * CAP;
+        for (int t = tid; t < m; t += GT) { k[t] = CJ[c0 + t]; vals[t] = 0.0; }
+        keys = k;
+    }
+    else
+    {
+        keys = CJ + c0;
+        vals = CA + c0;
+        for (int t = tid; t < m; t += GT) vals[t] = 0.0;
+    }
+    if (GT == 32) __syncwarp(); else __syncthreads();
+    if (active)
+    {
+        for (int ka = AI[row]; ka < AI[row + 1]; ++ka)
+        {
+            const int k = AJ[ka];
+            const double a = AA[ka];
+            for (int kb = BI[k] + tid; kb < BI[k + 1]; kb += GT)
+            {
+                const int col = BJ[kb];
+                int lo = 0, hi = m;
+                while (lo < hi) { const int mid = (lo + hi) >> 1; if (keys[mid] < col) lo = mid + 1; else hi = mid; }
+                if (lo < m && keys[lo] == col) vals[lo] = __dadd_rn(vals[lo], __dmul_rn(a, BA[kb]));
+            }
+            if (GT == 32) __syncwarp(); else __syncthreads();
+        }
+    }
+    if (CAP > 0) for (int t = tid; t < m; t += GT) CA[c0 + t] = vals[t];
+}
+
+int pe_devcsr_spgemm_numeric(pe_ctx *ctx, const DevCSR &A, const DevCSR &B, DevCSR &C)
+{
+    PE_CHECK(A.ncols == B.nrows && C.nrows == A.nrows && C.ncols == B.ncols, "spgemm_numeric: size mismatch");
+    const int n = A.nrows;
+    if (n == 0 || C.nnz == 0) return 0;
+    cudaStream_t st = ctx->stream;
+    // bins by the row length of C: <= 64 and <= 512 entries (a warp per row), <= 4096 (a CTA per row, shared memory),
+    // longer rows in place in global memory
+    const int L0 = 64, L1 = 512, L2 = 4096;
+    int *len_d, *counts_d, *lists_d;
+    PE_CUDA(cudaMalloc(&len_d, sizeof(int) * (size_t)n));
+    PE_CUDA(cudaMalloc(&counts_d, sizeof(int) * 4));
+    PE_CUDA(cudaMalloc(&lists_d, sizeof(int) * 4 * (size_t)n));
+    PE_CUDA(cudaMemsetAsync(counts_d, 0, sizeof(int) * 4, st));
+    k_row_len<<<pe_grid_for(n, 256), 256, 0, st>>>(n, C.I, len_d);
+    PE_LAUNCHED(ctx);
+    k_bin_rows<<<pe_grid_for(n, 256), 256, 0, st>>>(n, len_d, L0, L1, L2, counts_d, lists_d);
+    PE_LAUNCHED(ctx);
+    int counts[4];
+    PE_CUDA(cudaMemcpyAsync(counts, counts_d, sizeof(int) * 4, cudaMemcpyDeviceToHost, st));
+    PE_CUDA(cudaStreamSynchronize(st));
+    if (counts[0] > 0)
+    {
+        k_spgemm_refill<32, 64><<<pe_grid_for(counts[0], 8), 256, 12 * 64 * 8, st>>>(
+            counts[0], lists_d, A.I, A.J, A.A, B.I, B.J, B.A, C.I, C.J, C.A);
+        PE_LAUNCHED(ctx);
+    }
+    if (counts[1] > 0)
+    {
+        const int sm = 12 * 512 * 8;
+        PE_CUDA(cudaFuncSetAttribute(k_spgemm_refill<32, 512>, cudaFuncAttributeMaxDynamicSharedMemorySize, sm));
+        k_spgemm_refill<32, 512><<<pe_grid_for(counts[1], 8), 256, sm, st>>>(
+            counts[1], lists_d + (size_t)n, A.I, A.J, A.A, B.I, B.J, B.A, C.I, C.J, C.A);
+        PE_LAUNCHED(ctx);
+    }
+    if (counts[2] > 0)
+    {
+        const int sm = 12 * 4096;
+        PE_CUDA(cudaFuncSetAttribute(k_spgemm_refill<256, 4096>, cudaFuncAttributeMaxDynamicSharedMemorySize, sm));
+        k_spgemm_refill<256, 4096><<<counts[2], 256, sm, st>>>(
+            counts[2], lists_d + 2 * (size_t)n, A.I, A.J, A.A, B.I, B.J, B.A, C.I, C.J, C.A);
+        PE_LAUNCHED(ctx);
+    }
+    if (counts[3] > 0)
+    {
+        k_spgemm_refill<256, 0><<<counts[3], 256, 0, st>>>(
+            counts[3], lists_d + 3 * (size_t)n, A.I, A.J, A.A, B.I, B.J, B.A, C.I, C.J, C.A);
+        PE_LAUNCHED(ctx);
+    }
+    PE_CUDA(cudaStreamSynchronize(st));
+    cudaFree(len_d); cudaFree(counts_d); cudaFree(lists_d);
+    return 0;
+}
+
+extern "C" int pe_spgemm_numeric(pe_ctx *ctx, const pe_mat *A, const pe_mat *B, pe_mat *C)
+{
+    PE_CHECK(ctx && A && B && C, "bad arguments");
+    PE_CHECK(!A->distributed && !B->distributed && !C->distributed && C->offd.nnz == 0,
+             "pe_spgemm_numeric: single-rank matrices only");
+    PE_TRY(pe_devcsr_spgemm_numeric(ctx, A->diag, B->diag, C->diag));
+    pe_mat_values_changed(C);
+    return 0;
+}
+
+// A*P is recomputed with the two-pass product (its pattern is not kept from the build: no extra memory between
+// updates); the outer product R^T (A P) is the numeric pass into Ac's pattern.
+extern "C" int pe_rap_numeric(pe_ctx *ctx, const pe_mat *A, const pe_mat *P, pe_mat *Ac)
+{
+    PE_CHECK(ctx && A && P && Ac, "bad arguments");
+    PE_CHECK(!A->distributed && !P->distributed && !Ac->distributed && Ac->offd.nnz == 0,
+             "pe_rap_numeric: single-rank matrices only");
+    PE_CHECK(A->diag.ncols == P->diag.nrows && Ac->diag.nrows == P->diag.ncols && Ac->diag.ncols == P->diag.ncols,
+             "pe_rap_numeric: size mismatch");
+    DevCSR AP, Pt;
+    PE_TRY(pe_devcsr_spgemm(ctx, A->diag, P->diag, AP));
+    const bool own_pt = !P->T;
+    if (P->T) Pt = P->T->diag;
+    else PE_TRY(pe_devcsr_transpose(ctx, P->diag, Pt));
+    const int rc = pe_devcsr_spgemm_numeric(ctx, Pt, AP, Ac->diag);
+    devcsr_free(AP);
+    if (own_pt) devcsr_free(Pt);
+    PE_TRY(rc);
+    pe_mat_values_changed(Ac);
+    return 0;
+}
+
+// ---------------------------------------------------------------------------
+// mask_i = 1 where hypre_ParCSRMatrixFixZeroRows rewrites row i (l1 norm below DBL_EPSILON, as k_fix_zero_rows);
+// with `changed` set, *changed = 1 where that differs from the mask instead (the mask is only read)
+__global__ void k_zero_rows(int n, const int *__restrict__ dI, const double *__restrict__ dA,
+                            const int *__restrict__ oI, const double *__restrict__ oA, double *mask, int *changed)
+{
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    double l1 = 0.0;
+    for (int k = dI[i]; k < dI[i + 1]; ++k) l1 += fabs(dA[k]);
+    if (oI) for (int k = oI[i]; k < oI[i + 1]; ++k) l1 += fabs(oA[k]);
+    const double z = l1 < 2.2204460492503131e-16 ? 1.0 : 0.0;
+    if (!changed) mask[i] = z;
+    else if (mask[i] != z) *changed = 1;
+}
+extern "C" int pe_mat_zero_rows(pe_ctx *ctx, const pe_mat *A, pe_vec *mask, int32_t *changed)
+{
+    PE_CHECK(ctx && A && mask && mask->n == A->diag.nrows, "pe_mat_zero_rows: mask length differs from the rows of A");
+    const int n = A->diag.nrows;
+    int *flag = reinterpret_cast<int *>(ctx->scalar_d + 4);
+    if (changed) PE_CUDA(cudaMemsetAsync(flag, 0, sizeof(int), ctx->stream));
+    if (n > 0)
+    {
+        k_zero_rows<<<pe_grid_for(n, 256), 256, 0, ctx->stream>>>(n, A->diag.I, A->diag.A, A->offd.nnz > 0 ? A->offd.I : nullptr,
+                                                                  A->offd.A, mask->d, changed ? flag : nullptr);
+        PE_LAUNCHED(ctx);
+    }
+    if (changed)
+    {
+        int h = 0;
+        PE_CUDA(cudaMemcpyAsync(&h, flag, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+        PE_CUDA(cudaStreamSynchronize(ctx->stream));
+        *changed = h;
+    }
+    return 0;
+}
+
+// ---------------------------------------------------------------------------
 __global__ void k_fix_zero_rows(int n, const int *__restrict__ dI, const int *__restrict__ dJ, double *dA,
                                 const int *__restrict__ oI, double *oA, int *nfixed)
 {

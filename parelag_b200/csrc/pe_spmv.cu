@@ -330,6 +330,37 @@ extern "C" int pe_mat_renumbered(pe_ctx *ctx, pe_mat *A, int transpose, const in
     return 0;
 }
 
+__global__ void k_renumber_values(int n, const int *__restrict__ I, const double *__restrict__ A, const int *__restrict__ rpos,
+                                  const int *__restrict__ RI, double *RA)
+{
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    int q = RI[rpos ? rpos[i] : i];
+    for (int k = I[i]; k < I[i + 1]; ++k, ++q) RA[q] = A[k];
+}
+
+extern "C" int pe_mat_renumbered_values(pe_ctx *ctx, pe_mat *A, const int32_t *rpos, pe_mat *R)
+{
+    PE_CHECK(ctx && A && R, "bad arguments");
+    PE_CHECK(!A->distributed && A->offd.nnz == 0 && ctx->nranks == 1, "pe_mat_renumbered_values: single-rank matrices only");
+    DevCSR &src = A->diag;
+    PE_CHECK(R->diag.nnz == src.nnz && R->diag.nrows >= src.nrows && (rpos || R->diag.nrows == src.nrows),
+             "pe_mat_renumbered_values: R is not a renumbered copy of a matrix with A's pattern");
+    PE_TRY(pe_sell_for_spmv(ctx, src));
+    cudaStream_t st = ctx->stream;
+    if (src.nrows > 0)
+    {
+        k_renumber_values<<<pe_grid_for(src.nrows, 256), 256, 0, st>>>(src.nrows, src.I, src.A, rpos, R->diag.I, R->diag.A);
+        PE_LAUNCHED(ctx);
+    }
+    // the SELL copy is rebuilt from the new values (its layout is the pattern's; sign coding depends on the values)
+    pe_mat_values_changed(R);
+    if (src.sell) PE_TRY(pe_sell_for_spmv(ctx, R->diag, true));
+    else R->diag.sell_state = -1;
+    PE_CUDA(cudaStreamSynchronize(st));
+    return 0;
+}
+
 // ---------------------------------------------------------------------------
 __global__ void k_get_diag(int n, const int *__restrict__ I, const int *__restrict__ J,
                            const double *__restrict__ A, double *d)

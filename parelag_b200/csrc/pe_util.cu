@@ -2,6 +2,7 @@
 // delete-zeros, sign transformation, identity / diagonal factories, matrix norms, compare, R^T diag(d) P.
 #include "pe_core.cuh"
 #include <cub/cub.cuh>
+#include <algorithm>
 #include <cmath>
 
 // ---- hypre_CSRMatrixDeleteZeros (hypre, called by hypre_ParCSRMatrixDeleteZeros, deleteZeros.c:16-47): entries with
@@ -256,4 +257,34 @@ extern "C" int pe_rdp(pe_ctx *ctx, const pe_mat *R, const pe_vec *d, const pe_ma
     pe_mat_free(DP);
     if (rc) return rc;
     return pe_mat_wrap_local(ctx, C, out);
+}
+
+// ---- same sparsity pattern: sizes on the host, then row pointers and column indices in one pass whose threads raise
+// a shared flag (every writer stores 1, so the stores need no ordering); one int is downloaded
+__global__ void k_pattern_differs(int64_t n, int nrows, int64_t nnz, const int *__restrict__ AI, const int *__restrict__ AJ,
+                                  const int *__restrict__ BI, const int *__restrict__ BJ, int *flag)
+{
+    const int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= n) return;
+    if ((k < nnz && AJ[k] != BJ[k]) || (k <= nrows && AI[k] != BI[k])) *flag = 1;
+}
+extern "C" int pe_mat_same_pattern(pe_ctx *ctx, const pe_mat *A, const pe_mat *B, int32_t *same)
+{
+    PE_CHECK(ctx && A && B && same, "bad arguments");
+    *same = 0;
+    if (A == B) { *same = 1; return 0; }
+    PE_CHECK(!A->distributed && !B->distributed && A->offd.nnz == 0 && B->offd.nnz == 0,
+             "pe_mat_same_pattern: single-rank matrices only");
+    if (A->diag.nrows != B->diag.nrows || A->diag.ncols != B->diag.ncols || A->diag.nnz != B->diag.nnz) return 0;
+    int *flag = reinterpret_cast<int *>(ctx->scalar_d + 4);
+    PE_CUDA(cudaMemsetAsync(flag, 0, sizeof(int), ctx->stream));
+    const int64_t n = std::max<int64_t>(A->diag.nnz, (int64_t)A->diag.nrows + 1);
+    k_pattern_differs<<<pe_grid_for(n, 256), 256, 0, ctx->stream>>>(n, A->diag.nrows, A->diag.nnz, A->diag.I, A->diag.J,
+                                                                     B->diag.I, B->diag.J, flag);
+    PE_LAUNCHED(ctx);
+    int h = 0;
+    PE_CUDA(cudaMemcpyAsync(&h, flag, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+    PE_CUDA(cudaStreamSynchronize(ctx->stream));
+    *same = h == 0;
+    return 0;
 }

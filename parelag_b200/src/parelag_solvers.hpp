@@ -51,6 +51,44 @@ inline MatHandle RenumberedCopy(const mfem::HypreParMatrix &A, bool transpose, c
     return MatHandle(m, [](pe_mat *p) { pe_mat_free(p); });
 }
 
+/// a copy of A (pattern and values), to take new values in place of A's
+inline std::shared_ptr<mfem::HypreParMatrix> CopyOf(const mfem::HypreParMatrix &A)
+{
+    pe_mat *m = nullptr;
+    PE_CALL(pe_mat_clone(Device::Get(), A.Handle(), &m));
+    return std::make_shared<mfem::HypreParMatrix>(m);
+}
+/// the rows hypre_ParCSRMatrixFixZeroRows rewrites in A: 1.0 on those rows, 0.0 elsewhere
+inline mfem::Vector ZeroRows(const mfem::HypreParMatrix &A)
+{
+    mfem::Vector mask((int)A.Height());
+    PE_CALL(pe_mat_zero_rows(Device::Get(), A.Handle(), mask.Write(), nullptr));
+    return mask;
+}
+/// SetOperator on a built solver: the new operator must have the held one's size and sparsity pattern
+inline void CheckSamePattern(const mfem::HypreParMatrix &held, const mfem::HypreParMatrix &A, const char *who)
+{
+    int32_t same = 0;
+    PE_CALL(pe_mat_same_pattern(Device::Get(), held.Handle(), A.Handle(), &same));
+    PARELAG_TEST_FOR_EXCEPTION(!same, std::runtime_error,
+                               who << "::SetOperator(): the new operator has a different size or sparsity pattern; "
+                               "build a new solver for it");
+}
+/// the FixZeroRows step of an update: A (new values) must have the zero rows recorded at build time, then they are fixed
+inline void FixSameZeroRows(mfem::HypreParMatrix &A, const mfem::Vector &recorded, const std::string &where)
+{
+    int32_t changed = 0;
+    PE_CALL(pe_mat_zero_rows(Device::Get(), A.Handle(), const_cast<pe_vec *>(recorded.Read()), &changed));
+    PARELAG_TEST_FOR_EXCEPTION(changed, std::runtime_error,
+                               "SetOperator(): the set of zero rows FixZeroRows rewrites in " << where
+                               << " differs from the built solver's; build a new solver for this operator");
+    hypre_ParCSRMatrixFixZeroRows(A);
+}
+
+/// SetOperator on a solver and the solvers it holds: the preconditioner of a Krylov solver and the corrector of a
+/// stationary iteration first (their own SetOperator only swaps the operator), as an mfem driver orders it
+void SetNestedOperator(mfem::Operator &S, const Op_Ptr &op);
+
 inline bool SolverCaptureSafe(const mfem::Solver *s)
 {
     auto p = dynamic_cast<const Solver *>(s);
@@ -102,7 +140,14 @@ public:
         PE_CALL(pe_smoother_apply_colour(smoo_, rhs.Read(), mode == 1 ? sol.Write() : sol.ReadWrite(), mode));
     }
 private:
-    void _do_set_operator(const Op_Ptr &) override { PARELAG_NOT_IMPLEMENTED(); }
+    /// the smoother takes op's values (pe_smoother_update); op must have the size and pattern of the held matrix
+    void _do_set_operator(const Op_Ptr &op) override
+    {
+        auto A = std::dynamic_pointer_cast<mfem::HypreParMatrix>(op);
+        PARELAG_TEST_FOR_EXCEPTION(!A, std::runtime_error, "HypreSmootherWrapper::SetOperator(): operator must be a HypreParMatrix");
+        PE_CALL(pe_smoother_update(smoo_, A->Handle()));
+        A_ = std::move(A);
+    }
     std::shared_ptr<mfem::HypreParMatrix> A_;
     pe_smoother *smoo_ = nullptr;
 };
@@ -124,7 +169,7 @@ public:
     void MultTranspose(const mfem::Vector &rhs, mfem::Vector &sol) const override { jacobi_->Mult(rhs, sol); }
     bool CaptureSafe() const override { return true; }
 private:
-    void _do_set_operator(const Op_Ptr &) override { PARELAG_NOT_IMPLEMENTED(); }
+    void _do_set_operator(const Op_Ptr &op) override { jacobi_->SetOperator(op); }
     std::unique_ptr<HypreSmootherWrapper> jacobi_;
 };
 
@@ -198,6 +243,31 @@ public:
         PrimarySolver_->Mult(B, X);
     }
     Op_Ptr GetAuxiliaryOperator() const { return A_aux_; }
+    /// the auxiliary operator was computed as D^T A D and FixZeroRows rewrote zero_rows (ZeroRows): SetOperator
+    /// recomputes it.  Without this call the auxiliary operator came from the state and SetOperator keeps it.
+    void SetComputedAuxiliary(mfem::Vector zero_rows) { aux_zero_rows_ = std::move(zero_rows); aux_computed_ = true; }
+    /// The first half of SetOperator(op): the auxiliary operator for op, computed and checked without changing this
+    /// smoother (throws on a refusal).  CommitOperator(op, PrepareOperator(op)) is SetOperator(op).
+    Op_Ptr PrepareOperator(const Op_Ptr &op) const
+    {
+        auto A = std::dynamic_pointer_cast<mfem::HypreParMatrix>(op);
+        PARELAG_TEST_FOR_EXCEPTION(!A, std::runtime_error, "HiptmairSmoother::SetOperator(): operator must be a HypreParMatrix");
+        if (auto held = std::dynamic_pointer_cast<mfem::HypreParMatrix>(A_)) CheckSamePattern(*held, *A, "HiptmairSmoother");
+        if (!aux_computed_) return A_aux_;
+        auto aux = CopyOf(dynamic_cast<const mfem::HypreParMatrix &>(*A_aux_));
+        PE_CALL(pe_rap_numeric(Device::Get(), A->Handle(), dynamic_cast<const mfem::HypreParMatrix &>(*D_op_).Handle(), aux->Handle()));
+        FixSameZeroRows(*aux, aux_zero_rows_, "the Hiptmair auxiliary operator D^T A D");
+        return aux;
+    }
+    /// the second half: both smoothers and the residual take the new operators (the colour-numbered residual copy is
+    /// the enclosing Hierarchy's and refreshed there)
+    void CommitOperator(const Op_Ptr &op, const Op_Ptr &aux)
+    {
+        SetNestedOperator(*PrimarySolver_, op);
+        if (aux != A_aux_) SetNestedOperator(*AuxiliarySolver_, aux);
+        A_ = op;
+        A_aux_ = aux;
+    }
     bool CaptureSafe() const override
     { return SolverCaptureSafe(PrimarySolver_.get()) && SolverCaptureSafe(AuxiliarySolver_.get()); }
     pe_smoother *PrimaryHandle() const { return dynamic_cast<const HypreSmootherWrapper &>(*PrimarySolver_).Handle(); }
@@ -243,12 +313,14 @@ private:
         D_op_->Mult(AuxX_, PrimaryVec_);
         X += PrimaryVec_;
     }
-    void _do_set_operator(const Op_Ptr &) override { PARELAG_NOT_IMPLEMENTED(); }
+    void _do_set_operator(const Op_Ptr &op) override { CommitOperator(op, PrepareOperator(op)); }
     Op_Ptr A_, A_aux_, D_op_;
     std::shared_ptr<mfem::Solver> PrimarySolver_, AuxiliarySolver_;
     mutable mfem::Vector AuxB_, AuxX_, PrimaryVec_;
     MatHandle cres_, cDt_, cD_;                             // colour-numbered products (SetupColour)
     mutable mfem::Vector cPrimaryVec_, cAuxB_, cAuxX_;
+    bool aux_computed_ = false;                              // SetComputedAuxiliary
+    mfem::Vector aux_zero_rows_;
 };
 
 class HiptmairSmootherFactory : public SolverFactory
@@ -307,17 +379,21 @@ private:
         pri_timer.Stop();
         Timer aux_op_timer = TimeManager::AddTimer("Hiptmair: Build auxiliary operator");
         auto aux_op = my_state->GetOperator("Auxiliary A");
-        if (!aux_op) aux_op = _do_compute_aux_operator(*op, *d_op);
+        const bool computed = !aux_op;
+        mfem::Vector aux_zero_rows;
+        if (computed) aux_op = _do_compute_aux_operator(*op, *d_op, aux_zero_rows);
         aux_op_timer.Stop();
         PARELAG_ASSERT(aux_op);
         Timer aux_timer = TimeManager::AddTimer("Hiptmair: Build auxiliary smoother");
         auto AuxiliarySmoo = std::shared_ptr<mfem::Solver>{AuxiliaryFact_->BuildSolver(aux_op, *aux_state)};
         AuxiliarySmoo->iterative_mode = false;
         aux_timer.Stop();
-        return make_unique<HiptmairSmoother>(op, aux_op, d_op, PrimarySmoo, AuxiliarySmoo);
+        auto H = make_unique<HiptmairSmoother>(op, aux_op, d_op, PrimarySmoo, AuxiliarySmoo);
+        if (computed) H->SetComputedAuxiliary(std::move(aux_zero_rows));
+        return H;
     }
-    /// D^T A D followed by FixZeroRows (HiptmairSmootherFactory.cpp:143-165)
-    Op_Ptr _do_compute_aux_operator(mfem::Operator &A, mfem::Operator &D) const
+    /// D^T A D followed by FixZeroRows (HiptmairSmootherFactory.cpp:143-165); zero_rows: the rows FixZeroRows rewrote
+    Op_Ptr _do_compute_aux_operator(mfem::Operator &A, mfem::Operator &D, mfem::Vector &zero_rows) const
     {
         PARELAG_TEST_FOR_EXCEPTION(A.Width() != D.Height(), std::runtime_error,
                                    "A and D do not have compatible sizes to compute D^T*A*D!\nA = " << A.Height() << "x" << A.Width()
@@ -326,6 +402,7 @@ private:
         auto D_hyp = dynamic_cast<mfem::HypreParMatrix *>(&D);
         PARELAG_TEST_FOR_EXCEPTION(!A_hyp || !D_hyp, std::runtime_error, "Hiptmair: A and D must be HypreParMatrix");
         std::shared_ptr<mfem::HypreParMatrix> ret{mfem::RAP(A_hyp, D_hyp)};
+        zero_rows = ZeroRows(*ret);
         hypre_ParCSRMatrixFixZeroRows(*ret);
         return ret;
     }
@@ -803,6 +880,12 @@ public:
         Levels_.front()->Set<Op_Ptr>("A", A);
     }
     int GetNumLevels() const noexcept { return (int)Levels_.size(); }
+    /// the rows FixZeroRows rewrote in the operator of level l (ZeroRows), checked again by SetOperator
+    void SetZeroRows(int l, mfem::Vector rows)
+    {
+        if ((int)ZeroRows_.size() <= l) ZeroRows_.resize(l + 1);
+        ZeroRows_[l] = std::move(rows);
+    }
     Level &GetLevel(int l) { return *Levels_.at(l); }
     std::vector<std::shared_ptr<Level>>::const_iterator begin() const { return Levels_.begin(); }
     std::vector<std::shared_ptr<Level>>::const_iterator end() const { return Levels_.end(); }
@@ -1089,7 +1172,78 @@ private:
         pe_program_free(program_); program_ = nullptr;
         graph_rhs_ = graph_sol_ = warm_rhs_ = warm_sol_ = nullptr;
     }
-    void _do_set_operator(const Op_Ptr &) override { PARELAG_NOT_IMPLEMENTED(); }
+    /// New values on the same pattern (one rank, single-form hierarchies): the state BuildSolver(op) would produce with
+    /// the same sequence, parameters and boundary labels.  Level 0 adopts op; A_l = P_l^T A_{l-1} P_l is recomputed by
+    /// the numeric product into a copy of the held A_l's pattern, then FixZeroRows; Hiptmair's D^T A D likewise.  Every
+    /// check (rank count, operator type, pattern, the recorded FixZeroRows rows) runs before anything is changed, so a
+    /// refused call leaves the hierarchy as it was.  Then the smoothers, the coarse solver (a Krylov solver's
+    /// preconditioner first) and the colour-numbered residual copies take the new operators, and the recorded cycle is
+    /// dropped: the next two preconditioner calls run directly and record again.
+    void _do_set_operator(const Op_Ptr &op) override
+    {
+        pe_ctx *ctx = Device::Get();
+        PARELAG_TEST_FOR_EXCEPTION(pe_ctx_nranks(ctx) != 1, std::runtime_error,
+                                   "Hierarchy::SetOperator(): more than one rank is not supported; build a new solver");
+        const bool blocked = std::dynamic_pointer_cast<MfemBlockOperator>(op) ||
+                             std::dynamic_pointer_cast<MfemBlockOperator>(Levels_.front()->Get<Op_Ptr>("A"));
+        PARELAG_TEST_FOR_EXCEPTION(blocked, std::runtime_error,
+                                   "Hierarchy::SetOperator(): blocked operators (MfemBlockOperator) are not supported; build a new solver");
+        auto A = std::dynamic_pointer_cast<mfem::HypreParMatrix>(op);
+        auto A0 = std::dynamic_pointer_cast<mfem::HypreParMatrix>(Levels_.front()->Get<Op_Ptr>("A"));
+        PARELAG_TEST_FOR_EXCEPTION(!A || !A0, std::runtime_error, "Hierarchy::SetOperator(): operator must be a HypreParMatrix");
+        CheckSamePattern(*A0, *A, "Hierarchy");
+        const int L = (int)Levels_.size();
+        std::vector<std::shared_ptr<mfem::HypreParMatrix>> newA(L);
+        newA[0] = A;
+        Timer galerkin = TimeManager::AddTimer("SetOperator: Galerkin products");
+        for (int l = 1; l < L; ++l)
+        {
+            auto &P = dynamic_cast<const mfem::HypreParMatrix &>(*Levels_[l]->Get<Op_Ptr>("P"));
+            newA[l] = CopyOf(dynamic_cast<const mfem::HypreParMatrix &>(*Levels_[l]->Get<Op_Ptr>("A")));
+            PE_CALL(pe_rap_numeric(ctx, newA[l - 1]->Handle(), P.Handle(), newA[l]->Handle()));
+            if (l < (int)ZeroRows_.size() && ZeroRows_[l].Size() > 0)
+                FixSameZeroRows(*newA[l], ZeroRows_[l], "the operator of level " + std::to_string(l));
+        }
+        galerkin.Stop();
+        // the auxiliary operator of every Hiptmair smoother, once per object (pre- and post-smoother are often one)
+        Timer aux_timer = TimeManager::AddTimer("SetOperator: Hiptmair auxiliary operators");
+        std::vector<std::pair<HiptmairSmoother *, Op_Ptr>> aux;
+        for (int l = 0; l + 1 < L; ++l)
+            for (const char *key : {"PreSmoother", "PostSmoother"})
+                if (Levels_[l]->IsValidKey(key))
+                    if (auto h = dynamic_cast<HiptmairSmoother *>(Levels_[l]->Get<Op_Ptr>(key).get()))
+                        if (std::none_of(aux.begin(), aux.end(), [h](const std::pair<HiptmairSmoother *, Op_Ptr> &e) { return e.first == h; }))
+                            aux.emplace_back(h, h->PrepareOperator(newA[l]));
+        aux_timer.Stop();
+        // nothing has changed so far; from here on the hierarchy takes the new operators
+        Timer smoothers = TimeManager::AddTimer("SetOperator: smoothers and coarse solver");
+        for (int l = 0; l < L; ++l)
+        {
+            Level &lev = *Levels_[l];
+            lev.Reset<Op_Ptr>("A", Op_Ptr(newA[l]));
+            Op_Ptr done;
+            for (const char *key : {"PreSmoother", "PostSmoother"})
+            {
+                if (!lev.IsValidKey(key)) continue;
+                auto S = lev.Get<Op_Ptr>(key);
+                if (S == done) continue;      // pre- and post-smoother are often one object
+                if (auto h = dynamic_cast<HiptmairSmoother *>(S.get()))
+                    h->CommitOperator(newA[l], std::find_if(aux.begin(), aux.end(),
+                                                            [h](const std::pair<HiptmairSmoother *, Op_Ptr> &e) { return e.first == h; })->second);
+                else SetNestedOperator(*S, newA[l]);
+                done = S;
+            }
+            if (lev.IsValidKey("CoarseSolver")) SetNestedOperator(*lev.Get<Op_Ptr>("CoarseSolver"), newA[l]);
+        }
+        smoothers.Stop();
+        Timer colour = TimeManager::AddTimer("SetOperator: colour-numbered copies");
+        for (int l = 0; l < L; ++l)
+            if (colour_state_ > 0 && l < (int)cres_.size() && cres_[l])
+                PE_CALL(pe_mat_renumbered_values(ctx, newA[l]->Handle(), colour_[l].pos, cres_[l].get()));
+        colour.Stop();
+        DropRecordedCycle();
+    }
+    std::vector<mfem::Vector> ZeroRows_;        // per level: the rows FixZeroRows rewrote at build time (SetZeroRows)
     std::vector<std::shared_ptr<Level>> Levels_;
     mutable std::vector<mfem::Vector> CoarseResids_, CoarseSols_, tmp_resid_, tmp_correct_;
     std::vector<int> CycleMu_;
@@ -1133,7 +1287,11 @@ inline std::unique_ptr<Hierarchy> buildHierarchyFromDeRhamSequence(const Op_Ptr 
         }
         else P = seq->ComputeTrueP(form);
         std::shared_ptr<mfem::HypreParMatrix> Ac{mfem::RAP(A.get(), P.get())};
-        if (have_ess) hypre_ParCSRMatrixFixZeroRows(*Ac);
+        if (have_ess)
+        {
+            H->SetZeroRows(l, ZeroRows(*Ac));
+            hypre_ParCSRMatrixFixZeroRows(*Ac);
+        }
         Coarse.Set<Op_Ptr>("P", P);
         Coarse.Set<Op_Ptr>("A", Ac);
         A = Ac;
@@ -1349,6 +1507,7 @@ public:
     bool GetConverged() const { return Converged_; }
     /// ||r_k||, k = 0, 1, ... (what "Print Iterations" prints)
     const std::vector<double> &GetResidualHistory() const { return History_; }
+    const std::shared_ptr<mfem::Solver> &GetSolver() const { return Solver_; }
 private:
     void _do_set_operator(const Op_Ptr &op) override { A_ = op; }
     Op_Ptr A_;
@@ -1362,6 +1521,19 @@ private:
     mutable double FinalNorm_ = 0.0;
     mutable bool Converged_ = false;
 };
+
+inline void SetNestedOperator(mfem::Operator &S, const Op_Ptr &op)
+{
+    if (auto k = dynamic_cast<KrylovSolver *>(&S)) { if (k->GetPreconditioner()) SetNestedOperator(*k->GetPreconditioner(), op); }
+    else if (auto st = dynamic_cast<StationarySolver *>(&S))
+    {
+        PARELAG_ASSERT(st->GetSolver());
+        SetNestedOperator(*st->GetSolver(), op);
+    }
+    auto p = dynamic_cast<Solver *>(&S);
+    PARELAG_TEST_FOR_EXCEPTION(!p, std::runtime_error, "SetOperator(): the solver is not a parelag::Solver");
+    p->SetOperator(op);
+}
 
 /// ParELAG_StationarySolverFactory.hpp:27-107 (parameters "Solver", "Maximum Iterations" (size_t, default 1),
 /// "Absolute Tolerance", "Relative Tolerance", "Print Iterations")

@@ -468,6 +468,25 @@ extern "C" int pe_api_solver_build_device(const char *xml, const char *name, pe_
     *out = s.release();
     API_CATCH
 }
+/// SetOperator on a built solver (new values, same pattern); ownership of A passes to the solver, and A is released
+/// when the call is refused.  A Krylov solver's preconditioner takes the operator first, then the Krylov solver.
+extern "C" int pe_api_solver_set_operator(pe_solver *s, pe_mat *A)
+{
+    API_TRY
+    PARELAG_TEST_FOR_EXCEPTION(!A, std::runtime_error, "pe_api_solver_set_operator: bad arguments");
+    auto op = std::make_shared<mfem::HypreParMatrix>(A);      // A is released with op when the call is refused
+    PARELAG_TEST_FOR_EXCEPTION(!s, std::runtime_error, "pe_api_solver_set_operator: bad arguments");
+    PARELAG_TEST_FOR_EXCEPTION(std::dynamic_pointer_cast<MfemBlockOperator>(s->A), std::runtime_error,
+                               "pe_api_solver_set_operator: blocked operators (MfemBlockOperator) are not supported; build a new solver");
+    auto held = std::dynamic_pointer_cast<mfem::HypreParMatrix>(s->A);
+    PARELAG_TEST_FOR_EXCEPTION(!held, std::runtime_error, "pe_api_solver_set_operator: the solver's operator is not a HypreParMatrix");
+    PARELAG_TEST_FOR_EXCEPTION(pe_ctx_nranks(Device::Get()) != 1, std::runtime_error,
+                               "pe_api_solver_set_operator: more than one rank is not supported; build a new solver");
+    CheckSamePattern(*held, *op, "pe_api_solver_set_operator");
+    SetNestedOperator(*s->solver, op);
+    s->A = op;
+    API_CATCH
+}
 /// mixed (Darcy) system blocks as in examples/MultigridTestDarcy.cpp: M = mass(H(div)) (weights folded into
 /// the element matrices), B = W D with W = mass(L2), Bt = B^T; the driver solves [[M Bt][B 0]]
 extern "C" int pe_api_sequence_assemble_darcy(pe_sequence *s, int level, pe_mat **M_out, pe_mat **B_out, pe_mat **Bt_out)

@@ -321,13 +321,19 @@ int pe_fix_zero_rows(pe_ctx *ctx, pe_mat *A, int32_t *num_fixed);
 /* Numeric pass only (single rank): C / Ac already hold the pattern of the product (row pointers, ascending columns),
  * e.g. from an earlier pe_spgemm / pe_rap with operands of the same patterns; only their values are overwritten, with
  * the summation order of the two-pass product, so the values are those pe_spgemm / pe_rap compute, bit for bit.
- * pe_rap_numeric recomputes the intermediate A*P with the two-pass product and uses P's cached transpose. */
+ * pe_rap_numeric recomputes the intermediate A*P with the two-pass product and, as pe_rap, uses the cached transpose
+ * of R (of P when R_or_null is NULL).  pe_spgemm_numeric_scaled: C = A diag(d)^-1 B with the values pe_spgemm of A and
+ * a copy of B whose rows were scaled by pe_mat_scale_rows(copy, d, 1) computes (the Schur complement's A10 D^-1 A01). */
 int pe_spgemm_numeric(pe_ctx *ctx, const pe_mat *A, const pe_mat *B, pe_mat *C);
-int pe_rap_numeric(pe_ctx *ctx, const pe_mat *A, const pe_mat *P, pe_mat *Ac);
+int pe_spgemm_numeric_scaled(pe_ctx *ctx, const pe_mat *A, const pe_vec *d, const pe_mat *B, pe_mat *C);
+int pe_rap_numeric(pe_ctx *ctx, const pe_mat *R_or_null, const pe_mat *A, const pe_mat *P, pe_mat *Ac);
 /* The rows pe_fix_zero_rows rewrites (l1 norm below DBL_EPSILON).  changed == NULL: mask (length = rows of A) becomes
  * 1.0 on those rows and 0.0 elsewhere.  Otherwise mask is only read and *changed = 1 when that set differs from it. */
 int pe_mat_zero_rows(pe_ctx *ctx, const pe_mat *A, pe_vec *mask, int32_t *changed);
 int pe_spadd(pe_ctx *ctx, double a, const pe_mat *A, double b, const pe_mat *B, pe_mat **C);
+/* Values only (single rank): C holds the pattern pe_spadd(a, A, b, B) produced for operands of A's and B's patterns
+ * (A's entries in their order, then B's entries not in A); its values become those of pe_spadd, bit for bit. */
+int pe_spadd_numeric(pe_ctx *ctx, double a, const pe_mat *A, double b, const pe_mat *B, pe_mat *C);
 /* mfem::SparseMatrix::EliminateRowCol(rc, DIAG_ONE) for every marked dof (marker_host[n],
  * non-zero = essential): marked rows become unit rows, marked columns are zeroed; entries
  * stay in the pattern (examples/MultigridTest2Form.cpp:457-464). */

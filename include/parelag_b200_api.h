@@ -213,6 +213,9 @@ int pe_api_solver_replay_mode(const pe_solver *s, int *mode);
 int pe_api_solver_level_info(const pe_solver *s, int level, int64_t *nrows, int64_t *nnz, int64_t *nnz_P);
 /* download A (diag block) of a hierarchy level for parity tests; arrays sized from level_info */
 int pe_api_solver_level_matrix(const pe_solver *s, int level, int32_t *I, int32_t *J, double *A);
+/* copy of block (i, j) of a hierarchy level's operator ((0, 0): a single-form level), NULL for a zero block; free
+ * with pe_mat_free */
+int pe_api_solver_level_block(const pe_solver *s, int level, int i, int j, pe_mat **out);
 /* solver->SetOperator(A) (mfem::Solver::SetOperator, ParELAG_Solver.hpp:57-65): new values with the held operator's size
  * and sparsity pattern, e.g. the next time step of M + dt K.  The solver is left as a build on A would leave it (one
  * rank, single-form AMGe hierarchies: numeric-only Galerkin products, smoothers and coarse solver refreshed; the recorded
@@ -221,6 +224,13 @@ int pe_api_solver_level_matrix(const pe_solver *s, int level, int32_t *I, int32_
  * blocked operator, more than one rank.  A refused call leaves the solver as it was.  Krylov solvers: the preconditioner
  * takes A first, then the Krylov solver. */
 int pe_api_solver_set_operator(pe_solver *s, pe_mat *A);
+/* SetOperator on a solver built by pe_api_solver_build_block: blocks[nblocks*nblocks] row-major, NULL = zero block, e.g.
+ * the Darcy system [[M', Bt], [B, NULL]] with a new mobility in M'.  Zero blocks, block sizes and every block's
+ * sparsity pattern must be the held operator's.  The solver is left as a build on the new blocks would leave it (one
+ * rank): blocked AMGe levels by numeric block Galerkin products, Block Jacobi / GS / LDU with their inverses and their
+ * Schur complement made again ("MASS" is kept), the recorded V-cycle dropped.  Ownership of the blocks passes to the
+ * solver; they are released when the call is refused, and a refused call leaves the solver as it was. */
+int pe_api_solver_set_operator_block(pe_solver *s, int nblocks, pe_mat **blocks);
 int pe_api_solver_free(pe_solver *s);
 
 /* TimeManager: seconds accumulated under a timer name; clear all timers */

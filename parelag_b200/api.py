@@ -481,6 +481,26 @@ class BlockSolver(Solver):
                 if b is not None:
                     b.h = None
 
+    def set_blocks(self, blocks):
+        """SetOperator on the built block solver: blocks (nested list of capi.Mat or None) have the held operator's zero
+        blocks, block sizes and sparsity patterns, and new values.  Ownership passes to the solver, also when the call is
+        refused (capi.PEError)."""
+        nb = len(blocks)
+        arr = (C.c_void_p * (nb * nb))()
+        for i in range(nb):
+            for j in range(nb):
+                b = blocks[i][j]
+                arr[i * nb + j] = None if b is None else b.h
+                if b is not None:
+                    b.h = None
+        _chk(lib().pe_api_solver_set_operator_block(self.h, nb, arr))
+
+    def level_block(self, ctx, l, i, j):
+        """copy of block (i, j) of level l's operator as a capi.Mat, None for a zero block"""
+        out = capi.Mat(ctx)
+        _chk(lib().pe_api_solver_level_block(self.h, l, i, j, C.byref(out.h)))
+        return out if out.h else None
+
 
 def timer(name):
     s = C.c_double()

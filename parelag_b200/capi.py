@@ -393,9 +393,19 @@ def spgemm_numeric(ctx, A, B, Cm):
     _chk(lib().pe_spgemm_numeric(ctx.h, A.h, B.h, Cm.h))
 
 
-def rap_numeric(ctx, A, P, Ac):
-    """pe_rap_numeric: Ac (pattern of P^T A P) takes the values of P^T A P"""
-    _chk(lib().pe_rap_numeric(ctx.h, A.h, P.h, Ac.h))
+def rap_numeric(ctx, A, P, Ac, R=None):
+    """pe_rap_numeric: Ac (pattern of R^T A P, R = P when None) takes the values of R^T A P"""
+    _chk(lib().pe_rap_numeric(ctx.h, None if R is None else R.h, A.h, P.h, Ac.h))
+
+
+def spgemm_numeric_scaled(ctx, A, d, B, Cm):
+    """pe_spgemm_numeric_scaled: Cm (pattern of A*B) takes the values of A diag(d)^-1 B (d: Vec, one entry per row of B)"""
+    _chk(lib().pe_spgemm_numeric_scaled(ctx.h, A.h, d.h, B.h, Cm.h))
+
+
+def spadd_numeric(ctx, a, A, b, B, Cm):
+    """pe_spadd_numeric: Cm (pattern of spadd(a, A, b, B)) takes the values of a A + b B"""
+    _chk(lib().pe_spadd_numeric(ctx.h, C.c_double(a), A.h, C.c_double(b), B.h, Cm.h))
 
 
 def spadd(ctx, a, A, b, B):

@@ -369,18 +369,20 @@ extern "C" int pe_rap(pe_ctx *ctx, const pe_mat *R, const pe_mat *A, const pe_ma
 // distinct), so every entry of C is summed in the order of k_spgemm_smem / k_spgemm_gmem, starting from 0.0, and the
 // values are theirs bit for bit.  The product and the add are rounded separately, as the atomicAdd of those kernels.
 // CAP > 0: the row is staged in shared memory (CAP slots per group); CAP == 0: one CTA per row, in place in C.
+// SCALE: B's row k is read multiplied by s_k = 1.0 / d[k] (C = A diag(d)^-1 B), each b_kj * s_k rounded once, as
+// k_scale_rows rounds it on a scaled copy of B before the two-pass product.
 __global__ void k_row_len(int n, const int *__restrict__ I, int *len)
 {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n) len[i] = I[i + 1] - I[i];
 }
 
-template <int GT, int CAP>
+template <int GT, int CAP, bool SCALE>
 __global__ void __launch_bounds__(256)
 k_spgemm_refill(int nlist, const int *__restrict__ list,
                 const int *__restrict__ AI, const int *__restrict__ AJ, const double *__restrict__ AA,
                 const int *__restrict__ BI, const int *__restrict__ BJ, const double *__restrict__ BA,
-                const int *__restrict__ CI, const int *__restrict__ CJ, double *CA)
+                const double *__restrict__ d, const int *__restrict__ CI, const int *__restrict__ CJ, double *CA)
 {
     extern __shared__ unsigned char smem_raw[];
     constexpr int GROUPS = 256 / GT;
@@ -411,12 +413,14 @@ k_spgemm_refill(int nlist, const int *__restrict__ list,
         {
             const int k = AJ[ka];
             const double a = AA[ka];
+            const double sk = SCALE ? __ddiv_rn(1.0, d[k]) : 1.0;
             for (int kb = BI[k] + tid; kb < BI[k + 1]; kb += GT)
             {
                 const int col = BJ[kb];
                 int lo = 0, hi = m;
                 while (lo < hi) { const int mid = (lo + hi) >> 1; if (keys[mid] < col) lo = mid + 1; else hi = mid; }
-                if (lo < m && keys[lo] == col) vals[lo] = __dadd_rn(vals[lo], __dmul_rn(a, BA[kb]));
+                const double b = SCALE ? __dmul_rn(BA[kb], sk) : BA[kb];
+                if (lo < m && keys[lo] == col) vals[lo] = __dadd_rn(vals[lo], __dmul_rn(a, b));
             }
             if (GT == 32) __syncwarp(); else __syncthreads();
         }
@@ -424,7 +428,44 @@ k_spgemm_refill(int nlist, const int *__restrict__ list,
     if (CAP > 0) for (int t = tid; t < m; t += GT) CA[c0 + t] = vals[t];
 }
 
-int pe_devcsr_spgemm_numeric(pe_ctx *ctx, const DevCSR &A, const DevCSR &B, DevCSR &C)
+template <bool SCALE>
+static int refill_bins(pe_ctx *ctx, const int *counts, const int *lists_d, int n, const DevCSR &A, const DevCSR &B,
+                       const double *d, DevCSR &C)
+{
+    cudaStream_t st = ctx->stream;
+    if (counts[0] > 0)
+    {
+        k_spgemm_refill<32, 64, SCALE><<<pe_grid_for(counts[0], 8), 256, 12 * 64 * 8, st>>>(
+            counts[0], lists_d, A.I, A.J, A.A, B.I, B.J, B.A, d, C.I, C.J, C.A);
+        PE_LAUNCHED(ctx);
+    }
+    if (counts[1] > 0)
+    {
+        const int sm = 12 * 512 * 8;
+        PE_CUDA(cudaFuncSetAttribute(k_spgemm_refill<32, 512, SCALE>, cudaFuncAttributeMaxDynamicSharedMemorySize, sm));
+        k_spgemm_refill<32, 512, SCALE><<<pe_grid_for(counts[1], 8), 256, sm, st>>>(
+            counts[1], lists_d + (size_t)n, A.I, A.J, A.A, B.I, B.J, B.A, d, C.I, C.J, C.A);
+        PE_LAUNCHED(ctx);
+    }
+    if (counts[2] > 0)
+    {
+        const int sm = 12 * 4096;
+        PE_CUDA(cudaFuncSetAttribute(k_spgemm_refill<256, 4096, SCALE>, cudaFuncAttributeMaxDynamicSharedMemorySize, sm));
+        k_spgemm_refill<256, 4096, SCALE><<<counts[2], 256, sm, st>>>(
+            counts[2], lists_d + 2 * (size_t)n, A.I, A.J, A.A, B.I, B.J, B.A, d, C.I, C.J, C.A);
+        PE_LAUNCHED(ctx);
+    }
+    if (counts[3] > 0)
+    {
+        k_spgemm_refill<256, 0, SCALE><<<counts[3], 256, 0, st>>>(
+            counts[3], lists_d + 3 * (size_t)n, A.I, A.J, A.A, B.I, B.J, B.A, d, C.I, C.J, C.A);
+        PE_LAUNCHED(ctx);
+    }
+    return 0;
+}
+
+/// C (held pattern) = A B, or A diag(d)^-1 B when d is given (d: device array of B's row count)
+int pe_devcsr_spgemm_numeric(pe_ctx *ctx, const DevCSR &A, const DevCSR &B, DevCSR &C, const double *d = nullptr)
 {
     PE_CHECK(A.ncols == B.nrows && C.nrows == A.nrows && C.ncols == B.ncols, "spgemm_numeric: size mismatch");
     const int n = A.nrows;
@@ -445,37 +486,10 @@ int pe_devcsr_spgemm_numeric(pe_ctx *ctx, const DevCSR &A, const DevCSR &B, DevC
     int counts[4];
     PE_CUDA(cudaMemcpyAsync(counts, counts_d, sizeof(int) * 4, cudaMemcpyDeviceToHost, st));
     PE_CUDA(cudaStreamSynchronize(st));
-    if (counts[0] > 0)
-    {
-        k_spgemm_refill<32, 64><<<pe_grid_for(counts[0], 8), 256, 12 * 64 * 8, st>>>(
-            counts[0], lists_d, A.I, A.J, A.A, B.I, B.J, B.A, C.I, C.J, C.A);
-        PE_LAUNCHED(ctx);
-    }
-    if (counts[1] > 0)
-    {
-        const int sm = 12 * 512 * 8;
-        PE_CUDA(cudaFuncSetAttribute(k_spgemm_refill<32, 512>, cudaFuncAttributeMaxDynamicSharedMemorySize, sm));
-        k_spgemm_refill<32, 512><<<pe_grid_for(counts[1], 8), 256, sm, st>>>(
-            counts[1], lists_d + (size_t)n, A.I, A.J, A.A, B.I, B.J, B.A, C.I, C.J, C.A);
-        PE_LAUNCHED(ctx);
-    }
-    if (counts[2] > 0)
-    {
-        const int sm = 12 * 4096;
-        PE_CUDA(cudaFuncSetAttribute(k_spgemm_refill<256, 4096>, cudaFuncAttributeMaxDynamicSharedMemorySize, sm));
-        k_spgemm_refill<256, 4096><<<counts[2], 256, sm, st>>>(
-            counts[2], lists_d + 2 * (size_t)n, A.I, A.J, A.A, B.I, B.J, B.A, C.I, C.J, C.A);
-        PE_LAUNCHED(ctx);
-    }
-    if (counts[3] > 0)
-    {
-        k_spgemm_refill<256, 0><<<counts[3], 256, 0, st>>>(
-            counts[3], lists_d + 3 * (size_t)n, A.I, A.J, A.A, B.I, B.J, B.A, C.I, C.J, C.A);
-        PE_LAUNCHED(ctx);
-    }
+    const int rc = d ? refill_bins<true>(ctx, counts, lists_d, n, A, B, d, C) : refill_bins<false>(ctx, counts, lists_d, n, A, B, d, C);
     PE_CUDA(cudaStreamSynchronize(st));
     cudaFree(len_d); cudaFree(counts_d); cudaFree(lists_d);
-    return 0;
+    return rc;
 }
 
 extern "C" int pe_spgemm_numeric(pe_ctx *ctx, const pe_mat *A, const pe_mat *B, pe_mat *C)
@@ -488,23 +502,41 @@ extern "C" int pe_spgemm_numeric(pe_ctx *ctx, const pe_mat *A, const pe_mat *B, 
     return 0;
 }
 
+// C = A diag(d)^-1 B into C's pattern: the Schur complement's A10 D^-1 A01 without the build's scaled copy of A01.
+// That copy (pe_spadd(1, A01, 0, A01), then k_scale_rows) holds 1*b + 0*b = b for every finite entry b, -0.0
+// included (-0.0 + -0.0 = -0.0); and a signed zero product cannot change a sum that starts from +0.0.  The scale
+// 1.0 / d[k] and the products are rounded as k_scale_rows and the two-pass product round them, so the values are the
+// build's bit for bit.
+extern "C" int pe_spgemm_numeric_scaled(pe_ctx *ctx, const pe_mat *A, const pe_vec *d, const pe_mat *B, pe_mat *C)
+{
+    PE_CHECK(ctx && A && d && B && C, "bad arguments");
+    PE_CHECK(!A->distributed && !B->distributed && !C->distributed && C->offd.nnz == 0,
+             "pe_spgemm_numeric_scaled: single-rank matrices only");
+    PE_CHECK(d->n == B->diag.nrows, "pe_spgemm_numeric_scaled: d must have one entry per row of B");
+    PE_TRY(pe_devcsr_spgemm_numeric(ctx, A->diag, B->diag, C->diag, d->d));
+    pe_mat_values_changed(C);
+    return 0;
+}
+
 // A*P is recomputed with the two-pass product (its pattern is not kept from the build: no extra memory between
-// updates); the outer product R^T (A P) is the numeric pass into Ac's pattern.
-extern "C" int pe_rap_numeric(pe_ctx *ctx, const pe_mat *A, const pe_mat *P, pe_mat *Ac)
+// updates); the outer product R^T (A P) is the numeric pass into Ac's pattern, with R's cached transpose when it has
+// one (R = P when R is null), as pe_rap.
+extern "C" int pe_rap_numeric(pe_ctx *ctx, const pe_mat *R, const pe_mat *A, const pe_mat *P, pe_mat *Ac)
 {
     PE_CHECK(ctx && A && P && Ac, "bad arguments");
-    PE_CHECK(!A->distributed && !P->distributed && !Ac->distributed && Ac->offd.nnz == 0,
+    const pe_mat *Rm = R ? R : P;
+    PE_CHECK(!A->distributed && !P->distributed && !Rm->distributed && !Ac->distributed && Ac->offd.nnz == 0,
              "pe_rap_numeric: single-rank matrices only");
-    PE_CHECK(A->diag.ncols == P->diag.nrows && Ac->diag.nrows == P->diag.ncols && Ac->diag.ncols == P->diag.ncols,
-             "pe_rap_numeric: size mismatch");
-    DevCSR AP, Pt;
+    PE_CHECK(Rm->diag.nrows == A->diag.nrows && A->diag.ncols == P->diag.nrows && Ac->diag.nrows == Rm->diag.ncols &&
+             Ac->diag.ncols == P->diag.ncols, "pe_rap_numeric: size mismatch");
+    DevCSR AP, Rt;
     PE_TRY(pe_devcsr_spgemm(ctx, A->diag, P->diag, AP));
-    const bool own_pt = !P->T;
-    if (P->T) Pt = P->T->diag;
-    else PE_TRY(pe_devcsr_transpose(ctx, P->diag, Pt));
-    const int rc = pe_devcsr_spgemm_numeric(ctx, Pt, AP, Ac->diag);
+    const bool own_rt = !Rm->T;
+    if (Rm->T) Rt = Rm->T->diag;
+    else PE_TRY(pe_devcsr_transpose(ctx, Rm->diag, Rt));
+    const int rc = pe_devcsr_spgemm_numeric(ctx, Rt, AP, Ac->diag);
     devcsr_free(AP);
-    if (own_pt) devcsr_free(Pt);
+    if (own_rt) devcsr_free(Rt);
     PE_TRY(rc);
     pe_mat_values_changed(Ac);
     return 0;
@@ -595,6 +627,9 @@ __global__ void k_spadd_count(int n, const int *__restrict__ AI, const int *__re
     }
     len[i] = c;
 }
+// PATTERN = false (pe_spadd_numeric): C already holds this pattern; only its values are written, with the same
+// arithmetic, so they are pe_spadd's bit for bit.
+template <bool PATTERN>
 __global__ void k_spadd_fill(int n, double a, const int *__restrict__ AI, const int *__restrict__ AJ, const double *__restrict__ AA,
                              double b, const int *__restrict__ BI, const int *__restrict__ BJ, const double *__restrict__ BA,
                              const int *__restrict__ CI, int *CJ, double *CA)
@@ -603,13 +638,13 @@ __global__ void k_spadd_fill(int n, double a, const int *__restrict__ AI, const 
     if (i >= n) return;
     int p = CI[i];
     const int p0 = p;
-    for (int ka = AI[i]; ka < AI[i + 1]; ++ka, ++p) { CJ[p] = AJ[ka]; CA[p] = a * AA[ka]; }
+    for (int ka = AI[i]; ka < AI[i + 1]; ++ka, ++p) { if (PATTERN) CJ[p] = AJ[ka]; CA[p] = a * AA[ka]; }
     const int na = p - p0;
     for (int kb = BI[i]; kb < BI[i + 1]; ++kb) {
         int hit = -1;
         for (int q = 0; q < na; ++q) if (CJ[p0 + q] == BJ[kb]) { hit = p0 + q; break; }
         if (hit >= 0) CA[hit] += b * BA[kb];
-        else { CJ[p] = BJ[kb]; CA[p] = b * BA[kb]; ++p; }
+        else { if (PATTERN) CJ[p] = BJ[kb]; CA[p] = b * BA[kb]; ++p; }
     }
 }
 int pe_devcsr_spadd(pe_ctx *ctx, double a, const DevCSR &A, double b, const DevCSR &B, DevCSR &C)
@@ -635,7 +670,7 @@ int pe_devcsr_spadd(pe_ctx *ctx, double a, const DevCSR &A, double b, const DevC
     C.nrows = n; C.ncols = A.ncols; C.nnz = nnz;
     PE_CUDA(cudaMalloc(&C.J, sizeof(int) * (size_t)(nnz > 0 ? nnz : 1)));
     PE_CUDA(cudaMalloc(&C.A, sizeof(double) * (size_t)(nnz > 0 ? nnz : 1)));
-    if (n > 0) { k_spadd_fill<<<pe_grid_for(n, 256), 256, 0, st>>>(n, a, A.I, A.J, A.A, b, B.I, B.J, B.A, C.I, C.J, C.A); PE_LAUNCHED(ctx); }
+    if (n > 0) { k_spadd_fill<true><<<pe_grid_for(n, 256), 256, 0, st>>>(n, a, A.I, A.J, A.A, b, B.I, B.J, B.A, C.I, C.J, C.A); PE_LAUNCHED(ctx); }
     return 0;
 }
 extern "C" int pe_spadd(pe_ctx *ctx, double a, const pe_mat *A, double b, const pe_mat *B, pe_mat **Cout)
@@ -649,6 +684,26 @@ extern "C" int pe_spadd(pe_ctx *ctx, double a, const pe_mat *A, double b, const 
     DevCSR C;
     PE_TRY(pe_devcsr_spadd(ctx, a, A->diag, b, B->diag, C));
     PE_TRY(pe_mat_wrap_local(ctx, C, Cout));
+    return 0;
+}
+
+extern "C" int pe_spadd_numeric(pe_ctx *ctx, double a, const pe_mat *A, double b, const pe_mat *B, pe_mat *C)
+{
+    PE_CHECK(ctx && A && B && C, "bad arguments");
+    PE_CHECK(!A->distributed && !B->distributed && !C->distributed && A->offd.nnz == 0 && B->offd.nnz == 0 && C->offd.nnz == 0,
+             "pe_spadd_numeric: single-rank matrices only");
+    PE_CHECK(A->diag.nrows == B->diag.nrows && A->diag.ncols == B->diag.ncols && C->diag.nrows == A->diag.nrows &&
+             C->diag.ncols == A->diag.ncols, "pe_spadd_numeric: size mismatch");
+    PE_CHECK(C->diag.nnz >= A->diag.nnz && C->diag.nnz <= A->diag.nnz + B->diag.nnz,
+             "pe_spadd_numeric: C does not hold the pattern of a A + b B");
+    const int n = A->diag.nrows;
+    if (n > 0)
+    {
+        k_spadd_fill<false><<<pe_grid_for(n, 256), 256, 0, ctx->stream>>>(n, a, A->diag.I, A->diag.J, A->diag.A, b, B->diag.I,
+                                                                           B->diag.J, B->diag.A, C->diag.I, C->diag.J, C->diag.A);
+        PE_LAUNCHED(ctx);
+    }
+    pe_mat_values_changed(C);
     return 0;
 }
 

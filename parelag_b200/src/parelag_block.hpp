@@ -8,6 +8,7 @@
 //   Block2x2{Jacobi,GaussSeidel,LDU}SolverFactory   src/linalg/factories/ParELAG_Block2x2*SolverFactory.cpp
 #pragma once
 #include <algorithm>
+#include <tuple>
 #include "parelag_core.hpp"
 #include "parelag_sequence.hpp"
 
@@ -131,6 +132,109 @@ inline void ComputeResidualGeneric(const mfem::Operator &A, const mfem::Vector &
 }
 } // namespace mg_utils
 
+/// a copy of A (pattern and values), to take new values in place of A's
+inline std::shared_ptr<mfem::HypreParMatrix> CopyOf(const mfem::HypreParMatrix &A)
+{
+    pe_mat *m = nullptr;
+    PE_CALL(pe_mat_clone(Device::Get(), A.Handle(), &m));
+    return std::make_shared<mfem::HypreParMatrix>(m);
+}
+/// the rows hypre_ParCSRMatrixFixZeroRows rewrites in A: 1.0 on those rows, 0.0 elsewhere
+inline mfem::Vector ZeroRows(const mfem::HypreParMatrix &A)
+{
+    mfem::Vector mask((int)A.Height());
+    PE_CALL(pe_mat_zero_rows(Device::Get(), A.Handle(), mask.Write(), nullptr));
+    return mask;
+}
+/// SetOperator on a built solver: the new operator must have the held one's size and sparsity pattern
+inline void CheckSamePattern(const mfem::HypreParMatrix &held, const mfem::HypreParMatrix &A, const char *who)
+{
+    int32_t same = 0;
+    PE_CALL(pe_mat_same_pattern(Device::Get(), held.Handle(), A.Handle(), &same));
+    PARELAG_TEST_FOR_EXCEPTION(!same, std::runtime_error,
+                               who << "::SetOperator(): the new operator has a different size or sparsity pattern; "
+                               "build a new solver for it");
+}
+/// the FixZeroRows step of an update: A (new values) must have the zero rows recorded at build time, then they are fixed
+inline void FixSameZeroRows(mfem::HypreParMatrix &A, const mfem::Vector &recorded, const std::string &where)
+{
+    int32_t changed = 0;
+    PE_CALL(pe_mat_zero_rows(Device::Get(), A.Handle(), const_cast<pe_vec *>(recorded.Read()), &changed));
+    PARELAG_TEST_FOR_EXCEPTION(changed, std::runtime_error,
+                               "SetOperator(): the set of zero rows FixZeroRows rewrites in " << where
+                               << " differs from the built solver's; build a new solver for this operator");
+    hypre_ParCSRMatrixFixZeroRows(A);
+}
+
+/// SetOperator on a solver and the solvers it holds: the preconditioner of a Krylov solver and the corrector of a
+/// stationary iteration first (their own SetOperator only swaps the operator), as an mfem driver orders it
+void SetNestedOperator(mfem::Operator &S, const Op_Ptr &op);
+
+/// SetOperator on a block solver: op must be an MfemBlockOperator with the held one's block sizes, zero blocks and
+/// the sparsity pattern of every block (one rank)
+inline std::shared_ptr<MfemBlockOperator> SameBlockStructure(const MfemBlockOperator &held, const Op_Ptr &op, const char *who)
+{
+    PARELAG_TEST_FOR_EXCEPTION(pe_ctx_nranks(Device::Get()) != 1, std::runtime_error,
+                               who << "::SetOperator(): more than one rank is not supported; build a new solver");
+    auto A = std::dynamic_pointer_cast<MfemBlockOperator>(op);
+    PARELAG_TEST_FOR_EXCEPTION(!A, std::runtime_error, who << "::SetOperator(...): Operator must be an MfemBlockOperator!");
+    PARELAG_TEST_FOR_EXCEPTION(A->ViewRowOffsets() != held.ViewRowOffsets() || A->ViewColumnOffsets() != held.ViewColumnOffsets(),
+                               std::runtime_error, who << "::SetOperator(): the new operator has different block sizes; build a new solver for it");
+    for (size_t i = 0; i < held.GetNumBlockRows(); ++i)
+        for (size_t j = 0; j < held.GetNumBlockCols(); ++j)
+        {
+            PARELAG_TEST_FOR_EXCEPTION(A->IsZeroBlock(i, j) != held.IsZeroBlock(i, j), std::runtime_error,
+                                       who << "::SetOperator(): block (" << i << "," << j << ") is " << (held.IsZeroBlock(i, j) ? "" : "not ")
+                                       << "zero in the built solver's operator and " << (A->IsZeroBlock(i, j) ? "" : "not ")
+                                       << "zero in the new one; build a new solver for it");
+            if (held.IsZeroBlock(i, j)) continue;
+            auto h = dynamic_cast<const mfem::HypreParMatrix *>(&held.GetBlock(i, j));
+            auto a = dynamic_cast<const mfem::HypreParMatrix *>(&A->GetBlock(i, j));
+            PARELAG_TEST_FOR_EXCEPTION(!h || !a, std::runtime_error, who << "::SetOperator(): the blocks must be HypreParMatrix");
+            CheckSamePattern(*h, *a, who);
+        }
+    return A;
+}
+
+/// one inverse of a block preconditioner, the operator it takes and the one it holds
+struct InverseUpdate
+{
+    mfem::Solver *inv;
+    Op_Ptr next, held;
+};
+/// every inverse takes its new operator, each object once; when one refuses, those already updated take their held
+/// operators back (SetOperator with the held operators restores a solver bit for bit) and the refusal is passed on
+inline void SetInverseOperators(const std::vector<InverseUpdate> &u)
+{
+    auto first = [&](size_t i) { for (size_t k = 0; k < i; ++k) if (u[k].inv == u[i].inv) return false; return true; };
+    size_t i = 0;
+    try
+    {
+        for (; i < u.size(); ++i)
+            if (u[i].next != u[i].held && first(i)) SetNestedOperator(*u[i].inv, u[i].next);
+    }
+    catch (...)
+    {
+        for (size_t k = 0; k < i; ++k)
+            if (u[k].next != u[k].held && first(k)) SetNestedOperator(*u[k].inv, u[k].held);
+        throw;
+    }
+}
+
+class SchurComplementFactory;
+/// How a block preconditioner's second diagonal operator was made (BlockSolverFactory::SecondDiagonalOperator), so
+/// that SetOperator can make it again for new blocks
+struct SecondDiagonal
+{
+    std::shared_ptr<const SchurComplementFactory> fact;   // "S Type", "Alpha"; null: the (1,1) block itself
+    bool negative = true;                                 // "Use Negative S"
+    Op_Ptr S;                                             // the operator the A11 / S inverse was built on
+    std::shared_ptr<mfem::HypreParMatrix> product;        // A10 D^-1 A01 when S = A11 - alpha A10 D^-1 A01
+    /// the second diagonal operator of the new blocks A (same patterns as the held ones): S computed numerically
+    /// into copies of the held patterns, the held S for "MASS", A's (1,1) block without a factory
+    SecondDiagonal For(MfemBlockOperator &A) const;
+};
+
 inline bool BlockCaptureSafe(const std::vector<std::shared_ptr<mfem::Solver>> &ops)
 {
     for (auto &s : ops)
@@ -141,13 +245,29 @@ inline bool BlockCaptureSafe(const std::vector<std::shared_ptr<mfem::Solver>> &o
     return true;
 }
 
+/// SetOperator of BlockDiagonalSolver and BlockTriangularSolver: inverse b takes block (b, b) of op, inverse 1 the
+/// second diagonal operator made again for op
+inline void SetDiagonalInverses(std::shared_ptr<MfemBlockOperator> &A, SecondDiagonal &second,
+                                const std::vector<std::shared_ptr<mfem::Solver>> &inv_ops, const Op_Ptr &op, const char *who)
+{
+    auto next = SameBlockStructure(*A, op, who);
+    SecondDiagonal next_second = second.For(*next);
+    std::vector<InverseUpdate> u;
+    for (size_t b = 0; b < inv_ops.size(); ++b)
+        u.push_back({inv_ops[b].get(), b == 1 ? next_second.S : next->GetBlockPtr(b, b), b == 1 ? second.S : A->GetBlockPtr(b, b)});
+    Timer t = TimeManager::AddTimer("SetOperator: block inverses");
+    SetInverseOperators(u);
+    A = std::move(next);
+    second = std::move(next_second);
+}
+
 // ------------------------------------------------------------------ block Jacobi
 class BlockDiagonalSolver : public Solver
 {
 public:
-    BlockDiagonalSolver(std::shared_ptr<MfemBlockOperator> op, std::vector<std::shared_ptr<mfem::Solver>> inv_ops,
-                        std::vector<std::shared_ptr<mfem::Operator>> aux_ops = {})
-        : Solver(op->Width(), op->Height(), false), A_(std::move(op)), inv_ops_(std::move(inv_ops)), aux_ops_(std::move(aux_ops)) {}
+    /// second: how the operator of inv_ops[1] was made (its S keeps the Schur complement alive)
+    BlockDiagonalSolver(std::shared_ptr<MfemBlockOperator> op, std::vector<std::shared_ptr<mfem::Solver>> inv_ops, SecondDiagonal second)
+        : Solver(op->Width(), op->Height(), false), A_(std::move(op)), inv_ops_(std::move(inv_ops)), second_(std::move(second)) {}
     void Mult(const mfem::Vector &rhs, mfem::Vector &sol) const override { Apply(rhs, sol, false); }
     void MultTranspose(const mfem::Vector &rhs, mfem::Vector &sol) const override { Apply(rhs, sol, true); }
     bool CaptureSafe() const override { return BlockCaptureSafe(inv_ops_); }
@@ -178,14 +298,11 @@ private:
         PARELAG_ASSERT(!inv_ops_[b]->iterative_mode);
         if (transpose) inv_ops_[b]->MultTranspose(r, x); else inv_ops_[b]->Mult(r, x);
     }
-    void _do_set_operator(const Op_Ptr &op) override
-    {
-        A_ = std::dynamic_pointer_cast<MfemBlockOperator>(op);
-        PARELAG_TEST_FOR_EXCEPTION(!A_, std::runtime_error, "BlockDiagonalSolver::SetOperator(...): Operator must be an MfemBlockOperator!");
-    }
+    /// new block values on the held structure and patterns: the inverses take the new diagonal operators
+    void _do_set_operator(const Op_Ptr &op) override { SetDiagonalInverses(A_, second_, inv_ops_, op, "BlockDiagonalSolver"); }
     std::shared_ptr<MfemBlockOperator> A_;
     std::vector<std::shared_ptr<mfem::Solver>> inv_ops_;
-    std::vector<std::shared_ptr<mfem::Operator>> aux_ops_;    // keeps the Schur complement alive
+    SecondDiagonal second_;
     mutable mfem::Vector resid_, corr_;
 };
 
@@ -195,8 +312,8 @@ class BlockTriangularSolver : public Solver
 public:
     enum class Triangle { UPPER_TRIANGLE, LOWER_TRIANGLE };
     BlockTriangularSolver(std::shared_ptr<MfemBlockOperator> op, std::vector<std::shared_ptr<mfem::Solver>> inv_ops,
-                          std::vector<std::shared_ptr<mfem::Operator>> aux_ops, Triangle tri = Triangle::LOWER_TRIANGLE)
-        : Solver(op->Width(), op->Height(), false), A_(std::move(op)), inv_ops_(std::move(inv_ops)), aux_ops_(std::move(aux_ops)), tri_(tri) {}
+                          SecondDiagonal second, Triangle tri = Triangle::LOWER_TRIANGLE)
+        : Solver(op->Width(), op->Height(), false), A_(std::move(op)), inv_ops_(std::move(inv_ops)), second_(std::move(second)), tri_(tri) {}
     void Mult(const mfem::Vector &rhs, mfem::Vector &sol) const override { Apply(rhs, sol, false); }
     void MultTranspose(const mfem::Vector &rhs, mfem::Vector &sol) const override { Apply(rhs, sol, true); }
     bool CaptureSafe() const override { return BlockCaptureSafe(inv_ops_); }
@@ -243,14 +360,10 @@ private:
             if (transpose) inv_ops_[i]->MultTranspose(r, sol.GetBlock(i)); else inv_ops_[i]->Mult(r, sol.GetBlock(i));
         }
     }
-    void _do_set_operator(const Op_Ptr &op) override
-    {
-        A_ = std::dynamic_pointer_cast<MfemBlockOperator>(op);
-        PARELAG_TEST_FOR_EXCEPTION(!A_, std::runtime_error, "BlockTriangularSolver::SetOperator(...): Operator must be an MfemBlockOperator!");
-    }
+    void _do_set_operator(const Op_Ptr &op) override { SetDiagonalInverses(A_, second_, inv_ops_, op, "BlockTriangularSolver"); }
     std::shared_ptr<MfemBlockOperator> A_;
     std::vector<std::shared_ptr<mfem::Solver>> inv_ops_;
-    std::vector<std::shared_ptr<mfem::Operator>> aux_ops_;
+    SecondDiagonal second_;
     Triangle tri_;
     mutable mfem::Vector resid_, corr_, tmp_rhs_, tmp_;
 };
@@ -260,7 +373,7 @@ class Block2x2LDUInverseOperator : public Solver
 {
 public:
     Block2x2LDUInverseOperator(std::shared_ptr<MfemBlockOperator> A, std::shared_ptr<mfem::Solver> invA00_1, std::shared_ptr<mfem::Solver> invA00_2,
-                               std::shared_ptr<mfem::Solver> invA00_3, std::shared_ptr<mfem::Solver> invS, Op_Ptr S, double DampingFactor)
+                               std::shared_ptr<mfem::Solver> invA00_3, std::shared_ptr<mfem::Solver> invS, SecondDiagonal S, double DampingFactor)
         : Solver(A->Width(), A->Height(), false), A_(std::move(A)), invA00_1_(std::move(invA00_1)), invA00_2_(std::move(invA00_2)),
           invA00_3_(std::move(invA00_3)), invS_(std::move(invS)), S_(std::move(S)), DampingFactor_(DampingFactor) {}
     void Mult(const mfem::Vector &rhs, mfem::Vector &sol) const override
@@ -290,14 +403,22 @@ public:
     }
     void MultTranspose(const mfem::Vector &, mfem::Vector &) const override { PARELAG_NOT_IMPLEMENTED(); }
 private:
+    /// new block values on the held structure and patterns: the three A00 inverses take the new (0,0) block, the S
+    /// inverse the second diagonal operator made again for op
     void _do_set_operator(const Op_Ptr &op) override
     {
-        A_ = std::dynamic_pointer_cast<MfemBlockOperator>(op);
-        PARELAG_TEST_FOR_EXCEPTION(!A_, std::runtime_error, "Block2x2LDUInverseOperator::SetOperator(...): Operator must be an MfemBlockOperator!");
+        auto A = SameBlockStructure(*A_, op, "Block2x2LDUInverseOperator");
+        SecondDiagonal S = S_.For(*A);
+        const Op_Ptr A00 = A->GetBlockPtr(0, 0), held00 = A_->GetBlockPtr(0, 0);
+        Timer t = TimeManager::AddTimer("SetOperator: block inverses");
+        SetInverseOperators({{invA00_1_.get(), A00, held00}, {invA00_2_.get(), A00, held00}, {invA00_3_.get(), A00, held00},
+                             {invS_.get(), S.S, S_.S}});
+        A_ = std::move(A);
+        S_ = std::move(S);
     }
     std::shared_ptr<MfemBlockOperator> A_;
     std::shared_ptr<mfem::Solver> invA00_1_, invA00_2_, invA00_3_, invS_;
-    Op_Ptr S_;
+    SecondDiagonal S_;
     double DampingFactor_;
     mutable mfem::Vector Residual_, Tmp_, Correction_;
 };
@@ -312,7 +433,9 @@ public:
     }
     /// "MASS": sequence.ComputeTrueM(forms.front()); "DIAGONAL": A11 - alpha A10 diag(A00)^{-1} A01; "ABSROWSUM": the
     /// same with absolute row sums (ParELAG_SchurComplementFactory.cpp:36-177)
-    std::unique_ptr<mfem::Operator> BuildOperator(MfemBlockOperator &op, SolverState &state) const
+    /// product (may be null): receives A10 diag^{-1} A01 when A11 is non-zero (the pattern SecondDiagonal::For refills)
+    std::unique_ptr<mfem::Operator> BuildOperator(MfemBlockOperator &op, SolverState &state,
+                                                  std::shared_ptr<mfem::HypreParMatrix> *product_out = nullptr) const
     {
         PARELAG_ASSERT(op.GetNumBlockRows() == 2);
         PARELAG_ASSERT(op.GetNumBlockCols() == 2);
@@ -342,17 +465,53 @@ public:
         if (A11)
         {
             const int rc2 = pe_spadd(ctx, 1.0, A11->Handle(), -1.0 * Alpha_, product, &out);
-            pe_mat_free(product);
+            if (product_out) *product_out = std::make_shared<mfem::HypreParMatrix>(product);
+            else pe_mat_free(product);
             PE_CALL(rc2);
             return make_unique<mfem::HypreParMatrix>(out);
         }
         PE_CALL(pe_mat_scale(product, -1.0 * Alpha_));
         return make_unique<mfem::HypreParMatrix>(product);
     }
+    /// BuildOperator for new blocks of op's patterns, numerically into copies of S (BuildOperator's result, as held,
+    /// negated or not) and of product: the same values, bit for bit.  "MASS" does not depend on the blocks: S is kept.
+    std::pair<Op_Ptr, std::shared_ptr<mfem::HypreParMatrix>> UpdateOperator(MfemBlockOperator &op, const Op_Ptr &S,
+                                                                            const std::shared_ptr<mfem::HypreParMatrix> &product) const
+    {
+        if (Type_ == "MASS") return {S, product};
+        auto blk = [&](int i, int j) { return op.IsZeroBlock(i, j) ? nullptr : dynamic_cast<mfem::HypreParMatrix *>(&op.GetBlock(i, j)); };
+        auto A00 = blk(0, 0), A01 = blk(0, 1), A10 = blk(1, 0), A11 = blk(1, 1);
+        PARELAG_ASSERT(A00 && A01 && A10 && (!A11 || product));
+        pe_ctx *ctx = Device::Get();
+        mfem::Vector diag(A00->Height());
+        if (Type_ == "DIAGONAL") PE_CALL(pe_mat_get_diag(A00->Handle(), diag.Write()));
+        else PE_CALL(pe_mat_abs_row_sums(A00->Handle(), diag.Write()));
+        auto out = CopyOf(dynamic_cast<const mfem::HypreParMatrix &>(*S));
+        if (!A11)
+        {
+            PE_CALL(pe_spgemm_numeric_scaled(ctx, A10->Handle(), diag.Read(), A01->Handle(), out->Handle()));
+            PE_CALL(pe_mat_scale(out->Handle(), -1.0 * Alpha_));
+            return {out, nullptr};
+        }
+        auto prod = CopyOf(*product);
+        PE_CALL(pe_spgemm_numeric_scaled(ctx, A10->Handle(), diag.Read(), A01->Handle(), prod->Handle()));
+        PE_CALL(pe_spadd_numeric(ctx, 1.0, A11->Handle(), -1.0 * Alpha_, prod->Handle(), out->Handle()));
+        return {out, prod};
+    }
 private:
     std::string Type_;
     double Alpha_;
 };
+
+inline SecondDiagonal SecondDiagonal::For(MfemBlockOperator &A) const
+{
+    SecondDiagonal out = *this;
+    if (!fact) { out.S = A.GetBlockPtr(1, 1); return out; }
+    Timer t = TimeManager::AddTimer("SetOperator: Schur complements");
+    std::tie(out.S, out.product) = fact->UpdateOperator(A, S, product);
+    if (negative && out.S != S) PE_CALL(pe_mat_scale(dynamic_cast<mfem::HypreParMatrix &>(*out.S).Handle(), -1.0));
+    return out;
+}
 
 // ------------------------------------------------------------------ factories
 /// BlockSolverFactory: the operator must be an MfemBlockOperator
@@ -366,14 +525,17 @@ protected:
         return _do_build_block_solver(blop, state);
     }
     virtual std::unique_ptr<mfem::Solver> _do_build_block_solver(const std::shared_ptr<MfemBlockOperator> &blop, SolverState &state) const = 0;
-    /// S (negated when "Use Negative S") or A11
-    Op_Ptr SecondDiagonalOperator(MfemBlockOperator &blop, SolverState &state) const
+    /// S (negated when "Use Negative S") or A11, with how it was made
+    SecondDiagonal SecondDiagonalOperator(MfemBlockOperator &blop, SolverState &state) const
     {
-        if (!S_Fact_) return blop.GetBlockPtr(1, 1);
-        Op_Ptr A11 = S_Fact_->BuildOperator(blop, state);
+        SecondDiagonal out;
+        if (!S_Fact_) { out.S = blop.GetBlockPtr(1, 1); return out; }
+        out.fact = S_Fact_;
+        out.negative = UseNegativeS_;
+        out.S = Op_Ptr(S_Fact_->BuildOperator(blop, state, &out.product));
         if (UseNegativeS_)
-            if (auto s_mat = dynamic_cast<mfem::HypreParMatrix *>(A11.get())) PE_CALL(pe_mat_scale(s_mat->Handle(), -1.0));
-        return A11;
+            if (auto s_mat = dynamic_cast<mfem::HypreParMatrix *>(out.S.get())) PE_CALL(pe_mat_scale(s_mat->Handle(), -1.0));
+        return out;
     }
     void InitSchur()
     {
@@ -411,10 +573,10 @@ class Block2x2JacobiSolverFactory : public BlockSolverFactory
         std::vector<std::shared_ptr<mfem::Solver>> inv_ops(2);
         inv_ops[0] = std::shared_ptr<mfem::Solver>{InvA00_Fact_->BuildSolver(blop->GetBlockPtr(0, 0), *A00_state)};
         inv_ops[0]->iterative_mode = false;
-        Op_Ptr A11 = SecondDiagonalOperator(*blop, *A11_state);
-        inv_ops[1] = std::shared_ptr<mfem::Solver>{InvA11_Fact_->BuildSolver(A11, *A11_state)};
+        SecondDiagonal A11 = SecondDiagonalOperator(*blop, *A11_state);
+        inv_ops[1] = std::shared_ptr<mfem::Solver>{InvA11_Fact_->BuildSolver(A11.S, *A11_state)};
         inv_ops[1]->iterative_mode = false;
-        return make_unique<BlockDiagonalSolver>(blop, inv_ops, S_Fact_ ? std::vector<Op_Ptr>{A11} : std::vector<Op_Ptr>{});
+        return make_unique<BlockDiagonalSolver>(blop, inv_ops, std::move(A11));
     }
     void _do_set_default_parameters() override
     {
@@ -446,10 +608,10 @@ class Block2x2GaussSeidelSolverFactory : public BlockSolverFactory
         std::vector<std::shared_ptr<mfem::Solver>> inv_ops(2);
         inv_ops[0] = std::shared_ptr<mfem::Solver>{InvA00_Fact_->BuildSolver(blop->GetBlockPtr(0, 0), *A00_state)};
         inv_ops[0]->iterative_mode = false;
-        Op_Ptr A11 = SecondDiagonalOperator(*blop, *A11_state);
-        inv_ops[1] = std::shared_ptr<mfem::Solver>{InvA11_Fact_->BuildSolver(A11, *A11_state)};
+        SecondDiagonal A11 = SecondDiagonalOperator(*blop, *A11_state);
+        inv_ops[1] = std::shared_ptr<mfem::Solver>{InvA11_Fact_->BuildSolver(A11.S, *A11_state)};
         inv_ops[1]->iterative_mode = false;
-        return make_unique<BlockTriangularSolver>(blop, inv_ops, S_Fact_ ? std::vector<Op_Ptr>{A11} : std::vector<Op_Ptr>{}, tri_);
+        return make_unique<BlockTriangularSolver>(blop, inv_ops, std::move(A11), tri_);
     }
     void _do_set_default_parameters() override
     {
@@ -491,9 +653,9 @@ class Block2x2LDUSolverFactory : public BlockSolverFactory
         auto inv1 = std::shared_ptr<mfem::Solver>{InvA00_1_Fact_->BuildSolver(A00, *s1)};
         auto inv2 = std::shared_ptr<mfem::Solver>{InvA00_2_Fact_->BuildSolver(A00, *s2)};
         auto inv3 = std::shared_ptr<mfem::Solver>{InvA00_3_Fact_->BuildSolver(A00, *s3)};
-        Op_Ptr A11 = SecondDiagonalOperator(*blop, *sS);
-        auto invS = std::shared_ptr<mfem::Solver>{InvS_Fact_->BuildSolver(A11, *sS)};
-        return make_unique<Block2x2LDUInverseOperator>(blop, inv1, inv2, inv3, invS, A11, Damping_Factor_);
+        SecondDiagonal A11 = SecondDiagonalOperator(*blop, *sS);
+        auto invS = std::shared_ptr<mfem::Solver>{InvS_Fact_->BuildSolver(A11.S, *sS)};
+        return make_unique<Block2x2LDUInverseOperator>(blop, inv1, inv2, inv3, invS, std::move(A11), Damping_Factor_);
     }
     void _do_set_default_parameters() override
     {

@@ -51,44 +51,6 @@ inline MatHandle RenumberedCopy(const mfem::HypreParMatrix &A, bool transpose, c
     return MatHandle(m, [](pe_mat *p) { pe_mat_free(p); });
 }
 
-/// a copy of A (pattern and values), to take new values in place of A's
-inline std::shared_ptr<mfem::HypreParMatrix> CopyOf(const mfem::HypreParMatrix &A)
-{
-    pe_mat *m = nullptr;
-    PE_CALL(pe_mat_clone(Device::Get(), A.Handle(), &m));
-    return std::make_shared<mfem::HypreParMatrix>(m);
-}
-/// the rows hypre_ParCSRMatrixFixZeroRows rewrites in A: 1.0 on those rows, 0.0 elsewhere
-inline mfem::Vector ZeroRows(const mfem::HypreParMatrix &A)
-{
-    mfem::Vector mask((int)A.Height());
-    PE_CALL(pe_mat_zero_rows(Device::Get(), A.Handle(), mask.Write(), nullptr));
-    return mask;
-}
-/// SetOperator on a built solver: the new operator must have the held one's size and sparsity pattern
-inline void CheckSamePattern(const mfem::HypreParMatrix &held, const mfem::HypreParMatrix &A, const char *who)
-{
-    int32_t same = 0;
-    PE_CALL(pe_mat_same_pattern(Device::Get(), held.Handle(), A.Handle(), &same));
-    PARELAG_TEST_FOR_EXCEPTION(!same, std::runtime_error,
-                               who << "::SetOperator(): the new operator has a different size or sparsity pattern; "
-                               "build a new solver for it");
-}
-/// the FixZeroRows step of an update: A (new values) must have the zero rows recorded at build time, then they are fixed
-inline void FixSameZeroRows(mfem::HypreParMatrix &A, const mfem::Vector &recorded, const std::string &where)
-{
-    int32_t changed = 0;
-    PE_CALL(pe_mat_zero_rows(Device::Get(), A.Handle(), const_cast<pe_vec *>(recorded.Read()), &changed));
-    PARELAG_TEST_FOR_EXCEPTION(changed, std::runtime_error,
-                               "SetOperator(): the set of zero rows FixZeroRows rewrites in " << where
-                               << " differs from the built solver's; build a new solver for this operator");
-    hypre_ParCSRMatrixFixZeroRows(A);
-}
-
-/// SetOperator on a solver and the solvers it holds: the preconditioner of a Krylov solver and the corrector of a
-/// stationary iteration first (their own SetOperator only swaps the operator), as an mfem driver orders it
-void SetNestedOperator(mfem::Operator &S, const Op_Ptr &op);
-
 inline bool SolverCaptureSafe(const mfem::Solver *s)
 {
     auto p = dynamic_cast<const Solver *>(s);
@@ -255,7 +217,7 @@ public:
         if (auto held = std::dynamic_pointer_cast<mfem::HypreParMatrix>(A_)) CheckSamePattern(*held, *A, "HiptmairSmoother");
         if (!aux_computed_) return A_aux_;
         auto aux = CopyOf(dynamic_cast<const mfem::HypreParMatrix &>(*A_aux_));
-        PE_CALL(pe_rap_numeric(Device::Get(), A->Handle(), dynamic_cast<const mfem::HypreParMatrix &>(*D_op_).Handle(), aux->Handle()));
+        PE_CALL(pe_rap_numeric(Device::Get(), nullptr, A->Handle(), dynamic_cast<const mfem::HypreParMatrix &>(*D_op_).Handle(), aux->Handle()));
         FixSameZeroRows(*aux, aux_zero_rows_, "the Hiptmair auxiliary operator D^T A D");
         return aux;
     }
@@ -880,11 +842,13 @@ public:
         Levels_.front()->Set<Op_Ptr>("A", A);
     }
     int GetNumLevels() const noexcept { return (int)Levels_.size(); }
-    /// the rows FixZeroRows rewrote in the operator of level l (ZeroRows), checked again by SetOperator
-    void SetZeroRows(int l, mfem::Vector rows)
+    /// the rows FixZeroRows rewrote in the operator of level l (ZeroRows), in its diagonal block `block` on a blocked
+    /// hierarchy, checked again by SetOperator
+    void SetZeroRows(int l, mfem::Vector rows, int block = 0)
     {
         if ((int)ZeroRows_.size() <= l) ZeroRows_.resize(l + 1);
-        ZeroRows_[l] = std::move(rows);
+        if ((int)ZeroRows_[l].size() <= block) ZeroRows_[l].resize(block + 1);
+        ZeroRows_[l][block] = std::move(rows);
     }
     Level &GetLevel(int l) { return *Levels_.at(l); }
     std::vector<std::shared_ptr<Level>>::const_iterator begin() const { return Levels_.begin(); }
@@ -1172,38 +1136,78 @@ private:
         pe_program_free(program_); program_ = nullptr;
         graph_rhs_ = graph_sol_ = warm_rhs_ = warm_sol_ = nullptr;
     }
-    /// New values on the same pattern (one rank, single-form hierarchies): the state BuildSolver(op) would produce with
-    /// the same sequence, parameters and boundary labels.  Level 0 adopts op; A_l = P_l^T A_{l-1} P_l is recomputed by
-    /// the numeric product into a copy of the held A_l's pattern, then FixZeroRows; Hiptmair's D^T A D likewise.  Every
-    /// check (rank count, operator type, pattern, the recorded FixZeroRows rows) runs before anything is changed, so a
-    /// refused call leaves the hierarchy as it was.  Then the smoothers, the coarse solver (a Krylov solver's
-    /// preconditioner first) and the colour-numbered residual copies take the new operators, and the recorded cycle is
-    /// dropped: the next two preconditioner calls run directly and record again.
+    /// the FixZeroRows step of level l (block b) of an update, when the build applied it there
+    void FixRecordedZeroRows(mfem::HypreParMatrix &A, int l, int b, const std::string &where) const
+    {
+        if (l < (int)ZeroRows_.size() && b < (int)ZeroRows_[l].size() && ZeroRows_[l][b].Size() > 0)
+            FixSameZeroRows(A, ZeroRows_[l][b], where);
+    }
+    /// single-form levels: A_l = P_l^T A_{l-1} P_l into a copy of the held A_l's pattern, then FixZeroRows
+    std::vector<Op_Ptr> GalerkinProducts(const Op_Ptr &op) const
+    {
+        auto A = std::dynamic_pointer_cast<mfem::HypreParMatrix>(op);
+        auto A0 = std::dynamic_pointer_cast<mfem::HypreParMatrix>(Levels_.front()->Get<Op_Ptr>("A"));
+        PARELAG_TEST_FOR_EXCEPTION(!A || !A0, std::runtime_error, "Hierarchy::SetOperator(): operator must be a HypreParMatrix");
+        CheckSamePattern(*A0, *A, "Hierarchy");
+        std::vector<Op_Ptr> newA(Levels_.size());
+        newA[0] = A;
+        for (size_t l = 1; l < Levels_.size(); ++l)
+        {
+            auto &P = dynamic_cast<const mfem::HypreParMatrix &>(*Levels_[l]->Get<Op_Ptr>("P"));
+            auto Ac = CopyOf(dynamic_cast<const mfem::HypreParMatrix &>(*Levels_[l]->Get<Op_Ptr>("A")));
+            PE_CALL(pe_rap_numeric(Device::Get(), nullptr, dynamic_cast<const mfem::HypreParMatrix &>(*newA[l - 1]).Handle(),
+                                   P.Handle(), Ac->Handle()));
+            FixRecordedZeroRows(*Ac, (int)l, 0, "the operator of level " + std::to_string(l));
+            newA[l] = Ac;
+        }
+        return newA;
+    }
+    /// blocked levels (buildBlockedHierarchyFromDeRhamSequence): block (i,j) of A_l = P_i^T A_{l-1}(i,j) P_j into a copy
+    /// of the held block's pattern, then FixZeroRows on the diagonal blocks where the build applied it
+    std::vector<Op_Ptr> BlockGalerkinProducts(const MfemBlockOperator &held, const Op_Ptr &op) const
+    {
+        std::vector<Op_Ptr> newA(Levels_.size());
+        newA[0] = SameBlockStructure(held, op, "Hierarchy");
+        auto hyp = [](const mfem::Operator &M) -> const mfem::HypreParMatrix & { return dynamic_cast<const mfem::HypreParMatrix &>(M); };
+        for (size_t l = 1; l < Levels_.size(); ++l)
+        {
+            auto &Af = dynamic_cast<const MfemBlockOperator &>(*newA[l - 1]);
+            auto &Ac = dynamic_cast<const MfemBlockOperator &>(*Levels_[l]->Get<Op_Ptr>("A"));
+            auto &P = dynamic_cast<const MfemBlockOperator &>(*Levels_[l]->Get<Op_Ptr>("P"));
+            auto next = std::make_shared<MfemBlockOperator>(Ac.CopyRowOffsets());
+            for (size_t i = 0; i < Ac.GetNumBlockRows(); ++i)
+                for (size_t j = 0; j < Ac.GetNumBlockCols(); ++j)
+                {
+                    if (Ac.IsZeroBlock(i, j)) continue;
+                    auto blk = CopyOf(hyp(Ac.GetBlock(i, j)));
+                    PE_CALL(pe_rap_numeric(Device::Get(), hyp(P.GetBlock(i, i)).Handle(), hyp(Af.GetBlock(i, j)).Handle(),
+                                           hyp(P.GetBlock(j, j)).Handle(), blk->Handle()));
+                    if (i == j)
+                        FixRecordedZeroRows(*blk, (int)l, (int)i, "block (" + std::to_string(i) + "," + std::to_string(i) +
+                                                                  ") of the operator of level " + std::to_string(l));
+                    next->SetBlock(i, j, blk);
+                }
+            newA[l] = next;
+        }
+        return newA;
+    }
+    /// New values on the same pattern (one rank): the state BuildSolver(op) would produce with the same sequence,
+    /// parameters and boundary labels.  Level 0 adopts op; A_l = P_l^T A_{l-1} P_l is recomputed by the numeric product
+    /// into a copy of the held A_l's pattern (on a blocked hierarchy block by block, P_i^T A_{l-1}(i,j) P_j), then
+    /// FixZeroRows; Hiptmair's D^T A D likewise.  Every check (rank count, operator type, block structure, patterns, the
+    /// recorded FixZeroRows rows) runs before anything is changed, so a refused call leaves the hierarchy as it was.
+    /// Then the smoothers, the coarse solver (a Krylov solver's preconditioner first) and the colour-numbered residual
+    /// copies take the new operators, and the recorded cycle is dropped: the next two preconditioner calls run directly
+    /// and record again.
     void _do_set_operator(const Op_Ptr &op) override
     {
         pe_ctx *ctx = Device::Get();
         PARELAG_TEST_FOR_EXCEPTION(pe_ctx_nranks(ctx) != 1, std::runtime_error,
                                    "Hierarchy::SetOperator(): more than one rank is not supported; build a new solver");
-        const bool blocked = std::dynamic_pointer_cast<MfemBlockOperator>(op) ||
-                             std::dynamic_pointer_cast<MfemBlockOperator>(Levels_.front()->Get<Op_Ptr>("A"));
-        PARELAG_TEST_FOR_EXCEPTION(blocked, std::runtime_error,
-                                   "Hierarchy::SetOperator(): blocked operators (MfemBlockOperator) are not supported; build a new solver");
-        auto A = std::dynamic_pointer_cast<mfem::HypreParMatrix>(op);
-        auto A0 = std::dynamic_pointer_cast<mfem::HypreParMatrix>(Levels_.front()->Get<Op_Ptr>("A"));
-        PARELAG_TEST_FOR_EXCEPTION(!A || !A0, std::runtime_error, "Hierarchy::SetOperator(): operator must be a HypreParMatrix");
-        CheckSamePattern(*A0, *A, "Hierarchy");
         const int L = (int)Levels_.size();
-        std::vector<std::shared_ptr<mfem::HypreParMatrix>> newA(L);
-        newA[0] = A;
         Timer galerkin = TimeManager::AddTimer("SetOperator: Galerkin products");
-        for (int l = 1; l < L; ++l)
-        {
-            auto &P = dynamic_cast<const mfem::HypreParMatrix &>(*Levels_[l]->Get<Op_Ptr>("P"));
-            newA[l] = CopyOf(dynamic_cast<const mfem::HypreParMatrix &>(*Levels_[l]->Get<Op_Ptr>("A")));
-            PE_CALL(pe_rap_numeric(ctx, newA[l - 1]->Handle(), P.Handle(), newA[l]->Handle()));
-            if (l < (int)ZeroRows_.size() && ZeroRows_[l].Size() > 0)
-                FixSameZeroRows(*newA[l], ZeroRows_[l], "the operator of level " + std::to_string(l));
-        }
+        auto blocked = std::dynamic_pointer_cast<MfemBlockOperator>(Levels_.front()->Get<Op_Ptr>("A"));
+        const std::vector<Op_Ptr> newA = blocked ? BlockGalerkinProducts(*blocked, op) : GalerkinProducts(op);
         galerkin.Stop();
         // the auxiliary operator of every Hiptmair smoother, once per object (pre- and post-smoother are often one)
         Timer aux_timer = TimeManager::AddTimer("SetOperator: Hiptmair auxiliary operators");
@@ -1220,7 +1224,7 @@ private:
         for (int l = 0; l < L; ++l)
         {
             Level &lev = *Levels_[l];
-            lev.Reset<Op_Ptr>("A", Op_Ptr(newA[l]));
+            lev.Reset<Op_Ptr>("A", newA[l]);
             Op_Ptr done;
             for (const char *key : {"PreSmoother", "PostSmoother"})
             {
@@ -1239,11 +1243,12 @@ private:
         Timer colour = TimeManager::AddTimer("SetOperator: colour-numbered copies");
         for (int l = 0; l < L; ++l)
             if (colour_state_ > 0 && l < (int)cres_.size() && cres_[l])
-                PE_CALL(pe_mat_renumbered_values(ctx, newA[l]->Handle(), colour_[l].pos, cres_[l].get()));
+                PE_CALL(pe_mat_renumbered_values(ctx, dynamic_cast<const mfem::HypreParMatrix &>(*newA[l]).Handle(),
+                                                 colour_[l].pos, cres_[l].get()));
         colour.Stop();
         DropRecordedCycle();
     }
-    std::vector<mfem::Vector> ZeroRows_;        // per level: the rows FixZeroRows rewrote at build time (SetZeroRows)
+    std::vector<std::vector<mfem::Vector>> ZeroRows_;   // [level][block]: the rows FixZeroRows rewrote at build time (SetZeroRows)
     std::vector<std::shared_ptr<Level>> Levels_;
     mutable std::vector<mfem::Vector> CoarseResids_, CoarseSols_, tmp_resid_, tmp_correct_;
     std::vector<int> CycleMu_;
@@ -1354,7 +1359,11 @@ inline std::unique_ptr<Hierarchy> buildBlockedHierarchyFromDeRhamSequence(const 
                 {
                     auto &Aij = dynamic_cast<mfem::HypreParMatrix &>(A_blocked->GetBlock(row, col));
                     auto tmp = std::shared_ptr<mfem::HypreParMatrix>{mfem::RAP(P_blocks[row].get(), &Aij, P_blocks[col].get())};
-                    if (row == col && label_ess[row].size() > 0) hypre_ParCSRMatrixFixZeroRows(*tmp);
+                    if (row == col && label_ess[row].size() > 0)
+                    {
+                        H->SetZeroRows(l, ZeroRows(*tmp), row);
+                        hypre_ParCSRMatrixFixZeroRows(*tmp);
+                    }
                     Ac->SetBlock(row, col, std::move(tmp));
                 }
         for (int row = 0; row < NumBlockRows; ++row) P->SetBlock(row, row, P_blocks[row]);

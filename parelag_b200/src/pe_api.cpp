@@ -487,6 +487,34 @@ extern "C" int pe_api_solver_set_operator(pe_solver *s, pe_mat *A)
     s->A = op;
     API_CATCH
 }
+/// SetOperator on a solver built on an MfemBlockOperator: blocks[nblocks*nblocks] row-major, NULL = zero block, with
+/// the held operator's block structure and patterns; ownership of every block passes to the solver, and they are
+/// released when the call is refused
+extern "C" int pe_api_solver_set_operator_block(pe_solver *s, int nblocks, pe_mat **blocks)
+{
+    API_TRY
+    PARELAG_TEST_FOR_EXCEPTION(nblocks < 1 || !blocks, std::runtime_error, "pe_api_solver_set_operator_block: bad arguments");
+    std::vector<std::shared_ptr<mfem::HypreParMatrix>> mats((size_t)nblocks * nblocks);   // released when the call is refused
+    for (int k = 0; k < nblocks * nblocks; ++k)
+        if (blocks[k]) { mats[k] = std::make_shared<mfem::HypreParMatrix>(blocks[k]); blocks[k] = nullptr; }
+    PARELAG_TEST_FOR_EXCEPTION(!s, std::runtime_error, "pe_api_solver_set_operator_block: bad arguments");
+    auto held = std::dynamic_pointer_cast<MfemBlockOperator>(s->A);
+    PARELAG_TEST_FOR_EXCEPTION(!held, std::runtime_error,
+                               "pe_api_solver_set_operator_block: the solver's operator is not an MfemBlockOperator");
+    PARELAG_TEST_FOR_EXCEPTION(pe_ctx_nranks(Device::Get()) != 1, std::runtime_error,
+                               "pe_api_solver_set_operator_block: more than one rank is not supported; build a new solver");
+    PARELAG_TEST_FOR_EXCEPTION((size_t)nblocks != held->GetNumBlockRows() || (size_t)nblocks != held->GetNumBlockCols(),
+                               std::runtime_error, "pe_api_solver_set_operator_block: the solver's operator has "
+                               << held->GetNumBlockRows() << "x" << held->GetNumBlockCols() << " blocks, not " << nblocks << "x" << nblocks);
+    auto op = std::make_shared<MfemBlockOperator>(held->CopyRowOffsets(), held->CopyColumnOffsets());
+    for (int i = 0; i < nblocks; ++i)
+        for (int j = 0; j < nblocks; ++j)
+            if (mats[i * nblocks + j]) op->SetBlock(i, j, mats[i * nblocks + j]);     // refuses a block of the wrong size
+    SameBlockStructure(*held, op, "pe_api_solver_set_operator_block");
+    SetNestedOperator(*s->solver, op);
+    s->A = op;
+    API_CATCH
+}
 /// mixed (Darcy) system blocks as in examples/MultigridTestDarcy.cpp: M = mass(H(div)) (weights folded into
 /// the element matrices), B = W D with W = mass(L2), Bt = B^T; the driver solves [[M Bt][B 0]]
 extern "C" int pe_api_sequence_assemble_darcy(pe_sequence *s, int level, pe_mat **M_out, pe_mat **B_out, pe_mat **Bt_out)
@@ -800,6 +828,25 @@ extern "C" int pe_api_solver_level_matrix(const pe_solver *s, int level, int32_t
     auto M = std::dynamic_pointer_cast<mfem::HypreParMatrix>(h->GetLevel(level).Get<Op_Ptr>("A"));
     PARELAG_TEST_FOR_EXCEPTION(!M, std::runtime_error, "pe_api_solver_level_matrix: the level operator is not a ParCSR matrix");
     PE_CALL(pe_mat_download(M->Handle(), I, J, A, nullptr, nullptr, nullptr, nullptr));
+    API_CATCH
+}
+extern "C" int pe_api_solver_level_block(const pe_solver *s, int level, int i, int j, pe_mat **out)
+{
+    API_TRY
+    *out = nullptr;
+    auto op = const_cast<Hierarchy *>(as_hierarchy(s))->GetLevel(level).Get<Op_Ptr>("A");
+    const mfem::Operator *blk = op.get();
+    if (auto B = std::dynamic_pointer_cast<MfemBlockOperator>(op))
+    {
+        PARELAG_TEST_FOR_EXCEPTION(i < 0 || j < 0 || (size_t)i >= B->GetNumBlockRows() || (size_t)j >= B->GetNumBlockCols(),
+                                   std::runtime_error, "pe_api_solver_level_block: no block (" << i << "," << j << ")");
+        if (B->IsZeroBlock(i, j)) return 0;
+        blk = &B->GetBlock(i, j);
+    }
+    else PARELAG_TEST_FOR_EXCEPTION(i != 0 || j != 0, std::runtime_error, "pe_api_solver_level_block: the level operator is not blocked");
+    auto M = dynamic_cast<const mfem::HypreParMatrix *>(blk);
+    PARELAG_TEST_FOR_EXCEPTION(!M, std::runtime_error, "pe_api_solver_level_block: the block is not a ParCSR matrix");
+    PE_CALL(pe_mat_clone(Device::Get(), M->Handle(), out));
     API_CATCH
 }
 extern "C" int pe_api_solver_free(pe_solver *s) { delete s; return 0; }

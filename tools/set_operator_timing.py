@@ -11,7 +11,16 @@ smoothers and coarse solver, colour-numbered copies).  The fine-level numeric pr
 level-1 prolongator ComputeTrueP) is also timed on its own, with its two parts: the two-pass A P and the numeric
 P^T (A P) into A_1's pattern.  Bytes are computed from the shapes, each array read or written once (int32 indices,
 FP64 values): A P reads A and P and writes A P; P^T (A P) reads P^T and A P, the row pointers and columns of A_1, and
-writes A_1's values."""
+writes A_1's values.
+
+--config darcy / spe10: the mixed solver bench.py --config darcy / spe10 builds (configs[1] MultigridTestDarcy at 136^3 with
+4 levels, configs[3] SPE10-shaped 60 x 220 x 85 with the synthetic lognormal permeability; --mixed-solver ldu: GMRES +
+Block LDU with AMGe V-cycles on M and on the Schur complement, blocked: GMRES + the blocked AMGe hierarchy with Block
+Jacobi smoothers; multicolour ordering).  BuildSolver(M1, B, Bt); SetOperator(M2, B, Bt) with M2 = S M1 S (S a seeded
+positive diagonal); the first GMRES solve after the update; then BuildSolver(M2, B, Bt) and its first GMRES solve.  The
+update's phase timers nest: "block inverses" (the A00 and S inverses, for Block LDU the inner AMGe hierarchies with
+their own Galerkin products and smoothers) and "Schur complements" run inside "smoothers and coarse solver" of a blocked
+hierarchy."""
 import argparse
 import json
 import os
@@ -92,13 +101,80 @@ def fine_rap(ctx, S, A1, A2, ess, repeats=5):
     return out
 
 
+MIXED_PHASES = ("Galerkin products", "Schur complements", "block inverses", "smoothers and coarse solver")
+
+
+def mixed(ctx, args):
+    """--config darcy / spe10: SetOperator(M2, B, Bt) against BuildSolver on the same blocks, and the first GMRES solve"""
+    if args.config == "darcy":
+        S = api.Sequence.hex((136,) * 3, 4, jstart=2)
+        shape = {"size": 136, "levels": 4}
+    else:
+        dims, Lspe = (60, 220, 85), (1200.0, 2200.0, 170.0)
+        kinv = 10.0 ** (-np.clip(np.random.default_rng(13).normal(-1.0, 1.5, size=dims[0] * dims[1] * dims[2]), -4.0, 2.0))
+        S = api.Sequence.hex(dims, 4, L=Lspe, beta=kinv, jstart=2)
+        shape = {"dims": list(dims), "levels": 4}
+    Md, Bd, Btd = S.assemble_darcy(ctx, 0)
+    M1, B, Bt = Md.to_scipy(), Bd.to_scipy(), Btd.to_scipy()
+    for m in (Md, Bd, Btd):
+        m.free()
+    rows = np.repeat(np.arange(M1.shape[0]), np.diff(M1.indptr))
+    sc = np.random.default_rng(1).uniform(0.5, 2.0, M1.shape[0])
+    M2 = M1.copy()
+    M2.data = M1.data * sc[rows] * sc[M1.indices]
+    if args.mixed_solver == "ldu":
+        xml, name, ess = api.library_xml(bench.library_darcy_ldu("multicolor")), "GMRES with Block LDU", np.zeros((2, 6), dtype=np.int32)
+    else:
+        xml, name, ess = api.library_xml(bench.library_darcy("multicolor")), "GMRES with blocked AMGe", None
+    n = M1.shape[0] + B.shape[0]
+    b = np.random.default_rng(2).standard_normal(n)
+    vb, vz = capi.Vec(ctx, data=b), capi.Vec(ctx, n)
+    res = dict(shape, config=args.config, solver=name, rows_M=int(M1.shape[0]), nnz_M=int(M1.nnz), rows_B=int(B.shape[0]),
+               nnz_B=int(B.nnz))
+
+    def blocks(M):
+        return [[capi.Mat.from_scipy(ctx, M), capi.Mat.from_scipy(ctx, Bt)], [capi.Mat.from_scipy(ctx, B), None]]
+    m1 = blocks(M1)
+    res["build_solver_M1_s"], solver = timed(ctx, lambda: api.BlockSolver(xml, name, m1, S, 0, [2, 3], ess_attr=ess))
+    for _ in range(3):
+        solver.prec_mult_device(vb, vz)
+    m2 = blocks(M2)
+    api.lib().pe_api_timer_clear()
+    res["set_operator_M2_s"], _ = timed(ctx, lambda: solver.set_blocks(m2))
+    res["set_operator_phases_s"] = {k: api.timer("SetOperator: " + k) for k in MIXED_PHASES}
+    res["first_solve_after_update_s"], x_upd = timed(ctx, lambda: solver.mult(b))
+    h_upd = solver.history()
+    solver.free()
+    m2b = blocks(M2)
+    res["build_solver_M2_s"], fresh = timed(ctx, lambda: api.BlockSolver(xml, name, m2b, S, 0, [2, 3], ess_attr=ess))
+    res["first_solve_fresh_s"], x_fresh = timed(ctx, lambda: fresh.mult(b))
+    h_fresh = fresh.history()
+    fresh.free()
+    res["gmres_iterations_update_fresh"] = [h_upd[1], h_fresh[1]]
+    res["fresh_equals_update"] = bool(np.array_equal(x_upd, x_fresh) and np.array_equal(h_upd[0], h_fresh[0]))
+    vb.free(); vz.free()
+    S.free()
+    return res
+
+
 def main():
     ap = argparse.ArgumentParser()
+    ap.add_argument("--config", default="hdiv", choices=["hdiv", "darcy", "spe10"])
+    ap.add_argument("--mixed-solver", default="ldu", choices=["ldu", "blocked"], help="darcy / spe10, as bench.py")
     ap.add_argument("--size", type=int, default=144)
     ap.add_argument("--levels", type=int, default=5)
     ap.add_argument("--out", default=None)
     args = ap.parse_args()
     ctx = api.session()
+    if args.config != "hdiv":
+        res = mixed(ctx, args)
+        res["card"], res["power_limit"] = card()
+        line = json.dumps(res)
+        print(line)
+        if args.out:
+            with open(args.out, "w") as f:
+                f.write(line + "\n")
+        return
     ESS = np.ones(6, dtype=np.int32)
     S = api.Sequence.hex((args.size,) * 3, args.levels, jstart=1)
     xml = api.library_xml(bench.library("multicolor", 2))
